@@ -19,6 +19,11 @@ independent batches -- no data-path collective (SURVEY.md 8e), NCCL only for the
 `parity`  : GPU outputs against the reference's on the cpu_baseline frames: |dp|, mask pixels / droplets differing.
 `config4` : BASELINE configs[3] -- `--frames 4096` frames sharded round-robin over the ranks (strong scaling), tables
            gathered to rank 0 in frame order inside the timed region, merged-table checksum (equal for every N).
+`--dump-outputs DIR` : after the timed steps, rank 0 writes what the device-resident arm returned in its last step as
+           DIR/<name>.npy (float32 / float64, under 64 MB; see last_step_outputs).  The inputs depend only on the
+           arguments, so two builds run with the same arguments can be compared output for output.  With N > 1 the
+           files hold rank 0's frames only, and each rank's frames depend on its rank: compare dumps taken with the
+           same --gpus.
 """
 from __future__ import annotations
 
@@ -313,6 +318,50 @@ def run_config4(pipe, dev, rank, world, frames_total, batch, size, barrier, dist
     return out
 
 
+# ------------------------------------------------------------------------------------ --dump-outputs
+DUMP_BYTES = 60 << 20           # all arrays together: with the .npy headers, under 64 MB
+DUMP_MASK_BYTES = 16 << 20      # of which the mask rows
+
+
+def last_step_outputs(masks, tables):
+    """The timed path's results (masks u8 [B,H,W] and the droplet tables) as host float32 / float64 arrays.
+
+    mask_rows [n, W] holds whole mask rows, mask_row_index [n, 2] their (image, row): every row while the batch fits in
+    DUMP_MASK_BYTES as float32, otherwise a sample of rows drawn with seed 0.  droplet_counts [B] is the number of
+    droplets per image; droplets_<column> holds one entry per droplet, image by image, for the columns of
+    DropletTables.to_host() plus `image`; past the remaining budget a seed-0 sample of droplets is kept (their
+    `image` and `label` say which)."""
+    import torch
+    rng = np.random.default_rng(0)
+    B, H, W = masks.shape
+    n_rows = min(B * H, max(1, DUMP_MASK_BYTES // (4 * W)))
+    rows = np.sort(rng.choice(B * H, n_rows, replace=False))
+    picked = masks.reshape(B * H, W).index_select(0, torch.from_numpy(rows).to(masks.device))
+    out = {"mask_rows": picked.cpu().numpy().astype(np.float32),
+           "mask_row_index": np.stack([rows // H, rows % H], 1).astype(np.float64)}
+    per_image = tables.to_host()
+    out["droplet_counts"] = np.array([len(t["label"]) for t in per_image], np.float64)
+    cols = {"image": np.concatenate([np.full(len(t["label"]), b, np.float64) for b, t in enumerate(per_image)])}
+    for c in per_image[0]:
+        cols[c] = np.concatenate([np.asarray(t[c], np.float64) for t in per_image])
+    n = len(cols["image"])
+    room = (DUMP_BYTES - sum(a.nbytes for a in out.values())) // (8 * len(cols))
+    if n > room:
+        keep = np.sort(rng.choice(n, room, replace=False))
+        cols = {c: v[keep] for c, v in cols.items()}
+    out.update({f"droplets_{c}": v for c, v in cols.items()})
+    return out
+
+
+def write_outputs(directory, arrays):
+    d = Path(directory)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(d / f"{name}.npy", a)
+    total = sum(a.nbytes for a in arrays.values())
+    print(f"bench.py: wrote {len(arrays)} arrays ({total / 2**20:.1f} MiB) to {d}", file=sys.stderr)
+
+
 # ------------------------------------------------------------------------------------ B200 arm
 def run_b200(args):
     import torch
@@ -399,6 +448,7 @@ def run_b200(args):
     stage_ms = [sum(ev[k][i].elapsed_time(ev[k][i + 1]) for k in range(K)) / K for i in range(3)]
     step_ms = [ev[k][0].elapsed_time(ev[k + 1][0]) if k + 1 < K else ev[k][0].elapsed_time(end) for k in range(K)]
     counts = last.counts.cpu().numpy()
+    dumped = last_step_outputs(masks, last) if args.dump_outputs and rank == 0 else None
     value = world * B * K / (ms_total / 1e3)
 
     # ---- end-to-end arm: pinned host frames in, host masks + table rows out, every copy inside the timed region.
@@ -530,6 +580,8 @@ def run_b200(args):
         except Exception as exc:  # noqa: BLE001  (the CPU leg must not cost the GPU line)
             line.setdefault("cpu_baseline", {"error": f"{type(exc).__name__}: {exc}"})
             line.setdefault("parity", {"error": f"{type(exc).__name__}: {exc}"})
+    if dumped is not None:
+        write_outputs(args.dump_outputs, dumped)
     if rank == 0:
         _OUT.write(json.dumps(line) + "\n")
         _OUT.flush()
@@ -563,7 +615,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--graphs", action="store_true",
                     help="e2e arm: replay each batch's launches as one CUDA graph (DropletPipeline(use_graphs=True))")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's masks and droplet tables to DIR/<name>.npy (rank 0, --impl b200)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 path (--impl b200)")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     global _OUT
     _OUT = _claim_stdout()

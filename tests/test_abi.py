@@ -74,25 +74,38 @@ def test_workspace_queries_and_argument_errors_need_no_gpu():
     assert ei.value.code == _lib.DC_EINVAL
 
 
+NO_GPU_CHECK = r"""
+import ctypes as C, sys
+import numpy as np
+import pytest
+import torch
+sys.path.insert(0, sys.argv[1])
+import unet_dc_segmentation_b200 as pkg
+assert not torch.cuda.is_available()
+m = pkg.UNetDC(3, 1).eval()
+with pytest.raises(RuntimeError, match="no CPU"):
+    m(torch.zeros(1, 3, 16, 16))
+with pytest.raises((RuntimeError, AssertionError)):
+    pkg.quantify(np.zeros((8, 8), np.uint8), 1, None)
+with pytest.raises((RuntimeError, AssertionError)):
+    pkg.rolling_ball_correction_rgb(np.zeros((8, 8, 3), np.uint8), 5)
+from unet_dc_segmentation_b200 import _lib
+lib = _lib.load()
+args = _lib.LabelArgs()
+rc = lib.dc_label_stats(C.byref(args), None)
+assert rc in (_lib.DC_ECUDA, _lib.DC_EDEVICE) and lib.dc_last_error()
+print("NO_FALLBACK_OK")
+"""
+
+
 def test_no_cpu_fallback():
-    """Without a CUDA tensor the product raises; it never routes to the oracle or to PyTorch ops."""
-    import numpy as np
-    import torch
-    import unet_dc_segmentation_b200 as pkg
-    if torch.cuda.is_available():
-        pytest.skip("this check is for the GPU-less container")
-    m = pkg.UNetDC(3, 1).eval()
-    with pytest.raises(RuntimeError, match="no CPU"):
-        m(torch.zeros(1, 3, 16, 16))
-    with pytest.raises((RuntimeError, AssertionError)):
-        pkg.quantify(np.zeros((8, 8), np.uint8), 1, None)
-    with pytest.raises((RuntimeError, AssertionError)):
-        pkg.rolling_ball_correction_rgb(np.zeros((8, 8, 3), np.uint8), 5)
-    from unet_dc_segmentation_b200 import _lib
-    lib = _lib.load()
-    args = _lib.LabelArgs()
-    rc = lib.dc_label_stats(C.byref(args), None)
-    assert rc in (_lib.DC_ECUDA, _lib.DC_EDEVICE) and lib.dc_last_error()
+    """Without a GPU the product raises; it never routes to the oracle or to PyTorch ops.  Checked in a child process
+    that sees no CUDA device, so that it holds on machines with and without one."""
+    import os
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    r = subprocess.run([sys.executable, "-c", NO_GPU_CHECK, str(REPO)], env=env, capture_output=True, text=True,
+                       timeout=300)
+    assert r.returncode == 0 and "NO_FALLBACK_OK" in r.stdout, r.stdout[-2000:] + r.stderr[-2000:]
 
 
 def test_product_never_imports_the_oracle():
