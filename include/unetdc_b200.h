@@ -49,7 +49,7 @@ extern "C" {
 
 /* Bumped whenever a struct or signature in this header changes; dc_version() returns the value the library was
  * built with and the Python binding refuses to load a library that disagrees. */
-#define DC_ABI_VERSION 205
+#define DC_ABI_VERSION 206
 
 const char* dc_last_error(void);
 int dc_version(void);
@@ -250,13 +250,30 @@ typedef struct dc_rolling_ball_args {
     size_t workspace_bytes;
 } dc_rolling_ball_args_t;
 
+/* Radius 1..dc_rolling_ball_tiled_max_radius() (170): the tiled chord kernel (haloed tiles in shared memory).
+ * Larger radii, up to dc_rolling_ball_max_radius() (2047): the banded pass (rectangle decomposition of the ellipse,
+ * full rows of a band of output rows in shared memory), which takes rows of at most
+ * DC_ROLLING_BALL_BANDED_MAX_WIDTH pixels and returns DC_EINVAL for wider ones.  Both run three kernels inside the
+ * same workspace, allocate nothing, do not synchronise, and allow out == in. */
+#define DC_ROLLING_BALL_BANDED_MAX_WIDTH 32768
 int dc_rolling_ball_workspace_bytes(int B, int H, int W, int C, size_t* bytes);
 int dc_rolling_ball(const dc_rolling_ball_args_t* args, void* stream);
-/* Largest `radius` dc_rolling_ball accepts (the haloed tile of the element has to fit in shared memory). */
+/* The banded pass at any radius 1..dc_rolling_ball_max_radius(), also where dc_rolling_ball would run the tiled
+ * kernel (the two agree bit for bit); same arguments and workspace as dc_rolling_ball. */
+int dc_rolling_ball_banded(const dc_rolling_ball_args_t* args, void* stream);
+/* Largest `radius` dc_rolling_ball accepts: 2047, an element half as wide as a 4096^2 frame. */
 int dc_rolling_ball_max_radius(void);
+/* Largest `radius` dc_rolling_ball runs with the tiled kernel (the haloed tile of the element has to fit in shared
+ * memory); above it, the banded pass. */
+int dc_rolling_ball_tiled_max_radius(void);
 /* TEST AID (host only, no GPU needed): dumps the chord plan the kernel would run for `radius` with tiles of
  * `tile_h` rows; returns the number of ints written (layout: csrc/morph.cu) or a negative DC_E* code. */
 int dc_debug_rolling_ball_plan(int radius, int tile_h, int* out, int cap);
+/* TEST AID (host only, no GPU needed): dumps the rectangles of the banded pass for `radius`:
+ * [k, K, piece], then {ya, yb, xa, xb} (rows and columns relative to the output pixel) for each of the K rectangles
+ * in walk order, widest chord first; `piece` is the run of pixels one thread scans.  Returns the number of ints
+ * written or a negative DC_E* code. */
+int dc_debug_rolling_ball_bands(int radius, int* out, int cap);
 
 /* ------------------------------------------------------------------ bilinear resize (u8)
  * The two cv2.resize calls of quantify_droplets_batch.py:44 (frame -> IMG_SIZE x IMG_SIZE) and :57 (mask -> original

@@ -292,7 +292,7 @@ def build_parser() -> argparse.ArgumentParser:
     p.add_argument("--px_per_micron", type=float, help="pixels per micron for physical-unit columns")
     p.add_argument("--save_overlays", action="store_true")
     p.add_argument("--background_radius", type=int, default=50,
-                   help="radius for rolling ball background correction (the GPU kernel takes 1..174)")
+                   help="radius for rolling ball background correction (1..2047)")
     p.add_argument("--skip_excel", action="store_true", help="skip generation of the Excel workbook")
     p.add_argument("--skip_histogram", action="store_true", help="skip histogram plot generation")
     p.add_argument("--density_maps", action="store_true",

@@ -198,12 +198,22 @@ int dc_rolling_ball_workspace_bytes(int B, int H, int W, int C, size_t* bytes) {
 
 int dc_rolling_ball_max_radius(void) { return rolling_ball_max_radius(); }
 
+int dc_rolling_ball_tiled_max_radius(void) { return rolling_ball_tiled_max_radius(); }
+
 int dc_debug_rolling_ball_plan(int radius, int tile_h, int* out, int cap) { return rolling_ball_plan_dump(radius, tile_h, out, cap); }
+
+int dc_debug_rolling_ball_bands(int radius, int* out, int cap) { return rolling_ball_bands_dump(radius, out, cap); }
 
 int dc_rolling_ball(const dc_rolling_ball_args_t* args, void* stream) {
     int rc = check_current_device(nullptr);
     if (rc != DC_OK) return rc;
     return launch_rolling_ball(args, (cudaStream_t)stream);
+}
+
+int dc_rolling_ball_banded(const dc_rolling_ball_args_t* args, void* stream) {
+    int rc = check_current_device(nullptr);
+    if (rc != DC_OK) return rc;
+    return launch_rolling_ball_banded(args, (cudaStream_t)stream, "dc_rolling_ball_banded");
 }
 
 int dc_resize_linear_u8(const dc_resize_args_t* args, void* stream) {

@@ -38,6 +38,7 @@ int upfuse_schedule(int* out, int cap);
 int set_upfuse_mode(int mode);
 int launch_label_stats(const dc_label_args_t* a, cudaStream_t stream);
 int launch_rolling_ball(const dc_rolling_ball_args_t* a, cudaStream_t stream);
+int launch_rolling_ball_banded(const dc_rolling_ball_args_t* a, cudaStream_t stream, const char* who);
 int launch_resize_linear_u8(const dc_resize_args_t* a, cudaStream_t stream);
 size_t label_workspace_bytes(int B, int H, int W);
 int launch_overlay_stencil(const dc_overlay_args_t* a, cudaStream_t stream);
@@ -50,7 +51,9 @@ int launch_spatial_density(const dc_spatial_args_t* a, cudaStream_t stream);
 size_t spatial_workspace_bytes(int B, int H, int W);
 size_t rolling_ball_workspace_bytes(int planes, int H, int W);
 int rolling_ball_max_radius();
+int rolling_ball_tiled_max_radius();
 int rolling_ball_plan_dump(int radius, int th, int* out, int cap);
+int rolling_ball_bands_dump(int radius, int* out, int cap);
 int num_sms();
 int launch_pad_input(const float* in, void* out_nhwc64, int B, int C, int H, int W, cudaStream_t stream);
 int launch_head1x1(const void* feat_nhwc64, const float* w, const float* b, float* prob, uint8_t* mask, float thresh, int B,

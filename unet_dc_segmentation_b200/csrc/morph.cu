@@ -20,9 +20,19 @@
 // ones, against 100 unaligned fetches for the row-by-row form, and only 3 small range tables instead of 6.
 // A block owns a 64 x 128 tile; chord tables are double-buffered in shared memory with one barrier per chord.
 // All arithmetic is u8 (as 16-bit lanes for the DPX min/max), so the result is bit-exact.
+//
+// Radii past the tiled kernel's limit (the haloed tile stops fitting shared memory at 171) run the banded pass
+// (morph_band_kernel, below).  cv2's ellipse is the union of K rectangles Y_m x X_m: X_m are the distinct row
+// intervals (nested), Y_m the rows whose interval contains X_m (a contiguous band holding the anchor row).  So
+//   erode(y,x) = min_m min_{x' in x+X_m} V_m(y,x'),   V_m(y,x') = min_{y' in y+Y_m} src(y',x'),
+// walked from the widest chord (shortest band) to the narrowest (tallest band): V_m is V_{m-1} plus the rows the band
+// newly covers, and the horizontal range-min over the shrinking X_m is van Herk / Gil-Werman (prefix / suffix extrema
+// over blocks of |X_m| pixels, two lookups per pixel) on full rows in shared memory, which needs no horizontal halo.
+// Every rectangle contains the anchor, so taps outside the image are the identity (255 erode, 0 dilate).
 #include "common.cuh"
 #include <math.h>
 #include <string.h>
+#include <algorithm>
 
 namespace dc {
 
@@ -374,6 +384,227 @@ __global__ void __launch_bounds__(256) stretch_kernel(const uint8_t* __restrict_
         dst[i * out_c] = lut[src[i]];
 }
 
+// ---------------------------------------------------------------- banded pass (any radius up to RB_MAX_K)
+constexpr int RB_NT = 512;             // threads per block
+constexpr int RB_PIECE = 31;           // pixels of a van Herk block one thread scans (odd: the byte streams of
+                                       // neighbouring threads fall on different banks)
+constexpr int RB_MAX_K = 2047;         // largest element: covers frames up to 4096^2
+constexpr int RB_MAX_BANDS = 1024;     // rectangles of the element (600 at k = 2047)
+constexpr int RB_TMAX = 16;            // output rows per block
+
+struct Band { short ya, yb, xa, xb; };  // rows [ya, yb] x columns [xa, xb] relative to the output pixel
+struct BandPlan {
+    int k, nbands;
+    Band band[RB_MAX_BANDS];           // walk order: widest chord (shortest band) first
+};
+
+template <bool IS_MAX>
+__device__ __forceinline__ uint8_t op8(uint8_t a, uint8_t b) { return IS_MAX ? (a > b ? a : b) : (a < b ? a : b); }
+
+// One morphology pass over T output rows x the full width of one plane (blockIdx.x: row band, blockIdx.y: plane).
+// Planes are addressed as in the tiled kernel; SUBTRACT as there.  Shared memory, per output row:
+//   V  vp bytes  vertical extremum over the current band Y_m        (word per 4 pixels)
+//   A  vp bytes  result so far
+//   P  lp bytes  block prefix extrema over u = x' - xa_m in [0, W + |X_m| - 1), blocks [j |X_m|, (j + 1) |X_m|)
+//   S  lp bytes  block suffix extrema
+//   PC cp bytes  per piece of RB_PIECE pixels: extremum of the earlier pieces of its block (blocks wider than a piece)
+//   SC cp bytes  ... of the later pieces
+// Output x then takes op(S[x], P[x + |X_m| - 1]): the window [x + xa, x + xb] is the suffix of one block and the
+// prefix of the next (or all of one block).
+template <bool IS_MAX, bool SUBTRACT>
+__global__ void __launch_bounds__(RB_NT) morph_band_kernel(const uint8_t* __restrict__ in, int in_c,
+                                                           uint8_t* __restrict__ out, const uint8_t* __restrict__ orig,
+                                                           int orig_c, int H, int W, int T, int vp, int lp, int cp,
+                                                           int* __restrict__ minmax, const __grid_constant__ BandPlan bp) {
+    extern __shared__ __align__(16) uint8_t bsm[];
+    uint8_t* V = bsm;
+    uint8_t* A = V + T * vp;
+    uint8_t* P = A + T * vp;
+    uint8_t* S = P + T * lp;
+    uint8_t* PC = S + T * lp;
+    uint8_t* SC = PC + T * cp;
+    unsigned* V32 = reinterpret_cast<unsigned*>(V);
+    unsigned* A32 = reinterpret_cast<unsigned*>(A);
+    const unsigned* P32 = reinterpret_cast<const unsigned*>(P);
+    const unsigned* S32 = reinterpret_cast<const unsigned*>(S);
+    const int vpw = vp >> 2, lpw = lp >> 2;
+
+    const unsigned ident = IS_MAX ? 0u : 0xffffffffu;
+    const uint8_t id8 = IS_MAX ? 0 : 255;
+    const int tid = threadIdx.x, plane = blockIdx.y, y0 = blockIdx.x * T;
+    const int b = plane / in_c, c = plane % in_c;
+    if (!SUBTRACT && minmax && blockIdx.x == 0 && tid == 0) {
+        minmax[2 * plane] = 255;                 // the dilate pass (a later launch) reduces into these
+        minmax[2 * plane + 1] = 0;
+    }
+    const uint8_t* src = in + (size_t)b * H * W * in_c + c;
+    const bool vec = in_c == 1 && (W & 3) == 0 && (reinterpret_cast<uintptr_t>(in) & 3) == 0;
+    const int ww = (W + 3) >> 2, nw = T * ww;    // words per row, words of the band
+
+    // op of source row yy into the word xw of a V row (identity outside the image)
+    auto fold = [&](unsigned v, int yy, int xw) -> unsigned {
+        if ((unsigned)yy >= (unsigned)H) return v;
+        unsigned w;
+        if (vec) {
+            w = __ldg(reinterpret_cast<const unsigned*>(src + (size_t)yy * W) + xw);
+        } else {
+            w = 0;
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                const int x = 4 * xw + q;
+                const unsigned p = x < W ? src[((size_t)yy * W + x) * in_c] : id8;
+                w |= p << (8 * q);
+            }
+        }
+        return vop<IS_MAX>(v, w);
+    };
+
+    const int K = bp.nbands;
+    int pya = bp.band[0].ya, pyb = bp.band[0].yb;          // band folded into V
+    for (int i = tid; i < nw; i += RB_NT) {
+        const int t = i / ww, xw = i - t * ww, y = y0 + t;
+        unsigned v = ident;
+        for (int dy = pya; dy <= pyb; ++dy) v = fold(v, y + dy, xw);
+        V32[t * vpw + xw] = v;
+        A32[t * vpw + xw] = ident;
+    }
+    __syncthreads();
+
+    for (int m = 0; m < K; ++m) {
+        const int xa = bp.band[m].xa, w = bp.band[m].xb - xa + 1, L = W + w - 1;
+        const int nb = (L + w - 1) / w, np = (w + RB_PIECE - 1) / RB_PIECE, npr = nb * np;
+        // 1. prefix and suffix extrema of every piece (u outside the image's columns is the identity)
+        for (int i = tid; i < T * npr; i += RB_NT) {
+            const int t = i / npr, r = i - t * npr, blk = r / np, pc = r - blk * np;
+            const int bs = blk * w, u0 = bs + pc * RB_PIECE;
+            if (u0 >= L) continue;
+            const int u1 = min(min(u0 + RB_PIECE, bs + w), L);
+            const uint8_t* vr = V + t * vp;
+            uint8_t* pr = P + t * lp;
+            uint8_t* sr = S + t * lp;
+            uint8_t run = id8;
+            for (int u = u0; u < u1; ++u) {
+                const int x = u + xa;
+                run = op8<IS_MAX>(run, (unsigned)x < (unsigned)W ? vr[x] : id8);
+                pr[u] = run;
+            }
+            run = id8;
+            for (int u = u1 - 1; u >= u0; --u) {
+                const int x = u + xa;
+                run = op8<IS_MAX>(run, (unsigned)x < (unsigned)W ? vr[x] : id8);
+                sr[u] = run;
+            }
+        }
+        __syncthreads();
+        if (np > 1) {
+            // 2. blocks of several pieces: carry the extrema of the other pieces of the block into P and S
+            for (int i = tid; i < T * nb; i += RB_NT) {
+                const int t = i / nb, blk = i - t * nb, bs = blk * w;
+                const int npb = min(np, (L - bs + RB_PIECE - 1) / RB_PIECE);     // pieces of this block inside [0, L)
+                const uint8_t* pr = P + t * lp;
+                const uint8_t* sr = S + t * lp;
+                uint8_t* pcr = PC + t * cp + blk * np;
+                uint8_t* scr = SC + t * cp + blk * np;
+                uint8_t run = id8;
+                for (int q = 0; q < npb; ++q) {
+                    pcr[q] = run;
+                    run = op8<IS_MAX>(run, pr[min(min(bs + (q + 1) * RB_PIECE, bs + w), L) - 1]);
+                }
+                run = id8;
+                for (int q = npb - 1; q >= 0; --q) {
+                    scr[q] = run;
+                    run = op8<IS_MAX>(run, sr[bs + q * RB_PIECE]);
+                }
+            }
+            __syncthreads();
+            for (int i = tid; i < T * npr; i += RB_NT) {
+                const int t = i / npr, r = i - t * npr, blk = r / np, pc = r - blk * np;
+                const int bs = blk * w, u0 = bs + pc * RB_PIECE;
+                if (u0 >= L) continue;
+                const int u1 = min(min(u0 + RB_PIECE, bs + w), L);
+                uint8_t* pr = P + t * lp;
+                uint8_t* sr = S + t * lp;
+                const uint8_t pcv = PC[t * cp + r], scv = SC[t * cp + r];
+                for (int u = u0; u < u1; ++u) {
+                    pr[u] = op8<IS_MAX>(pr[u], pcv);
+                    sr[u] = op8<IS_MAX>(sr[u], scv);
+                }
+            }
+            __syncthreads();
+        }
+        // 3. fold this rectangle into the result, and grow V to the next rectangle's band
+        const bool more = m + 1 < K;
+        const int nya = more ? bp.band[m + 1].ya : pya, nyb = more ? bp.band[m + 1].yb : pyb;
+        for (int i = tid; i < nw; i += RB_NT) {
+            const int t = i / ww, xw = i - t * ww;
+            const int e = 4 * xw + w - 1;
+            const unsigned sv = S32[t * lpw + xw];
+            const unsigned pv = __funnelshift_r(P32[t * lpw + (e >> 2)], P32[t * lpw + (e >> 2) + 1], (e & 3) * 8);
+            A32[t * vpw + xw] = vop<IS_MAX>(A32[t * vpw + xw], vop<IS_MAX>(sv, pv));
+            if (more) {
+                const int y = y0 + t;
+                unsigned v = V32[t * vpw + xw];
+                for (int dy = nya; dy < pya; ++dy) v = fold(v, y + dy, xw);
+                for (int dy = pyb + 1; dy <= nyb; ++dy) v = fold(v, y + dy, xw);
+                V32[t * vpw + xw] = v;
+            }
+        }
+        pya = nya;
+        pyb = nyb;
+        __syncthreads();
+    }
+
+    // ---- write (and, for the second pass, subtract + reduce) ----
+    int mn = 255, mx = 0;
+    for (int i = tid; i < nw; i += RB_NT) {
+        const int t = i / ww, xw = i - t * ww, gy = y0 + t, gx = 4 * xw;
+        if (gy >= H) continue;
+        const unsigned acc = A32[t * vpw + xw];
+        uint8_t* dst = out + ((size_t)plane * H + gy) * W + gx;
+        unsigned res = acc;
+        if (SUBTRACT) {
+            const int ob = plane / orig_c, oc = plane % orig_c;
+            const uint8_t* o = orig + ((size_t)ob * H * W + (size_t)gy * W + gx) * orig_c + oc;
+            unsigned ov = 0;
+            if (orig_c == 1 && gx + 3 < W && ((reinterpret_cast<uintptr_t>(o) & 3) == 0)) {
+                ov = __ldg(reinterpret_cast<const unsigned*>(o));
+            } else {
+#pragma unroll
+                for (int q = 0; q < 4; ++q)
+                    if (gx + q < W) ov |= (unsigned)o[(size_t)q * orig_c] << (8 * q);
+            }
+            res = __vsubus4(ov, acc);            // cv2.subtract saturates at 0
+        }
+        if (gx + 3 < W && ((reinterpret_cast<uintptr_t>(dst) & 3) == 0)) {
+            *reinterpret_cast<unsigned*>(dst) = res;
+            if (SUBTRACT) {
+#pragma unroll
+                for (int q = 0; q < 4; ++q) {
+                    const int v = (res >> (8 * q)) & 0xff;
+                    mn = min(mn, v); mx = max(mx, v);
+                }
+            }
+        } else {
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                if (gx + q < W) {
+                    const int v = (res >> (8 * q)) & 0xff;
+                    dst[q] = (uint8_t)v;
+                    mn = min(mn, v); mx = max(mx, v);
+                }
+            }
+        }
+    }
+    if (SUBTRACT) {
+        mn = __reduce_min_sync(0xffffffffu, mn);
+        mx = __reduce_max_sync(0xffffffffu, mx);
+        if ((tid & 31) == 0) {
+            atomicMin(&minmax[2 * plane], mn);
+            atomicMax(&minmax[2 * plane + 1], mx);
+        }
+    }
+}
+
 // Element rows of cv2.getStructuringElement(MORPH_ELLIPSE, (k, k)) (OpenCV: dx = cvRound(c * sqrt((r^2 - dy^2) / r^2)),
 // j1 = max(c - dx, 0), j2 = min(c + dx + 1, k)) turned into the chord plan of morph_chord_kernel.
 int build_plan(int k, int th, SEPlan* se) {
@@ -464,6 +695,48 @@ int build_plan(int k, int th, SEPlan* se) {
     return 0;
 }
 
+// The rectangles Y_m x X_m of the k x k ellipse (same cvRound rows as build_plan), widest chord first.  Fails (-1)
+// unless the rows are nested intervals and each Y_m is one contiguous band through the anchor row.
+int build_bands(int k, BandPlan* bp) {
+    if (k < 1 || k > RB_MAX_K) return -1;
+    const int r = k / 2, c = k / 2;
+    const double inv_r2 = r ? 1.0 / ((double)r * r) : 0.0;
+    int lo[RB_MAX_K], hi[RB_MAX_K], order[RB_MAX_K];
+    for (int i = 0; i < k; ++i) {
+        const int dy = i - r;
+        const int dx = (int)nearbyint(c * sqrt(((double)r * r - (double)dy * dy) * inv_r2));   // cvRound
+        const int j1 = c - dx < 0 ? 0 : c - dx;
+        const int j2 = c + dx + 1 > k ? k : c + dx + 1;
+        if (j2 - j1 <= 0) return -1;
+        lo[i] = j1 - c;
+        hi[i] = j2 - 1 - c;
+        order[i] = i;
+    }
+    std::sort(order, order + k, [&](int a, int b) {
+        const int wa = hi[a] - lo[a], wb = hi[b] - lo[b];
+        return wa != wb ? wa > wb : (lo[a] != lo[b] ? lo[a] < lo[b] : a < b);
+    });
+    bp->k = k;
+    bp->nbands = 0;
+    int ya = 1 << 30, yb = -(1 << 30), rows = 0;
+    for (int j = 0; j < k;) {
+        const int a = lo[order[j]], b = hi[order[j]];
+        if (bp->nbands > 0) {
+            const Band& p = bp->band[bp->nbands - 1];
+            if (a < p.xa || b > p.xb) return -1;                       // not nested
+        }
+        for (; j < k && lo[order[j]] == a && hi[order[j]] == b; ++j) {   // rows of exactly this interval
+            ya = std::min(ya, order[j] - c);
+            yb = std::max(yb, order[j] - c);
+            ++rows;
+        }
+        // the rows containing [a, b] are those of this and every wider interval: one band through the anchor
+        if (yb - ya + 1 != rows || ya > 0 || yb < 0 || bp->nbands >= RB_MAX_BANDS) return -1;
+        bp->band[bp->nbands++] = Band{(short)ya, (short)yb, (short)a, (short)b};
+    }
+    return 0;
+}
+
 int plan_groups(const SEPlan& se) { return (se.th == 128 && se.RH <= 192) ? 6 : 8; }     // NA of the instantiation used
 size_t plan_smem_bytes(const SEPlan& se) {
     return ((size_t)se.ntables * se.level_words + 2 * (size_t)(plan_groups(se) * 32) * HP) * 4;
@@ -477,9 +750,9 @@ size_t rolling_ball_workspace_bytes(int planes, int H, int W) {
     return 2 * align256((size_t)planes * H * W) + align256(sizeof(int) * 2 * (size_t)planes);
 }
 
-// Largest radius this build can run: the haloed region of the smallest tile must fit in shared memory and the
+// Largest radius the tiled kernel can run: the haloed region of the smallest tile must fit in shared memory and the
 // per-thread row state covers 256 region rows.
-int rolling_ball_max_radius() {
+int rolling_ball_tiled_max_radius() {
     static int cached = 0;
     if (!cached) {
         int best = 1;
@@ -517,12 +790,100 @@ int rolling_ball_plan_dump(int radius, int th, int* out, int cap) {
     return n;
 }
 
+int rolling_ball_max_radius() { return RB_MAX_K; }
+
+// Host-only dump of the banded pass's rectangles: [k, K, RB_PIECE], then {ya, yb, xa, xb} per rectangle in walk order.
+int rolling_ball_bands_dump(int radius, int* out, int cap) {
+    static BandPlan bp;                       // 8 KB: off the stack (host-only test aid)
+    DC_REQUIRE(out && radius >= 1 && radius <= RB_MAX_K, DC_EINVAL, "dc_debug_rolling_ball_bands: radius %d outside [1,%d]",
+               radius, RB_MAX_K);
+    DC_REQUIRE(build_bands(radius, &bp) == 0, DC_EINVAL, "dc_debug_rolling_ball_bands: no rectangle cover for radius %d", radius);
+    const int need = 3 + 4 * bp.nbands;
+    DC_REQUIRE(cap >= need, DC_EINVAL, "dc_debug_rolling_ball_bands: need %d ints", need);
+    int n = 0;
+    out[n++] = bp.k; out[n++] = bp.nbands; out[n++] = RB_PIECE;
+    for (int m = 0; m < bp.nbands; ++m) {
+        const Band& r = bp.band[m];
+        out[n++] = r.ya; out[n++] = r.yb; out[n++] = r.xa; out[n++] = r.xb;
+    }
+    return n;
+}
+
+static int check_rolling_ball_args(const dc_rolling_ball_args_t* a, const char* who, int max_radius) {
+    DC_REQUIRE(a && a->in && a->out, DC_EINVAL, "%s: null pointer argument", who);
+    DC_REQUIRE(a->B > 0 && a->H > 0 && a->W > 0 && a->C > 0, DC_EINVAL, "%s: bad shape", who);
+    DC_REQUIRE(a->radius >= 1 && a->radius <= max_radius, DC_EINVAL, "%s: radius %d outside [1,%d]", who, a->radius, max_radius);
+    DC_REQUIRE(a->B * a->C <= 65535, DC_EINVAL, "%s: more than 65535 planes in one call", who);
+    DC_REQUIRE(a->workspace && a->workspace_bytes >= rolling_ball_workspace_bytes(a->B * a->C, a->H, a->W), DC_EWORKSPACE,
+               "%s: workspace too small", who);
+    return DC_OK;
+}
+
+// erode in -> er, dilate er -> corr with the subtract and the per-plane min / max, stretch corr -> out: the banded
+// pass in place of the tiled one, same workspace.
+int launch_rolling_ball_banded(const dc_rolling_ball_args_t* a, cudaStream_t stream, const char* who) {
+    int rc = check_rolling_ball_args(a, who, RB_MAX_K);
+    if (rc != DC_OK) return rc;
+    const int planes = a->B * a->C, H = a->H, W = a->W;
+    DC_REQUIRE(W <= DC_ROLLING_BALL_BANDED_MAX_WIDTH, DC_EINVAL,
+               "%s: rows of %d pixels are wider than the %d the banded pass (radius > %d) keeps in shared memory",
+               who, W, DC_ROLLING_BALL_BANDED_MAX_WIDTH, rolling_ball_tiled_max_radius());
+    thread_local BandPlan bp;
+    DC_REQUIRE(build_bands(a->radius, &bp) == 0, DC_EINVAL, "%s: no rectangle cover for radius %d", who, a->radius);
+
+    // shared memory per output row (morph_band_kernel): V, A, P, S and the piece carries
+    const int ww = (W + 3) >> 2;
+    const int vp = 4 * ww;
+    int wmax = 0, cmax = 0;
+    for (int m = 0; m < bp.nbands; ++m) {
+        const int w = bp.band[m].xb - bp.band[m].xa + 1, L = W + w - 1;
+        const int np = (w + RB_PIECE - 1) / RB_PIECE;
+        wmax = std::max(wmax, w);
+        if (np > 1) cmax = std::max(cmax, ((L + w - 1) / w) * np);
+    }
+    const int lp = (vp + wmax + 8 + 15) & ~15;
+    const int cp = (cmax + 15) & ~15;
+    auto smem_of = [&](int T) { return (size_t)T * (2 * (size_t)vp + 2 * (size_t)lp + 2 * (size_t)cp); };
+    // band height: at most RB_TMAX rows, no taller than the image, two blocks per SM where they fit, and enough
+    // blocks for two per SM where the batch allows
+    int T = RB_TMAX;
+    while (T > 1 && T / 2 >= H) T >>= 1;
+    while (T > 1 && (smem_of(T) > 112 * 1024 || (long long)ceil_div(H, T) * planes < 2LL * num_sms())) T >>= 1;
+    const size_t smem = smem_of(T);
+    DC_REQUIRE(smem <= 226 * 1024, DC_EINVAL, "%s: a %d-pixel row does not fit shared memory", who, W);
+
+    char* p = (char*)a->workspace;
+    uint8_t* er = (uint8_t*)p;   p += align256((size_t)planes * H * W);
+    uint8_t* corr = (uint8_t*)p; p += align256((size_t)planes * H * W);
+    int* minmax = (int*)p;
+
+    static unsigned long long attr_done = 0;
+    {
+        int dev = 0;
+        DC_CUDA(cudaGetDevice(&dev));
+        const unsigned long long bit = 1ull << (dev & 63);
+        if (!(__atomic_load_n(&attr_done, __ATOMIC_ACQUIRE) & bit)) {      // per (function, device), once
+            DC_CUDA(cudaFuncSetAttribute(morph_band_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
+            DC_CUDA(cudaFuncSetAttribute(morph_band_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
+            __atomic_fetch_or(&attr_done, bit, __ATOMIC_RELEASE);
+        }
+    }
+    const dim3 grid(ceil_div(H, T), planes);
+    morph_band_kernel<false, false><<<grid, RB_NT, smem, stream>>>(a->in, a->C, er, nullptr, 0, H, W, T, vp, lp, cp, minmax, bp);
+    morph_band_kernel<true, true><<<grid, RB_NT, smem, stream>>>(er, 1, corr, a->in, a->C, H, W, T, vp, lp, cp, minmax, bp);
+    int sblocks = ceil_div(H * W, 256 * 64);
+    if (sblocks > 1024) sblocks = 1024;
+    if (sblocks < 1) sblocks = 1;
+    stretch_kernel<<<dim3(sblocks, planes), 256, 0, stream>>>(corr, a->out, a->C, H, W, minmax);
+    DC_CUDA(cudaGetLastError());
+    return DC_OK;
+}
+
 int launch_rolling_ball(const dc_rolling_ball_args_t* a, cudaStream_t stream) {
     DC_REQUIRE(a && a->in && a->out, DC_EINVAL, "dc_rolling_ball: null pointer argument");
+    if (a->radius > rolling_ball_tiled_max_radius()) return launch_rolling_ball_banded(a, stream, "dc_rolling_ball");
     DC_REQUIRE(a->B > 0 && a->H > 0 && a->W > 0 && a->C > 0, DC_EINVAL, "dc_rolling_ball: bad shape");
-    DC_REQUIRE(a->radius >= 1 && a->radius <= rolling_ball_max_radius(), DC_EINVAL,
-               "dc_rolling_ball: radius %d outside [1,%d] (the haloed tile of a larger element does not fit in shared memory)",
-               a->radius, rolling_ball_max_radius());
+    DC_REQUIRE(a->radius >= 1, DC_EINVAL, "dc_rolling_ball: radius %d outside [1,%d]", a->radius, rolling_ball_max_radius());
     const int planes = a->B * a->C, H = a->H, W = a->W;
     DC_REQUIRE(planes <= 65535, DC_EINVAL, "dc_rolling_ball: more than 65535 planes in one call");
     DC_REQUIRE(a->workspace && a->workspace_bytes >= rolling_ball_workspace_bytes(planes, H, W), DC_EWORKSPACE,

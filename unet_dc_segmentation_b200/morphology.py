@@ -15,8 +15,14 @@ from . import _lib
 
 
 def max_radius() -> int:
-    """Largest background radius the GPU kernel accepts (the haloed tile of the element has to fit in shared memory)."""
+    """Largest background radius the GPU path accepts (2047).  Radii up to ``tiled_max_radius()`` run the tiled
+    chord kernel, larger ones the banded pass, which takes rows of at most 32768 pixels."""
     return int(_lib.load().dc_rolling_ball_max_radius())
+
+
+def tiled_max_radius() -> int:
+    """Largest radius the tiled chord kernel runs (170: the haloed tile of the element has to fit in shared memory)."""
+    return int(_lib.load().dc_rolling_ball_tiled_max_radius())
 
 
 def rolling_ball_workspace_bytes(B: int, H: int, W: int, Cc: int = 1) -> int:
@@ -26,10 +32,12 @@ def rolling_ball_workspace_bytes(B: int, H: int, W: int, Cc: int = 1) -> int:
 
 
 def rolling_ball_device(images: torch.Tensor, radius: int = 50, out: torch.Tensor | None = None,
-                        workspace: torch.Tensor | None = None) -> torch.Tensor:
+                        workspace: torch.Tensor | None = None, method: str = "auto") -> torch.Tensor:
     """images: CUDA u8 [B,H,W] (planar) or [B,H,W,C] (interleaved).  Returns the corrected images, same shape.
 
-    Per plane: opening with cv2's radius x radius ellipse, saturating subtract, min-max stretch to 0..255."""
+    Per plane: opening with cv2's radius x radius ellipse, saturating subtract, min-max stretch to 0..255.
+    method: "auto" (the tiled kernel up to ``tiled_max_radius()``, the banded pass above), "tiled" or "banded"
+    (either kernel on its own; both are bit-exact, so the choice only changes the speed)."""
     _lib.require_cuda(images, "images")
     if images.dtype != torch.uint8:
         raise TypeError("rolling ball works on uint8 images")
@@ -40,11 +48,16 @@ def rolling_ball_device(images: torch.Tensor, radius: int = 50, out: torch.Tenso
         B, H, W, Cc = images.shape
     else:
         raise ValueError(f"expected u8 [B,H,W] or [B,H,W,C], got {tuple(images.shape)}")
+    if method not in ("auto", "tiled", "banded"):
+        raise ValueError(f"method must be 'auto', 'tiled' or 'banded', got {method!r}")
     if not 1 <= int(radius) <= max_radius():
-        raise ValueError(f"radius must be in [1, {max_radius()}] (larger structuring elements do not fit the kernel's "
-                         "shared-memory tile)")
+        raise ValueError(f"radius must be in [1, {max_radius()}] (the structuring element is radius x radius pixels)")
+    if method == "tiled" and int(radius) > tiled_max_radius():
+        raise ValueError(f"method='tiled' takes radius 1..{tiled_max_radius()} (the haloed tile of a larger element does "
+                         "not fit in shared memory); use 'auto' or 'banded'")
     images = images.contiguous()
     lib = _lib.load()
+    entry = lib.dc_rolling_ball_banded if method == "banded" else lib.dc_rolling_ball
     need = rolling_ball_workspace_bytes(B, H, W, Cc)
     dev = images.device
     with torch.cuda.device(dev):
@@ -54,7 +67,7 @@ def rolling_ball_device(images: torch.Tensor, radius: int = 50, out: torch.Tenso
             out = torch.empty_like(images)
         args = _lib.RollingBallArgs(images.data_ptr(), out.data_ptr(), B, H, W, Cc, int(radius),
                                     workspace.data_ptr(), workspace.numel())
-        _lib.check(lib.dc_rolling_ball(C.byref(args), _lib.stream_ptr(dev)))
+        _lib.check(entry(C.byref(args), _lib.stream_ptr(dev)))
     return out
 
 
