@@ -47,9 +47,10 @@ extern "C" {
 #define DC_ECAPACITY (-4) /* droplet table capacity exceeded (counts are still exact) */
 #define DC_EWORKSPACE (-5)
 
-/* Bumped whenever a struct or signature in this header changes; dc_version() returns the value the library was
- * built with and the Python binding refuses to load a library that disagrees. */
-#define DC_ABI_VERSION 206
+/* Bumped whenever a struct or signature in this header changes, or an entry point's return code for some arguments
+ * does; dc_version() returns the value the library was built with and the Python binding refuses to load a library
+ * that disagrees. */
+#define DC_ABI_VERSION 207
 
 const char* dc_last_error(void);
 int dc_version(void);
@@ -225,7 +226,9 @@ int dc_model_destroy(dc_model_t* m);
 int dc_forward_workspace_bytes(const dc_model_t* m, int B, int H, int W, size_t* bytes);
 /* in_kind as dc_stem_args (in_kind 0: fp32 [B,in_channels,H,W]).  prob_out fp32 [B,out_channels,H,W] and/or mask_out
  * u8 [B,H,W] may be NULL.  mask = prob[:, 0] > thresh (fp32 compare, quantify_droplets_batch.py:56). H, W multiples
- * of 16. */
+ * of 16.  Shape limits: the batch has no limit of its own (B > 65535 runs, also through the in_channels /
+ * out_channels != (3, 1) kernels); each layer needs fewer than 2^31 output tiles (DC_EINVAL otherwise).  Element
+ * offsets are 64-bit: a level-0 activation or the unfused [B,H,W,128] skip concatenation may exceed 2^31 elements. */
 int dc_forward(dc_model_t* m, int in_kind, const void* in, int B, int H, int W, float thresh, float* prob_out,
                uint8_t* mask_out, void* workspace, size_t workspace_bytes, void* stream);
 /* number of kernels one dc_forward launches (for bench accounting) */
@@ -257,9 +260,16 @@ typedef struct dc_rolling_ball_args {
  * same workspace, allocate nothing, do not synchronise, and allow out == in. */
 #define DC_ROLLING_BALL_BANDED_MAX_WIDTH 32768
 int dc_rolling_ball_workspace_bytes(int B, int H, int W, int C, size_t* bytes);
+/* Shape limits of all three entry points (DC_EINVAL otherwise): B*C <= 65535 planes, H*W < 2^31 pixels per plane.
+ * The tiled kernel puts rows of tiles (128, 64 or 32 rows, by radius) in gridDim.y; a frame with more than 65535 rows
+ * of tiles (H > 8388480 at radius 50) runs the banded pass, bit for bit the same result. */
 int dc_rolling_ball(const dc_rolling_ball_args_t* args, void* stream);
+/* The tiled kernel alone: radius 1..dc_rolling_ball_tiled_max_radius(), at most 65535 rows of tiles; returns
+ * DC_EINVAL where dc_rolling_ball would hand the frame to the banded pass. */
+int dc_rolling_ball_tiled(const dc_rolling_ball_args_t* args, void* stream);
 /* The banded pass at any radius 1..dc_rolling_ball_max_radius(), also where dc_rolling_ball would run the tiled
- * kernel (the two agree bit for bit); same arguments and workspace as dc_rolling_ball. */
+ * kernel (the two agree bit for bit); same arguments and workspace as dc_rolling_ball.  Any height (row bands go in
+ * gridDim.x); rows of at most DC_ROLLING_BALL_BANDED_MAX_WIDTH pixels. */
 int dc_rolling_ball_banded(const dc_rolling_ball_args_t* args, void* stream);
 /* Largest `radius` dc_rolling_ball accepts: 2047, an element half as wide as a 4096^2 frame. */
 int dc_rolling_ball_max_radius(void);
@@ -288,6 +298,7 @@ typedef struct dc_resize_args {
     int dst_h, dst_w;
 } dc_resize_args_t;
 
+/* Shape limits (DC_EINVAL otherwise): B <= 65535 and dst_h <= 65535 (grid dimensions). */
 int dc_resize_linear_u8(const dc_resize_args_t* args, void* stream);
 
 /* ------------------------------------------------------------------ labelling + droplet table
@@ -314,6 +325,7 @@ typedef struct dc_label_args {
 } dc_label_args_t;
 
 int dc_label_workspace_bytes(int B, int H, int W, size_t* bytes);
+/* Shape limits (DC_EINVAL otherwise): B <= 65535, H*W < 2^31, H <= 65535 * 128 (rows of 128-row tiles in gridDim.y). */
 int dc_label_stats(const dc_label_args_t* args, void* stream);
 
 /* ---- overlay stencil --------------------------------------------------------------------------
@@ -332,6 +344,7 @@ typedef struct dc_overlay_args {
 } dc_overlay_args_t;
 
 int dc_overlay_workspace_bytes(int B, int H, int W, size_t* bytes);
+/* Shape limits as dc_label_stats: B <= 65535, H*W < 2^31, H <= 65535 * 128. */
 int dc_overlay_stencil(const dc_overlay_args_t* args, void* stream);
 
 /* ---- density maps of quantify_pipline.py (the reference's alternate front end) ---------------------------
@@ -351,6 +364,7 @@ typedef struct dc_roi_args {
 } dc_roi_args_t;
 
 int dc_roi_workspace_bytes(int B, int H, int W, size_t* bytes);
+/* Shape limits (DC_EINVAL otherwise): B <= 65535, H <= 65535, H*W < 2^31. */
 int dc_roi_mask(const dc_roi_args_t* args, void* stream);
 
 /* dc_radial_density: get_targets(mask, roi, nb_layers, cy, cx) (quantify_pipline.py:61-91).  The droplet
@@ -371,6 +385,7 @@ typedef struct dc_radial_args {
 } dc_radial_args_t;
 
 int dc_radial_workspace_bytes(int B, size_t* bytes);
+/* Shape limits (DC_EINVAL otherwise): B <= 65535, H*W < 2^31. */
 int dc_radial_density(const dc_radial_args_t* args, void* stream);
 
 /* dc_spatial_density: density_maps(mask, roi, kernel_size) (quantify_pipline.py:93-97):
@@ -390,6 +405,7 @@ typedef struct dc_spatial_args {
 } dc_spatial_args_t;
 
 int dc_spatial_workspace_bytes(int B, int H, int W, size_t* bytes);
+/* Shape limits (DC_EINVAL otherwise): B <= 65535, H <= 65535 * 16 (rows of 16-row tiles in gridDim.y). */
 int dc_spatial_density(const dc_spatial_args_t* args, void* stream);
 
 #ifdef __cplusplus

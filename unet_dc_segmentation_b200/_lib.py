@@ -16,12 +16,12 @@ DC_KIND_CONV3X3, DC_KIND_UPCONV2 = 0, 1
 DC_EPI_STORE, DC_EPI_STORE_POOL, DC_EPI_HEAD, DC_EPI_UPSCATTER = 0, 1, 2, 3
 DC_NUM_LAYERS = 23
 DC_CONV_FAMILY_AUTO, DC_CONV_FAMILY_NO_PAIR, DC_CONV_FAMILY_GENERIC = 0, 1, 2
-ABI_VERSION = 206          # DC_ABI_VERSION of include/unetdc_b200.h these ctypes structures mirror
+ABI_VERSION = 207          # DC_ABI_VERSION of include/unetdc_b200.h these ctypes structures mirror
 
 EXPORTS = [
     "dc_last_error", "dc_version", "dc_device_check", "dc_conv_tc", "dc_conv_upfused", "dc_debug_upfuse_schedule", "dc_debug_set_upfuse_mode", "dc_debug_set_conv_family", "dc_stem", "dc_model_create",
     "dc_model_destroy", "dc_forward_workspace_bytes", "dc_forward", "dc_forward_num_launches", "dc_forward_profile",
-    "dc_rolling_ball_workspace_bytes", "dc_rolling_ball", "dc_rolling_ball_banded", "dc_rolling_ball_max_radius",
+    "dc_rolling_ball_workspace_bytes", "dc_rolling_ball", "dc_rolling_ball_tiled", "dc_rolling_ball_banded", "dc_rolling_ball_max_radius",
     "dc_rolling_ball_tiled_max_radius", "dc_debug_rolling_ball_plan", "dc_debug_rolling_ball_bands", "dc_label_workspace_bytes", "dc_label_stats",
     "dc_resize_linear_u8", "dc_overlay_workspace_bytes", "dc_overlay_stencil",
     "dc_roi_workspace_bytes", "dc_roi_mask", "dc_radial_workspace_bytes", "dc_radial_density",
@@ -179,6 +179,7 @@ def load(build_if_missing: bool = True) -> C.CDLL:
                                        c_void_p, c_size_t, c_void_p, POINTER(c_float)]
     lib.dc_rolling_ball_workspace_bytes.argtypes = [c_int, c_int, c_int, c_int, POINTER(c_size_t)]
     lib.dc_rolling_ball.argtypes = [POINTER(RollingBallArgs), c_void_p]
+    lib.dc_rolling_ball_tiled.argtypes = [POINTER(RollingBallArgs), c_void_p]
     lib.dc_rolling_ball_banded.argtypes = [POINTER(RollingBallArgs), c_void_p]
     lib.dc_rolling_ball_max_radius.argtypes = []
     lib.dc_rolling_ball_tiled_max_radius.argtypes = []

@@ -207,7 +207,13 @@ int dc_debug_rolling_ball_bands(int radius, int* out, int cap) { return rolling_
 int dc_rolling_ball(const dc_rolling_ball_args_t* args, void* stream) {
     int rc = check_current_device(nullptr);
     if (rc != DC_OK) return rc;
-    return launch_rolling_ball(args, (cudaStream_t)stream);
+    return launch_rolling_ball(args, (cudaStream_t)stream, false);
+}
+
+int dc_rolling_ball_tiled(const dc_rolling_ball_args_t* args, void* stream) {
+    int rc = check_current_device(nullptr);
+    if (rc != DC_OK) return rc;
+    return launch_rolling_ball(args, (cudaStream_t)stream, true);
 }
 
 int dc_rolling_ball_banded(const dc_rolling_ball_args_t* args, void* stream) {

@@ -24,7 +24,7 @@ int  cuda_fail(cudaError_t e, const char* what);
         if (!(cond)) { dc::set_error(__VA_ARGS__); return (code); }           \
     } while (0)
 
-static inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
+static inline int ceil_div(int a, int b) { return a / b + (a % b != 0); }   // a >= 0, b > 0; no overflow near INT_MAX
 
 // ---------------------------------------------------------------- launchers implemented per .cu
 // bias_host: optional HOST copy of a->bias (dc_model_create keeps one); layers with Cout == 64 then take their bias
@@ -37,7 +37,7 @@ int set_conv_family(int family);
 int upfuse_schedule(int* out, int cap);
 int set_upfuse_mode(int mode);
 int launch_label_stats(const dc_label_args_t* a, cudaStream_t stream);
-int launch_rolling_ball(const dc_rolling_ball_args_t* a, cudaStream_t stream);
+int launch_rolling_ball(const dc_rolling_ball_args_t* a, cudaStream_t stream, bool tiled_only);
 int launch_rolling_ball_banded(const dc_rolling_ball_args_t* a, cudaStream_t stream, const char* who);
 int launch_resize_linear_u8(const dc_resize_args_t* a, cudaStream_t stream);
 size_t label_workspace_bytes(int B, int H, int W);

@@ -813,10 +813,17 @@ static int check_rolling_ball_args(const dc_rolling_ball_args_t* a, const char* 
     DC_REQUIRE(a && a->in && a->out, DC_EINVAL, "%s: null pointer argument", who);
     DC_REQUIRE(a->B > 0 && a->H > 0 && a->W > 0 && a->C > 0, DC_EINVAL, "%s: bad shape", who);
     DC_REQUIRE(a->radius >= 1 && a->radius <= max_radius, DC_EINVAL, "%s: radius %d outside [1,%d]", who, a->radius, max_radius);
-    DC_REQUIRE(a->B * a->C <= 65535, DC_EINVAL, "%s: more than 65535 planes in one call", who);
+    DC_REQUIRE((long long)a->B * a->C <= 65535, DC_EINVAL, "%s: more than 65535 planes in one call", who);
+    DC_REQUIRE((long long)a->H * a->W < (1ll << 31), DC_EINVAL, "%s: image too large for int32 indices", who);
     DC_REQUIRE(a->workspace && a->workspace_bytes >= rolling_ball_workspace_bytes(a->B * a->C, a->H, a->W), DC_EWORKSPACE,
                "%s: workspace too small", who);
     return DC_OK;
+}
+
+// blocks per plane of the stretch pass: one per 16 K pixels, 1..1024 (the pixel count is up to 2^31 - 1)
+static int stretch_blocks(int H, int W) {
+    const long long n = ((long long)H * W + 256 * 64 - 1) / (256 * 64);
+    return (int)std::min(std::max(n, 1ll), 1024ll);
 }
 
 // erode in -> er, dilate er -> corr with the subtract and the per-plane min / max, stretch corr -> out: the banded
@@ -871,23 +878,20 @@ int launch_rolling_ball_banded(const dc_rolling_ball_args_t* a, cudaStream_t str
     const dim3 grid(ceil_div(H, T), planes);
     morph_band_kernel<false, false><<<grid, RB_NT, smem, stream>>>(a->in, a->C, er, nullptr, 0, H, W, T, vp, lp, cp, minmax, bp);
     morph_band_kernel<true, true><<<grid, RB_NT, smem, stream>>>(er, 1, corr, a->in, a->C, H, W, T, vp, lp, cp, minmax, bp);
-    int sblocks = ceil_div(H * W, 256 * 64);
-    if (sblocks > 1024) sblocks = 1024;
-    if (sblocks < 1) sblocks = 1;
+    const int sblocks = stretch_blocks(H, W);
     stretch_kernel<<<dim3(sblocks, planes), 256, 0, stream>>>(corr, a->out, a->C, H, W, minmax);
     DC_CUDA(cudaGetLastError());
     return DC_OK;
 }
 
-int launch_rolling_ball(const dc_rolling_ball_args_t* a, cudaStream_t stream) {
-    DC_REQUIRE(a && a->in && a->out, DC_EINVAL, "dc_rolling_ball: null pointer argument");
-    if (a->radius > rolling_ball_tiled_max_radius()) return launch_rolling_ball_banded(a, stream, "dc_rolling_ball");
-    DC_REQUIRE(a->B > 0 && a->H > 0 && a->W > 0 && a->C > 0, DC_EINVAL, "dc_rolling_ball: bad shape");
-    DC_REQUIRE(a->radius >= 1, DC_EINVAL, "dc_rolling_ball: radius %d outside [1,%d]", a->radius, rolling_ball_max_radius());
+// tiled_only: dc_rolling_ball_tiled, which refuses what the tiled kernel cannot run instead of handing it to the
+// banded pass (radius > rolling_ball_tiled_max_radius(), more than 65535 rows of tiles)
+int launch_rolling_ball(const dc_rolling_ball_args_t* a, cudaStream_t stream, bool tiled_only) {
+    const char* who = tiled_only ? "dc_rolling_ball_tiled" : "dc_rolling_ball";
+    int rc = check_rolling_ball_args(a, who, tiled_only ? rolling_ball_tiled_max_radius() : RB_MAX_K);
+    if (rc != DC_OK) return rc;
+    if (a->radius > rolling_ball_tiled_max_radius()) return launch_rolling_ball_banded(a, stream, who);
     const int planes = a->B * a->C, H = a->H, W = a->W;
-    DC_REQUIRE(planes <= 65535, DC_EINVAL, "dc_rolling_ball: more than 65535 planes in one call");
-    DC_REQUIRE(a->workspace && a->workspace_bytes >= rolling_ball_workspace_bytes(planes, H, W), DC_EWORKSPACE,
-               "dc_rolling_ball: workspace too small");
     // tile height: the tallest whose haloed region fits twice per SM (else once), within the per-thread row state
     SEPlan se;
     int th = 0;
@@ -898,7 +902,15 @@ int launch_rolling_ball(const dc_rolling_ball_args_t* a, cudaStream_t stream) {
             if (plan_smem_bytes(se) <= (pass == 0 ? 112 * 1024 : 226 * 1024)) th = cand;
             if (cand > 32 && cand / 2 >= H) th = 0;            // a shorter tile already covers the whole image
         }
-    DC_REQUIRE(th > 0 && build_plan(a->radius, th, &se) == 0, DC_EINVAL, "dc_rolling_ball: no tile fits radius %d", a->radius);
+    DC_REQUIRE(th > 0 && build_plan(a->radius, th, &se) == 0, DC_EINVAL, "%s: no tile fits radius %d", who, a->radius);
+    // rows of tiles go in gridDim.y (at most 65535).  A taller frame runs the banded pass, which gives the same
+    // result bit for bit and keeps its row bands in gridDim.x; such a frame has H * W < 2^31 and H > 65535 * 32, so
+    // its rows are narrower than the banded pass's width limit.
+    if (ceil_div(H, th) > 65535) {
+        DC_REQUIRE(!tiled_only, DC_EINVAL, "%s: image too tall (%d rows of %d-row tiles at radius %d; at most 65535)", who,
+                   ceil_div(H, th), th, a->radius);
+        return launch_rolling_ball_banded(a, stream, who);
+    }
     const size_t smem = plan_smem_bytes(se);
 
     char* p = (char*)a->workspace;
@@ -933,9 +945,7 @@ int launch_rolling_ball(const dc_rolling_ball_args_t* a, cudaStream_t stream) {
     DC_MORPH_LAUNCH(4, 6, 31, 3, special) DC_MORPH_LAUNCH(4, 6, 0, 0, !special) DC_MORPH_LAUNCH(4, 8, 0, 0, true)
     DC_MORPH_LAUNCH(2, 8, 0, 0, true) DC_MORPH_LAUNCH(1, 8, 0, 0, true)
 #undef DC_MORPH_LAUNCH
-    int sblocks = ceil_div(H * W, 256 * 64);
-    if (sblocks > 1024) sblocks = 1024;
-    if (sblocks < 1) sblocks = 1;
+    const int sblocks = stretch_blocks(H, W);
     stretch_kernel<<<dim3(sblocks, planes), 256, 0, stream>>>(corr, a->out, a->C, H, W, minmax);
     DC_CUDA(cudaGetLastError());
     return DC_OK;

@@ -36,8 +36,9 @@ def rolling_ball_device(images: torch.Tensor, radius: int = 50, out: torch.Tenso
     """images: CUDA u8 [B,H,W] (planar) or [B,H,W,C] (interleaved).  Returns the corrected images, same shape.
 
     Per plane: opening with cv2's radius x radius ellipse, saturating subtract, min-max stretch to 0..255.
-    method: "auto" (the tiled kernel up to ``tiled_max_radius()``, the banded pass above), "tiled" or "banded"
-    (either kernel on its own; both are bit-exact, so the choice only changes the speed)."""
+    method: "auto" (the tiled kernel up to ``tiled_max_radius()``, the banded pass above and for frames taller than
+    the tiled kernel's grid: more than 65535 rows of tiles), "tiled" or "banded" (either kernel on its own; both are
+    bit-exact, so the choice only changes the speed; "tiled" refuses what it cannot run)."""
     _lib.require_cuda(images, "images")
     if images.dtype != torch.uint8:
         raise TypeError("rolling ball works on uint8 images")
@@ -57,7 +58,7 @@ def rolling_ball_device(images: torch.Tensor, radius: int = 50, out: torch.Tenso
                          "not fit in shared memory); use 'auto' or 'banded'")
     images = images.contiguous()
     lib = _lib.load()
-    entry = lib.dc_rolling_ball_banded if method == "banded" else lib.dc_rolling_ball
+    entry = {"auto": lib.dc_rolling_ball, "tiled": lib.dc_rolling_ball_tiled, "banded": lib.dc_rolling_ball_banded}[method]
     need = rolling_ball_workspace_bytes(B, H, W, Cc)
     dev = images.device
     with torch.cuda.device(dev):
