@@ -50,7 +50,7 @@ extern "C" {
 /* Bumped whenever a struct or signature in this header changes, or an entry point's return code for some arguments
  * does; dc_version() returns the value the library was built with and the Python binding refuses to load a library
  * that disagrees. */
-#define DC_ABI_VERSION 207
+#define DC_ABI_VERSION 208
 
 const char* dc_last_error(void);
 int dc_version(void);
@@ -68,6 +68,17 @@ int dc_device_check(int device, int* sm_count);
  *   DC_KIND_UPCONV2 : w[(a*2 + b)*Cout + co][ci]             bf16, row length Cin
  *                     (a, b = output row / column parity, models/model_2.py:20)
  * bias: fp32 [Cout].
+ *
+ * fp32 precision (planes == 3): every activation tensor holds three bf16 planes hi, mid, lo with x = hi + (mid + lo)
+ * exactly in fp32 (hi = bf16_rn(x), mid = bf16_rn(x - hi), lo = bf16_rn(x - hi - mid)); plane p of a pixel is the
+ * channel range [p * plane_stride, p * plane_stride + C) of its in_stride / out_stride / pool_stride channels.  The
+ * weights (BatchNorm folded in float64, rounded to fp32, then split the same way) carry the planes inside each row:
+ *   DC_KIND_CONV3X3 : w[co][((ky*3 + kx)*3 + plane)*Cin + ci]   bf16, row length 27*Cin
+ *   DC_KIND_UPCONV2 : w[(a*2 + b)*Cout + co][plane*Cin + ci]     bf16, row length 3*Cin
+ * The layer sums the six products a_i * b_j with i + j <= 2 (plane i of the activations, plane j of the weights) in
+ * fp32 in TMEM; bias, ReLU and the 2x2 max are fp32, and the result is split again (the pooled planes are the split
+ * of the max of the four fp32 values).  HEAD reads the fp32 accumulator as in the bf16 path.  Always the per-tap
+ * kernel: weight_par is ignored.
  */
 enum { DC_KIND_CONV3X3 = 0, DC_KIND_UPCONV2 = 1 };
 enum {
@@ -103,6 +114,12 @@ typedef struct dc_conv_args {
      * runs per output parity class with windows shared between classes (see dc_conv_upfused); NULL = the generic
      * kernels from `weight`. */
     const void* weight_par;
+    /* 0 or 1: bf16 activations and weights (everything above).  3: fp32 precision as described above; the strides
+     * below are in channels, and out_plane_stride / pool_plane_stride are read only by the epilogues that store. */
+    int planes;
+    int in_plane_stride;
+    int out_plane_stride;
+    int pool_plane_stride;
 } dc_conv_args_t;
 
 int dc_conv_tc(const dc_conv_args_t* args, void* stream);
@@ -219,7 +236,17 @@ typedef struct dc_model_desc {
     /* Optional: weights of enc1.3 ([0]) and dec1.3 ([1]) in the dc_conv_args.weight_par layout (used when
      * dilations[0] == 1); NULL = weight[1] / weight[21] through the generic kernels. */
     const void* par_weight[2];
+    /* DC_PRECISION_BF16 (0): activations and weights in bf16, the schedule described above.  DC_PRECISION_FP32: every
+     * activation stored as three bf16 planes and every product formed to about 2^-24 relative (see dc_conv_args.planes),
+     * fp32 accumulation, fp32 head; about six times the MMAs and three times the workspace of the unfused bf16 forward.
+     * Then weight[0] is the enc1.0 weights in the split DC_KIND_CONV3X3 layout over 64 input channels (channels >=
+     * in_channels zero), weight[1..21] the split layouts above (biases fp32 as before), and every in_kind goes through
+     * an input kernel that writes the three planes (u8 as u8 / 255 in IEEE fp32, fp32 split as it is).  The fused and
+     * parity blobs must be NULL (DC_EINVAL otherwise): the fp32 forward runs every layer on the per-tap kernel. */
+    int precision;
 } dc_model_desc_t;
+
+enum { DC_PRECISION_BF16 = 0, DC_PRECISION_FP32 = 1 };
 
 int dc_model_create(dc_model_t** out, int device, const dc_model_desc_t* desc);
 int dc_model_destroy(dc_model_t* m);

@@ -16,7 +16,8 @@ DC_KIND_CONV3X3, DC_KIND_UPCONV2 = 0, 1
 DC_EPI_STORE, DC_EPI_STORE_POOL, DC_EPI_HEAD, DC_EPI_UPSCATTER = 0, 1, 2, 3
 DC_NUM_LAYERS = 23
 DC_CONV_FAMILY_AUTO, DC_CONV_FAMILY_NO_PAIR, DC_CONV_FAMILY_GENERIC = 0, 1, 2
-ABI_VERSION = 207          # DC_ABI_VERSION of include/unetdc_b200.h these ctypes structures mirror
+DC_PRECISION_BF16, DC_PRECISION_FP32 = 0, 1
+ABI_VERSION = 208          # DC_ABI_VERSION of include/unetdc_b200.h these ctypes structures mirror
 
 EXPORTS = [
     "dc_last_error", "dc_version", "dc_device_check", "dc_conv_tc", "dc_conv_upfused", "dc_debug_upfuse_schedule", "dc_debug_set_upfuse_mode", "dc_debug_set_conv_family", "dc_stem", "dc_model_create",
@@ -47,6 +48,7 @@ class ConvArgs(Structure):
         ("head_w", c_void_p), ("head_b", c_float), ("thresh", c_float),
         ("prob_out", c_void_p), ("mask_out", c_void_p),
         ("weight_par", c_void_p),
+        ("planes", c_int), ("in_plane_stride", c_int), ("out_plane_stride", c_int), ("pool_plane_stride", c_int),
     ]
 
 
@@ -65,6 +67,7 @@ class ModelDesc(Structure):
         ("fused_weight1", c_void_p), ("fused_bias1", c_void_p),
         ("fused_wide_x", c_void_p * 3), ("fused_wide_s", c_void_p * 3), ("fused_wide_b", c_void_p * 3),
         ("par_weight", c_void_p * 2),
+        ("precision", c_int),
     ]
 
 

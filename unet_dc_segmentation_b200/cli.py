@@ -301,6 +301,9 @@ def build_parser() -> argparse.ArgumentParser:
                    help="run the reference-shaped per-image loop (preprocess / run_batch) instead of the batched pipeline")
     p.add_argument("--img_size", type=int, default=IMG_SIZE,
                    help="network input size (reference constant IMG_SIZE = 512); use the frame size for native-resolution inference")
+    p.add_argument("--precision", choices=("bf16", "fp32"), default="bf16",
+                   help="fp32: activations and weights to fp32 accuracy (about six times the tensor-core work), for "
+                        "masks and counts that match the reference's fp32 network")
     return p
 
 
@@ -324,6 +327,7 @@ def main(argv=None) -> int:
         overlay_dir.mkdir(exist_ok=True)
 
     model = load_model(args.ckpt_path)
+    model.precision = args.precision
     images = sorted(p for p in in_dir.iterdir() if p.suffix.lower() in SUFFIXES)
     from . import shard
     mine = shard.shard_indices(len(images), rank, world)

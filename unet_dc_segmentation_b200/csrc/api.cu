@@ -67,11 +67,14 @@ struct dc_model {
     bool fused1;             // upconv1 + dec1.0 as one launch (desc.fused_weight1)
     bool fused[4];           // [l]: upconv{l+1} + dec{l+1}.0 as one launch ([0] == fused1)
     float fused_bias9[9 * 64];
+    int planes;              // 3 under DC_PRECISION_FP32 (every activation as three bf16 planes), else 1
 };
 
 namespace {
 
-// Activation buffers of one forward, carved out of the caller's workspace (all bf16 NHWC).
+// Activation buffers of one forward, carved out of the caller's workspace (all bf16 NHWC; with `planes` = 3 every pixel
+// holds the three planes of its channels one after the other, and cat[l] is [up_0 enc_0 up_1 enc_1 up_2 enc_2] so that
+// plane p of a decoder input is one contiguous channel range).
 struct ForwardBuffers {
     char* a[5];      // first-conv output of enc1..enc4 / bottleneck
     char* ad[4];     // dec{l}.0 output
@@ -91,7 +94,7 @@ struct ForwardBuffers {
 // fused[l] (upconv{l+1} + dec{l+1}.0 as one launch, at the number of the dec launch): cat[l] holds only the skip half,
 // and the transposed conv's input is read by the launch that writes ad[l], so it has to live one launch longer.
 ForwardBuffers carve(char* base, int B, int H, int W, bool generic_in = false, bool generic_out = false,
-                     const bool* fused = nullptr) {
+                     const bool* fused = nullptr, int planes = 1) {
     const bool none[4] = {false, false, false, false};
     if (!fused) fused = none;
     ForwardBuffers f;
@@ -100,7 +103,7 @@ ForwardBuffers carve(char* base, int B, int H, int W, bool generic_in = false, b
     Item items[24];
     int n = 0;
     auto add = [&](char** slot, size_t elems, int t0, int t1) {
-        Item it = {align256(elems * 2), t0, t1, slot, 0};
+        Item it = {align256(elems * 2 * planes), t0, t1, slot, 0};
         items[n++] = it;
     };
     if (generic_in) add(&f.xin, (size_t)B * H * W * 64, -1, 0);
@@ -304,12 +307,22 @@ int dc_model_create(dc_model_t** out, int device, const dc_model_desc_t* desc) {
                    desc->dilations[i]);
     const int cin = desc->in_channels > 0 ? desc->in_channels : 3, cout = desc->out_channels > 0 ? desc->out_channels : 1;
     DC_REQUIRE(cin <= 64 && cout <= 64, DC_EINVAL, "dc_model_create: in_channels %d / out_channels %d (at most 64)", cin, cout);
+    DC_REQUIRE(desc->precision == DC_PRECISION_BF16 || desc->precision == DC_PRECISION_FP32, DC_EINVAL,
+               "dc_model_create: precision %d", desc->precision);
+    if (desc->precision == DC_PRECISION_FP32) {
+        bool any = desc->fused_weight1 || desc->fused_bias1 || desc->par_weight[0] || desc->par_weight[1];
+        for (int i = 0; i < 3; ++i) any = any || desc->fused_wide_x[i] || desc->fused_wide_s[i] || desc->fused_wide_b[i];
+        DC_REQUIRE(!any, DC_EINVAL,
+                   "dc_model_create: DC_PRECISION_FP32 runs every layer on the per-tap kernel; the fused and parity "
+                   "blobs must be NULL");
+    }
     dc_model* m = new (std::nothrow) dc_model;
     DC_REQUIRE(m, DC_EINVAL, "dc_model_create: out of host memory");
     m->device = device;
     m->desc = *desc;
     m->cin = cin;
     m->cout = cout;
+    m->planes = desc->precision == DC_PRECISION_FP32 ? 3 : 1;
     cudaError_t e = cudaMemcpy(&m->head_b, desc->bias[22], sizeof(float), cudaMemcpyDeviceToHost);
     if (e != cudaSuccess) {
         delete m;
@@ -356,14 +369,14 @@ int dc_forward_workspace_bytes(const dc_model_t* m, int B, int H, int W, size_t*
     DC_REQUIRE(m && bytes, DC_EINVAL, "dc_forward_workspace_bytes: null argument");
     DC_REQUIRE(B > 0 && H > 0 && W > 0 && H % 16 == 0 && W % 16 == 0, DC_EINVAL,
                "dc_forward: H and W must be positive multiples of 16 (got %d x %d x %d)", B, H, W);
-    *bytes = carve(nullptr, B, H, W, m->cin != 3, m->cout != 1, m->fused).total;
+    *bytes = carve(nullptr, B, H, W, m->cin != 3 || m->planes == 3, m->cout != 1, m->fused, m->planes).total;
     return DC_OK;
 }
 
 int dc_forward_num_launches(const dc_model_t* m) {
-    // stem + 17 conv3x3 + 4 upconv (+ the input conversion / the 1x1 head kernel for other channel counts), minus one per
-    // decoder level whose upconv is composed into the following conv
-    int n = 22 + (m && m->cin != 3 ? 1 : 0) + (m && m->cout != 1 ? 1 : 0);
+    // stem + 17 conv3x3 + 4 upconv (+ the input conversion / the 1x1 head kernel for other channel counts or fp32
+    // precision), minus one per decoder level whose upconv is composed into the following conv
+    int n = 22 + (m && (m->cin != 3 || m->planes == 3) ? 1 : 0) + (m && m->cout != 1 ? 1 : 0);
     for (int l = 0; m && l < 4; ++l) n -= m->fused[l] ? 1 : 0;
     return n;
 }
@@ -382,25 +395,31 @@ static int forward_impl(dc_model_t* m, int in_kind, const void* in, int B, int H
     int dev = -1;
     DC_CUDA(cudaGetDevice(&dev));
     DC_REQUIRE(dev == m->device, DC_EINVAL, "dc_forward: model lives on device %d, current device is %d", m->device, dev);
-    const bool gen_in = m->cin != 3, gen_out = m->cout != 1;
-    DC_REQUIRE(!gen_in || in_kind == 0, DC_EINVAL, "dc_forward: u8 inputs need in_channels == 3 (model has %d)", m->cin);
-    ForwardBuffers f = carve((char*)workspace, B, H, W, gen_in, gen_out, m->fused);
+    const int P = m->planes;
+    const bool gen_in = m->cin != 3 || P == 3, gen_out = m->cout != 1;
+    DC_REQUIRE(m->cin == 3 || in_kind == 0, DC_EINVAL, "dc_forward: u8 inputs need in_channels == 3 (model has %d)", m->cin);
+    ForwardBuffers f = carve((char*)workspace, B, H, W, gen_in, gen_out, m->fused, P);
     DC_REQUIRE(workspace_bytes >= f.total, DC_EWORKSPACE, "dc_forward: workspace too small (%zu < %zu)", workspace_bytes,
                f.total);
     DC_REQUIRE(((uintptr_t)workspace & 255) == 0, DC_EINVAL, "dc_forward: workspace must be 256-byte aligned");
     cudaStream_t stream = (cudaStream_t)stream_;
     const dc_model_desc_t& d = m->desc;
 
+    // strides are those of one plane; with P = 3 planes a pixel holds P times as many channels, planes one stride apart
     auto conv = [&](int layer, int kind, int epi, int relu, int h, int w, int cin, int cout, int dil, const void* src,
                     int src_stride, void* dst, int dst_stride, int dst_off, void* pool) -> int {
         dc_conv_args_t a;
         memset(&a, 0, sizeof(a));
         a.kind = kind; a.epilogue = epi; a.relu = relu;
         a.B = B; a.H = h; a.W = w; a.Cin = cin; a.Cout = cout; a.dilation = dil;
-        a.in = src; a.in_stride = src_stride;
+        a.in = src; a.in_stride = src_stride * P;
         a.weight = d.weight[layer]; a.bias = d.bias[layer];
-        a.out = dst; a.out_stride = dst_stride; a.out_offset = dst_off;
-        a.pool_out = pool; a.pool_stride = cout;
+        a.out = dst; a.out_stride = dst_stride * P; a.out_offset = dst_off;
+        a.pool_out = pool; a.pool_stride = cout * P;
+        if (P == 3) {
+            a.planes = 3;
+            a.in_plane_stride = src_stride; a.out_plane_stride = dst_stride; a.pool_plane_stride = cout;
+        }
         if (layer == 1) a.weight_par = d.par_weight[0];        // launch_conv_tc takes it only when dilation == 1
         if (layer == 21) a.weight_par = d.par_weight[1];
         if (epi == DC_EPI_HEAD) {
@@ -423,7 +442,10 @@ static int forward_impl(dc_model_t* m, int in_kind, const void* in, int B, int H
     } while (0)
 
     // encoder (model_2.py:58-61) -- layer ids per include/unetdc_b200.h
-    if (gen_in) {
+    if (P == 3) {
+        DC_TRY(launch_split_input(in, in_kind, m->cin, f.xin, B, H, W, stream));
+        DC_TRY(conv(0, DC_KIND_CONV3X3, DC_EPI_STORE, 1, H, W, 64, 64, d.dilations[0], f.xin, 64, f.a[0], 64, 0, nullptr));
+    } else if (gen_in) {
         DC_TRY(launch_pad_input((const float*)in, f.xin, B, m->cin, H, W, stream));
         DC_TRY(conv(0, DC_KIND_CONV3X3, DC_EPI_STORE, 1, H, W, 64, 64, d.dilations[0], f.xin, 64, f.a[0], 64, 0, nullptr));
     } else {
@@ -480,7 +502,7 @@ static int forward_impl(dc_model_t* m, int in_kind, const void* in, int B, int H
         } else {
             DC_TRY(conv(base + 2, DC_KIND_CONV3X3, DC_EPI_STORE, 1, h, w, c, c, 1, f.ad[l], c, f.feat, c, 0, nullptr));
             DC_TRY(launch_head1x1(f.feat, (const float*)d.weight[22], d.bias[22], prob_out, mask_out, thresh, B, m->cout, H, W,
-                                  stream));
+                                  stream, P));
         }
     }
 #undef DC_TRY

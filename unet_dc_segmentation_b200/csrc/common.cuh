@@ -56,8 +56,10 @@ int rolling_ball_plan_dump(int radius, int th, int* out, int cap);
 int rolling_ball_bands_dump(int radius, int* out, int cap);
 int num_sms();
 int launch_pad_input(const float* in, void* out_nhwc64, int B, int C, int H, int W, cudaStream_t stream);
+int launch_split_input(const void* in, int in_kind, int C, void* out_planes, int B, int H, int W, cudaStream_t stream);
+// planes 3: the feature map is [B,H,W][3][64] (DC_PRECISION_FP32), else bf16 [B,H,W,64]
 int launch_head1x1(const void* feat_nhwc64, const float* w, const float* b, float* prob, uint8_t* mask, float thresh, int B,
-                   int OC, int H, int W, cudaStream_t stream);
+                   int OC, int H, int W, cudaStream_t stream, int planes = 1);
 
 #ifdef __CUDACC__
 // ---------------------------------------------------------------- PTX wrappers (sm_100a)

@@ -30,6 +30,8 @@
 //   conv_halo2_kernel  the same on a CTA pair (cta_group::2): M = 256 MMAs over two SMs, each SM holds half of the
 //                      weight rows and its own pixel tile.  Runs every 3x3 layer with dilation <= 4.
 //   stem_tc_kernel     first layer (Cin = 3): im2col tile built by producer warps, K = 9 -> 16 or 27 -> 32.
+//   conv_tc_split_kernel  the generic kernel on fp32 values held as three bf16 planes (UNetDC.precision = "fp32"):
+//                      six plane products per (tap, chunk), every layer of that forward.
 //
 // Warp roles (384 threads, 1 CTA / SM, persistent over tiles):
 //   warp 0 : TMA producer           warp 1 : tcgen05.mma issuer       (warp-uniform loops, one elected lane issues)
@@ -111,6 +113,8 @@ struct alignas(64) ConvParams {
     // parity-class kernels: 1 = p.bias is row 4 of a [9][Cout] border-class table (upconv folded in)
     int border_bias;
     int real_ntiles;                // conv_upfused_wide_kernel: n-tiles of Cout (p.n_tiles also counts the class groups)
+    // conv_tc_split_kernel only: channel distance between the bf16 planes of the input, output and pooled output
+    int in_plane_stride, out_plane_stride, pool_plane_stride;
 };
 
 struct TileCoord {
@@ -215,13 +219,27 @@ __device__ __forceinline__ void release_accumulator(uint64_t* bar, int lane) {
     }
 }
 
+// fp32 precision (dc_conv_args.planes == 3): the value is stored as three bf16 planes hi + mid + lo, each the
+// round-to-nearest bf16 of what the planes before it leave (exact residuals in fp32).  Term t of the six products
+// a_i * b_j (i + j <= 2) of a split layer takes activation plane SPLIT_PLANE_A(t) and weight plane SPLIT_PLANE_B(t):
+// (0,0) (0,1) (0,2) (1,0) (1,1) (2,0); a1 b2, a2 b1 and a2 b2 are below one fp32 rounding of the product.
+__host__ __device__ constexpr int split_plane_a(int t) { return (0x940 >> (2 * t)) & 3; }
+__host__ __device__ constexpr int split_plane_b(int t) { return (0x124 >> (2 * t)) & 3; }
+constexpr int SPLIT_TERMS = 6;
+static_assert(split_plane_a(3) == 1 && split_plane_b(2) == 2 && split_plane_a(5) == 2 && split_plane_b(4) == 1, "terms");
+
+__device__ __forceinline__ float bf16_lo_f(uint32_t v) { return __uint_as_float(v << 16); }
+__device__ __forceinline__ float bf16_hi_f(uint32_t v) { return __uint_as_float(v & 0xFFFF0000u); }
+
 // UPF (conv_upfused2_kernel): the tile is TH x TW pixels of the HALF-resolution grid and the NHALF = 4 accumulators are
 // the four output parities (py, px) = (half / 2, half % 2): pixel (h, w) of accumulator `half` is output pixel
 // (2h + py, 2w + px); p.H, p.W are the half-resolution shape and the bias depends on the border class of the pixel.
-template <int BN, int TH, int TW, int NHALF = 1, bool PAIR = false, bool COOP = true, bool UPF = false>
+// SPLIT (conv_tc_split_kernel only): fp32 values stored as three bf16 planes, see split_plane_a.
+template <int BN, int TH, int TW, int NHALF = 1, bool PAIR = false, bool COOP = true, bool UPF = false, bool SPLIT = false>
 __device__ __forceinline__ void run_epilogue(const ConvParams& p, const int e, const int lane, const int group,
                                              const uint32_t tmem_base, uint64_t* tfull_bar, uint64_t* tempty_bar,
                                              const float* bias_s, uint8_t* stg_all) {
+    static_assert(!SPLIT || (TH == 8 && TW == 16 && NHALF == 1 && !PAIR && COOP && !UPF), "split epilogue: generic tiles only");
     const int L = e * 32 + lane;                               // e == warp % 4: TMEM lanes [32e, 32e+32)
     const int lh = L / TW, lw = L % TW;
     const float* head_s = bias_s + p.Cout;                     // out_conv weights follow the bias (HEAD only)
@@ -406,6 +424,66 @@ __device__ __forceinline__ void run_epilogue(const ConvParams& p, const int e, c
                     for (int k = 0; k < 32; ++k) x[k] += __ldg(bc + k) - __ldg(b4 + k);
                 }
             }
+            if constexpr (SPLIT) {
+                if (p.relu) {
+#pragma unroll
+                    for (int k = 0; k < 32; ++k) x[k] = fmaxf(x[k], 0.f);
+                }
+                if (p.epilogue == DC_EPI_STORE_POOL) {
+                    // 2x2 max of the fp32 values, then split: a max per plane is not the max of the sums.  Pixel
+                    // (row, col) of this warp's two rows is lane row * 16 + col, so the window of pooled pixel (e, pc)
+                    // is lanes 2 pc, 2 pc + 1, 2 pc + 16, 2 pc + 17 and lane 2 pc stores it.
+                    const int pc = (lane >> 1) & 7;
+                    const bool pown = (lane & 17) == 0 && (2 * e < hmax) && (2 * pc < p.W - t.w0);
+                    __nv_bfloat16* const pdst = p.pool_out + (ptile_off + ((long long)e * (p.W >> 1) + pc) * p.pool_stride + c0);
+#pragma unroll
+                    for (int g = 0; g < 4; ++g) {
+                        float m[8];
+#pragma unroll
+                        for (int k = 0; k < 8; ++k) {
+                            const float a = fmaxf(x[8 * g + k], __shfl_xor_sync(0xffffffffu, x[8 * g + k], 1));
+                            m[k] = fmaxf(a, __shfl_xor_sync(0xffffffffu, a, 16));
+                        }
+#pragma unroll
+                        for (int pl = 0; pl < 3; ++pl) {
+                            uint32_t q[4];
+#pragma unroll
+                            for (int k = 0; k < 4; ++k) {
+                                q[k] = pack_bf16(m[2 * k], m[2 * k + 1]);
+                                m[2 * k] -= bf16_lo_f(q[k]);
+                                m[2 * k + 1] -= bf16_hi_f(q[k]);
+                            }
+                            if (pown)
+                                *reinterpret_cast<uint4*>(pdst + (8 * g + (long long)pl * p.pool_plane_stride)) =
+                                    make_uint4(q[0], q[1], q[2], q[3]);
+                        }
+                    }
+                }
+                // plane pl = round-to-nearest bf16 of what planes 0..pl-1 leave of x; each through the staged transpose
+#pragma unroll 1
+                for (int pl = 0; pl < 3; ++pl) {
+                    uint32_t pk[16];
+#pragma unroll
+                    for (int k = 0; k < 16; ++k) {
+                        pk[k] = pack_bf16(x[2 * k], x[2 * k + 1]);
+                        x[2 * k] -= bf16_lo_f(pk[k]);
+                        x[2 * k + 1] -= bf16_hi_f(pk[k]);
+                    }
+#pragma unroll
+                    for (int q = 0; q < 4; ++q)
+                        *reinterpret_cast<uint4*>(stg + stg_off(lane, q)) = make_uint4(pk[4 * q], pk[4 * q + 1], pk[4 * q + 2], pk[4 * q + 3]);
+                    __syncwarp();
+                    __nv_bfloat16* const pdst = dst + (long long)pl * p.out_plane_stride;
+#pragma unroll
+                    for (int r = 0; r < 4; ++r) {
+                        const uint4 val = *reinterpret_cast<const uint4*>(stg + stg_off(8 * r + (lane >> 2), sq));
+                        const long long d = (r & 1) * 8 * cs + (r >> 1) * rs;
+                        if (vmask & (1u << r)) *reinterpret_cast<uint4*>(pdst + d) = val;
+                    }
+                    __syncwarp();
+                }
+                continue;
+            }
             uint32_t pk[16];
             if (p.relu) {
 #pragma unroll
@@ -472,8 +550,10 @@ __device__ __forceinline__ void stage_bias(const ConvParams& p, float* bias_s) {
         for (int i = threadIdx.x; i < p.Cout; i += blockDim.x) bias_s[p.Cout + i] = p.head_w[i];
 }
 
-template <int BN, int NSTAGES>
-__global__ void __launch_bounds__(NUM_THREADS, 1) conv_tc_kernel(const __grid_constant__ ConvParams p) {
+// The body of conv_tc_kernel (bf16) and conv_tc_split_kernel (fp32 precision: the K walk of every tap is (term,
+// 64-channel chunk) over the six terms of split_plane_a, and the epilogue stores three planes).
+template <int BN, int NSTAGES, bool SPLIT>
+__device__ __forceinline__ void conv_tc_body(const ConvParams& p) {
     constexpr int B_STAGE_BYTES = BN * KCHUNK * 2;
     constexpr int STAGE_BYTES = A_STAGE_BYTES + B_STAGE_BYTES;
     constexpr int TMEM_COLS = 2 * BN;   // 128 / 256 / 512: a power of two >= 32
@@ -518,13 +598,22 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) conv_tc_kernel(const __grid_co
             for (int tap = 0; tap < p.ntaps; ++tap) {
                 int dy, dx;
                 if (!tap_offset(p, t, tap, dy, dx)) continue;
-                for (int kc = 0; kc < p.kchunks; ++kc) {
+                for (int kc = 0; kc < (SPLIT ? SPLIT_TERMS * p.kchunks : p.kchunks); ++kc) {
                     mbar_wait(&empty_bar[stage], phase ^ 1u);
                     if (elect_one()) {
                         uint8_t* sa = smem + stage * STAGE_BYTES;
                         mbar_expect_tx(&full_bar[stage], STAGE_BYTES);
-                        tma_load_4d(sa, &p.tmA, &full_bar[stage], kc * KCHUNK, t.w0 + dx, t.h0 + dy, t.img);
-                        tma_load_2d(sa + A_STAGE_BYTES, &p.tmB, &full_bar[stage], tap * p.Cin + kc * KCHUNK, t.n0);
+                        if constexpr (SPLIT) {
+                            // weights [Cout][9 taps][3 planes][Cin]: column tap * 3 Cin + plane * Cin + channel
+                            const int term = kc / p.kchunks, ch = (kc - term * p.kchunks) * KCHUNK;
+                            tma_load_4d(sa, &p.tmA, &full_bar[stage], split_plane_a(term) * p.in_plane_stride + ch, t.w0 + dx,
+                                        t.h0 + dy, t.img);
+                            tma_load_2d(sa + A_STAGE_BYTES, &p.tmB, &full_bar[stage], (3 * tap + split_plane_b(term)) * p.Cin + ch,
+                                        t.n0);
+                        } else {
+                            tma_load_4d(sa, &p.tmA, &full_bar[stage], kc * KCHUNK, t.w0 + dx, t.h0 + dy, t.img);
+                            tma_load_2d(sa + A_STAGE_BYTES, &p.tmB, &full_bar[stage], tap * p.Cin + kc * KCHUNK, t.n0);
+                        }
                     }
                     __syncwarp();
                     if (++stage == NSTAGES) { stage = 0; phase ^= 1u; }
@@ -548,7 +637,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) conv_tc_kernel(const __grid_co
             for (int tap = 0; tap < p.ntaps; ++tap) {
                 int dy, dx;
                 if (!tap_offset(p, t, tap, dy, dx)) continue;
-                for (int kc = 0; kc < p.kchunks; ++kc) {
+                for (int kc = 0; kc < (SPLIT ? SPLIT_TERMS * p.kchunks : p.kchunks); ++kc) {
                     mbar_wait(&full_bar[stage], phase);
                     tc_fence_after();
                     const uint32_t sa = smem_u32(smem + stage * STAGE_BYTES);
@@ -573,7 +662,8 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) conv_tc_kernel(const __grid_co
         }
     } else if (warp >= EPI_WARP0) {
         // ------------------------------------------------------------------ epilogue
-        run_epilogue<BN, TILE_H, TILE_W>(p, warp & 3, lane, (warp - EPI_WARP0) >> 2, tmem_base, tfull_bar, tempty_bar, bias_s, stg_s);
+        run_epilogue<BN, TILE_H, TILE_W, 1, false, true, false, SPLIT>(p, warp & 3, lane, (warp - EPI_WARP0) >> 2, tmem_base,
+                                                                       tfull_bar, tempty_bar, bias_s, stg_s);
     }
 
     tc_fence_before();
@@ -582,6 +672,16 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) conv_tc_kernel(const __grid_co
         tc_fence_after();
         tmem_dealloc(tmem_base, TMEM_COLS);
     }
+}
+
+template <int BN, int NSTAGES>
+__global__ void __launch_bounds__(NUM_THREADS, 1) conv_tc_kernel(const __grid_constant__ ConvParams p) {
+    conv_tc_body<BN, NSTAGES, false>(p);
+}
+
+template <int BN, int NSTAGES>
+__global__ void __launch_bounds__(NUM_THREADS, 1) conv_tc_split_kernel(const __grid_constant__ ConvParams p) {
+    conv_tc_body<BN, NSTAGES, true>(p);
 }
 
 // ---------------------------------------------------------------------------- halo variant
@@ -1877,16 +1977,17 @@ int encode_map(CUtensorMap* m, const void* base, int rank, const cuuint64_t* dim
     return DC_OK;
 }
 
-template <int BN, int NSTAGES>
+template <int BN, int NSTAGES, bool SPLIT = false>
 int launch_variant(const ConvParams& p, cudaStream_t stream) {
     constexpr int STAGE_BYTES = A_STAGE_BYTES + BN * KCHUNK * 2;
     constexpr size_t SMEM = (size_t)NSTAGES * STAGE_BYTES + 1024 /* alignment slack */ + 256 /* barriers */ +
                             4096 + 256 /* bias (<= 1024 ch) + out_conv weights */ + EPI_STAGE_TOTAL;
     static_assert(SMEM <= 227 * 1024, "stage ring exceeds shared memory");
     static unsigned long long attr_done = 0;
-    { int rc = set_max_smem_once(conv_tc_kernel<BN, NSTAGES>, (int)SMEM, &attr_done); if (rc != DC_OK) return rc; }
+    void (*kernel)(ConvParams) = SPLIT ? conv_tc_split_kernel<BN, NSTAGES> : conv_tc_kernel<BN, NSTAGES>;
+    { int rc = set_max_smem_once(kernel, (int)SMEM, &attr_done); if (rc != DC_OK) return rc; }
     int grid = p.total_tiles < num_sms() ? p.total_tiles : num_sms();
-    conv_tc_kernel<BN, NSTAGES><<<grid, NUM_THREADS, SMEM, stream>>>(p);
+    kernel<<<grid, NUM_THREADS, SMEM, stream>>>(p);
     DC_CUDA(cudaGetLastError());
     return DC_OK;
 }
@@ -1985,8 +2086,25 @@ int launch_conv_tc(const dc_conv_args_t* a, cudaStream_t stream, const float* bi
                    DC_EINVAL, "dc_conv_tc: pool_out / pool_stride");
         DC_REQUIRE(a->H % 2 == 0 && a->W % 2 == 0, DC_EINVAL, "dc_conv_tc: pooled layer needs even H, W");
     }
-    if (!up && a->weight_par && a->Cin == 64 && a->Cout == 64 && a->dilation == 1 && a->H % 2 == 0 && a->W % 2 == 0 &&
-        g_kernel_family == DC_CONV_FAMILY_AUTO)
+    // fp32 precision: three bf16 planes per tensor, `*_plane_stride` channels apart within a pixel; always the per-tap
+    // kernel (conv_tc_split_kernel)
+    DC_REQUIRE(a->planes == 0 || a->planes == 1 || a->planes == 3, DC_EINVAL, "dc_conv_tc: planes %d (1 or 3)", a->planes);
+    const bool split = a->planes == 3;
+    if (split) {
+        DC_REQUIRE(a->in_plane_stride >= a->Cin && a->in_plane_stride % 8 == 0 && a->in_stride >= 2 * a->in_plane_stride + a->Cin,
+                   DC_EINVAL, "dc_conv_tc: in_plane_stride %d with in_stride %d", a->in_plane_stride, a->in_stride);
+        if (a->epilogue != DC_EPI_HEAD)
+            DC_REQUIRE(a->out_plane_stride >= a->Cout && a->out_plane_stride % 8 == 0 &&
+                           a->out_stride >= a->out_offset + 2 * a->out_plane_stride + a->Cout,
+                       DC_EINVAL, "dc_conv_tc: out_plane_stride %d with out_stride %d / out_offset %d", a->out_plane_stride,
+                       a->out_stride, a->out_offset);
+        if (a->epilogue == DC_EPI_STORE_POOL)
+            DC_REQUIRE(a->pool_plane_stride >= a->Cout && a->pool_plane_stride % 8 == 0 &&
+                           a->pool_stride >= 2 * a->pool_plane_stride + a->Cout,
+                       DC_EINVAL, "dc_conv_tc: pool_plane_stride %d with pool_stride %d", a->pool_plane_stride, a->pool_stride);
+    }
+    if (!split && !up && a->weight_par && a->Cin == 64 && a->Cout == 64 && a->dilation == 1 && a->H % 2 == 0 &&
+        a->W % 2 == 0 && g_kernel_family == DC_CONV_FAMILY_AUTO)
         return launch_conv_par(a, stream, bias_host);
     const int gemm_n = up ? 4 * a->Cout : a->Cout;      // upconv: the four output parities are one wide GEMM N
     const int BN = gemm_n % 256 == 0 ? 256 : (gemm_n % 128 == 0 ? 128 : 64);
@@ -1999,7 +2117,7 @@ int launch_conv_tc(const dc_conv_args_t* a, cudaStream_t stream, const float* bi
     bool halo = false, halo_wres = true, halo_pair = false;
     int halo_nhalf = 1;
     size_t halo_smem = 0;
-    if (!up && a->dilation <= 4 && g_kernel_family == DC_CONV_FAMILY_AUTO) {
+    if (!split && !up && a->dilation <= 4 && g_kernel_family == DC_CONV_FAMILY_AUTO) {
         // CTA pair (cta_group::2): half of the weight rows per SM.  BN <= 128: two 8-wide halves per tile (two MMA
         // chains); BN = 256: one half (a 128-cycle MMA hides its own latency, and 2 x 2 x 256 columns would not fit
         // TMEM).  Weights resident when Cout == BN and the layer's half fits next to two regions, else streamed
@@ -2037,7 +2155,7 @@ int launch_conv_tc(const dc_conv_args_t* a, cudaStream_t stream, const float* bi
         }
         }
     }
-    if (!halo && !up && a->Cout == BN && BN <= 128 && a->dilation <= 4) {
+    if (!split && !halo && !up && a->Cout == BN && BN <= 128 && a->dilation <= 4) {
         // TMA and the MMA unit both take the swizzle phase from absolute address bits, so a region only needs
         // TMA's 128 B alignment, not a 1024 B one: regions are packed back to back
         const size_t w_tile = (size_t)BN * KCHUNK * 2;
@@ -2079,7 +2197,8 @@ int launch_conv_tc(const dc_conv_args_t* a, cudaStream_t stream, const float* bi
     }
     if (g_kernel_family == DC_CONV_FAMILY_GENERIC) halo = halo_pair = false;      // test-only override (dc_debug_set_conv_family)
     {
-        cuuint64_t dims[4] = {(cuuint64_t)a->Cin, (cuuint64_t)a->W, (cuuint64_t)a->H, (cuuint64_t)a->B};
+        const int cin_span = split ? 2 * a->in_plane_stride + a->Cin : a->Cin;      // channels the boxes may read
+        cuuint64_t dims[4] = {(cuuint64_t)cin_span, (cuuint64_t)a->W, (cuuint64_t)a->H, (cuuint64_t)a->B};
         cuuint64_t str[3] = {(cuuint64_t)a->in_stride * 2, (cuuint64_t)a->W * a->in_stride * 2,
                              (cuuint64_t)a->H * a->W * a->in_stride * 2};
         cuuint32_t box[4] = {KCHUNK, TILE_W, TILE_H, 1};
@@ -2088,7 +2207,7 @@ int launch_conv_tc(const dc_conv_args_t* a, cudaStream_t stream, const float* bi
         if (rc != DC_OK) return rc;
     }
     {
-        const int ktot = up ? a->Cin : 9 * a->Cin;
+        const int ktot = (up ? a->Cin : 9 * a->Cin) * (split ? 3 : 1);
         const int rows = up ? 4 * a->Cout : a->Cout;
         cuuint64_t dims[2] = {(cuuint64_t)ktot, (cuuint64_t)rows};
         cuuint64_t str[1] = {(cuuint64_t)ktot * 2};
@@ -2121,7 +2240,15 @@ int launch_conv_tc(const dc_conv_args_t* a, cudaStream_t stream, const float* bi
     p.pool_stride = a->pool_stride;
     p.head_w = a->head_w; p.head_b = a->head_b; p.thresh = a->thresh;
     p.prob_out = a->prob_out; p.mask_out = a->mask_out;
+    p.in_plane_stride = a->in_plane_stride; p.out_plane_stride = a->out_plane_stride; p.pool_plane_stride = a->pool_plane_stride;
 
+    if (split) {
+        switch (BN) {
+            case 256: return launch_variant<256, 4, true>(p, stream);
+            case 128: return launch_variant<128, 6, true>(p, stream);
+            default:  return launch_variant<64, 8, true>(p, stream);
+        }
+    }
     if (halo_pair) {
         const int m_tiles = p.total_tiles / p.n_tiles;
         const int n_pairs = ((m_tiles + 1) / 2) * p.n_tiles;

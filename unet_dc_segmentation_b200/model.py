@@ -9,6 +9,10 @@ are BatchNorm-folded in fp32, repacked K-major to bf16 and handed to ``dc_model_
 runs ``dc_forward`` (18 kernel launches with the decoder levels fused, 22 without; see csrc/api.cu).  There is no PyTorch or CPU fallback.
 
 ``UNet`` is the reference's plain ``models/model.py`` network: identical state_dict, dilation 1 everywhere.
+
+``precision = "fp32"`` (class or instance attribute) runs the same network to fp32 accuracy, still on tcgen05: every
+activation and weight is held as three bf16 planes (``split_bf16``), each layer sums the six plane products that matter,
+and BatchNorm is folded in float64.  About six times the MMAs and three times the workspace of the bf16 forward.
 """
 from __future__ import annotations
 
@@ -36,12 +40,32 @@ def _conv_pair(cin: int, cout: int, d: int) -> nn.Sequential:
         nn.Conv2d(cout, cout, 3, padding=d, dilation=d), nn.BatchNorm2d(cout), nn.ReLU(inplace=True))
 
 
-def fold_conv_bn(conv_w, conv_b, bn_w, bn_b, bn_mean, bn_var, eps: float = 1e-5):
-    """Eval-mode BatchNorm folded into the preceding conv, in fp32 (model_2.py:41-46)."""
-    scale = bn_w.float() / torch.sqrt(bn_var.float() + eps)
-    w = conv_w.float() * scale.view(-1, 1, 1, 1)
-    b = (conv_b.float() - bn_mean.float()) * scale + bn_b.float()
+def fold_conv_bn(conv_w, conv_b, bn_w, bn_b, bn_mean, bn_var, eps: float = 1e-5, dtype=torch.float32):
+    """Eval-mode BatchNorm folded into the preceding conv, in fp32 (model_2.py:41-46); the fp32-precision forward folds
+    in float64 (dtype)."""
+    scale = bn_w.to(dtype) / torch.sqrt(bn_var.to(dtype) + eps)
+    w = conv_w.to(dtype) * scale.view(-1, 1, 1, 1)
+    b = (conv_b.to(dtype) - bn_mean.to(dtype)) * scale + bn_b.to(dtype)
     return w, b
+
+
+BF16_MAX = float(torch.finfo(torch.bfloat16).max)
+
+
+def split_bf16(t):
+    """float32(t) as three bf16 planes (hi, mid, lo): hi = bf16(x), mid = bf16(x - hi), lo = bf16(x - hi - mid), round to
+    nearest even, every residual exact in fp32, so that hi + (mid + lo) == x bit for bit in fp32 (also (hi + mid) + lo
+    below the overflow threshold).  Where bf16(x) would overflow (|x| within half a bf16 ulp of FLT_MAX) hi is the
+    largest finite bf16 instead, as the device's split does (csrc/generic.cu split3)."""
+    x = t.float()
+    hi = x.bfloat16()
+    over = hi.float().isinf() & ~x.isinf()
+    if bool(over.any()):
+        hi = torch.where(over, x.sign() * BF16_MAX, hi.float()).bfloat16()
+    r = x - hi.float()
+    mid = r.bfloat16()
+    lo = (r - mid.float()).bfloat16()
+    return hi, mid, lo
 
 
 def pack_conv3x3(w):
@@ -54,6 +78,20 @@ def pack_upconv(w):
     """ConvTranspose2d weight [Cin,Cout,2,2] -> bf16 [(a*2+b)*Cout + co, ci] (DC_KIND_UPCONV2 layout)."""
     ci, co = w.shape[:2]
     return w.float().permute(2, 3, 1, 0).reshape(4 * co, ci).to(torch.bfloat16).contiguous()
+
+
+def pack_conv3x3_split(w):
+    """[Cout,Cin,3,3] (float64 or float32) -> bf16 [Cout, ((ky*3+kx)*3 + plane)*Cin + ci]: the three planes of
+    split_bf16 per tap (DC_KIND_CONV3X3 layout of the fp32-precision forward)."""
+    co, ci = w.shape[:2]
+    return torch.stack(split_bf16(w.permute(0, 2, 3, 1)), 3).reshape(co, 27 * ci).contiguous()
+
+
+def pack_upconv_split(w):
+    """ConvTranspose2d weight [Cin,Cout,2,2] -> bf16 [(a*2+b)*Cout + co, plane*Cin + ci] (the fp32-precision
+    DC_KIND_UPCONV2 layout)."""
+    ci, co = w.shape[:2]
+    return torch.stack(split_bf16(w.permute(2, 3, 1, 0)), 3).reshape(4 * co, 3 * ci).contiguous()
 
 
 def compose_upconv(wu, bu, wd, bd):
@@ -170,9 +208,30 @@ class _Packed:
         lib = _lib.load()
         sd = {k: v.detach().to(device) for k, v in module.state_dict().items()}
         self.blobs = []          # keeps the device tensors alive for the lifetime of the handle
+        self.precision = module.precision
+        if self.precision not in ("bf16", "fp32"):
+            raise ValueError(f"UNetDC.precision must be 'bf16' or 'fp32', got {self.precision!r}")
+        fp32 = self.precision == "fp32"
         desc = _lib.ModelDesc()
         for i, (name, idx) in enumerate(_LAYER_ORDER):
-            if idx is None:
+            if fp32:
+                # every layer on the per-tap kernel in three bf16 planes, BatchNorm folded in float64; enc1.0 runs as an
+                # ordinary 3x3 layer on the input planes padded to 64 channels
+                if idx is None:
+                    w = pack_upconv_split(sd[f"{name}.weight"].double())
+                    b = sd[f"{name}.bias"].float().contiguous()
+                else:
+                    wf, b = fold_conv_bn(sd[f"{name}.{idx}.weight"], sd[f"{name}.{idx}.bias"],
+                                         sd[f"{name}.{idx + 1}.weight"], sd[f"{name}.{idx + 1}.bias"],
+                                         sd[f"{name}.{idx + 1}.running_mean"], sd[f"{name}.{idx + 1}.running_var"],
+                                         module._bn_eps(name, idx + 1), dtype=torch.float64)
+                    if i == 0:
+                        wp = torch.zeros((wf.shape[0], 64, 3, 3), dtype=wf.dtype, device=wf.device)
+                        wp[:, :module.in_channels] = wf
+                        wf = wp
+                    w = pack_conv3x3_split(wf)
+                    b = b.float().contiguous()
+            elif idx is None:
                 w = pack_upconv(sd[f"{name}.weight"])
                 b = sd[f"{name}.bias"].float().contiguous()
             else:
@@ -207,14 +266,15 @@ class _Packed:
         desc.base_channels = 64
         desc.in_channels = module.in_channels
         desc.out_channels = module.out_channels
-        if module.fuse_level1:
+        desc.precision = _lib.DC_PRECISION_FP32 if fp32 else _lib.DC_PRECISION_BF16
+        if module.fuse_level1 and not fp32:
             comp, skipw, fb = fused_level1_blobs(sd, module._bn_eps("dec1", 1))
             fw = pack_upfused(comp, skipw)
             self.blobs += [fw, fb]
             desc.fused_weight1 = fw.data_ptr()
             desc.fused_bias1 = fb.data_ptr()
         for lvl in (2, 3, 4):
-            if lvl in module.fuse_levels:
+            if lvl in module.fuse_levels and not fp32:
                 comp, skipw, fb = fused_level_blobs(sd, lvl, module._bn_eps(f"dec{lvl}", 1))
                 wx, ws = pack_upfused_wide(comp, skipw)
                 self.blobs += [wx, ws, fb]
@@ -256,6 +316,10 @@ class UNetDC(nn.Module):
     # enc1.3 and dec1.3 per output parity class with shared windows (conv_par2_kernel; taken when dilations[0] == 1)
     parity_level1 = True
     parity_layers = ("enc1", "dec1")
+    # "bf16" (activations and weights in bf16) or "fp32" (three bf16 planes each, products to ~2^-24 relative, the
+    # unfused schedule on the per-tap kernel; the fuse / parity settings above are then ignored).  Read when the weights
+    # are packed; changing it repacks on the next call.
+    precision = "bf16"
 
     def __init__(self, in_channels: int = 3, out_channels: int = 1):
         super().__init__()
@@ -293,7 +357,7 @@ class UNetDC(nn.Module):
     def packed(self) -> _Packed:
         dev = self.out_conv.weight.device
         _lib.require_cuda(self.out_conv.weight, "UNetDC parameters (call .to('cuda') first)")
-        if self._packed is None or self._packed.device != dev:
+        if self._packed is None or self._packed.device != dev or self._packed.precision != self.precision:
             self._packed = _Packed(self, dev)
         return self._packed
 
