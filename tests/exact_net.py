@@ -21,6 +21,9 @@ modes) must give identical bits, equal to the plain float64 evaluation ``forward
 """
 from __future__ import annotations
 
+import ctypes
+
+import pytest
 import torch
 import torch.nn.functional as F
 
@@ -385,3 +388,58 @@ TEETH_SHAPE = (1, 64, 128)            # the shape every network is also run at o
 def net(name):
     cin, cout, dil, seed = NETS[name]
     return exact_state_dict(cin, cout, dil, seed), dil
+
+
+# ----------------------------------------------------------------------------- device buffers and launches (GPU tests)
+
+GUARD = 4096                                   # bytes of sentinel before and after every output view
+SENT = 0xA5
+SENT16 = -23131                                # int16 view of the bytes 0xA5 0xA5
+
+
+def _lib():
+    from unet_dc_segmentation_b200 import _lib as L
+    return L
+
+
+@pytest.fixture
+def family():
+    """dc_debug_set_conv_family for one test, restored to auto afterwards (import it into a test module to use it)."""
+    L = _lib()
+    codes = {"auto": L.DC_CONV_FAMILY_AUTO, "no_pair": L.DC_CONV_FAMILY_NO_PAIR, "generic": L.DC_CONV_FAMILY_GENERIC}
+    try:
+        yield lambda name: L.check(L.load().dc_debug_set_conv_family(codes[name]))
+    finally:
+        L.check(L.load().dc_debug_set_conv_family(L.DC_CONV_FAMILY_AUTO))
+
+
+def guarded(shape, dtype):
+    """(raw uint8 buffer, view of `shape`) on the device: the view sits between GUARD sentinel bytes, and is itself
+    sentinel-filled."""
+    n = torch.Size(shape).numel() * torch.empty((), dtype=dtype).element_size()
+    raw = torch.full((n + 2 * GUARD,), SENT, dtype=torch.uint8, device="cuda")
+    return raw, raw[GUARD:GUARD + n].view(dtype).view(shape)
+
+
+def check_guards(raw, case):
+    r = raw.cpu()
+    assert bool((r[:GUARD] == SENT).all()), f"{case}: wrote before its output buffer"
+    assert bool((r[-GUARD:] == SENT).all()), f"{case}: wrote after its output buffer"
+
+
+def check_outside(raw, view, off, n, case):
+    """Guards intact and channels [0, off) and [off + n, S) of a bf16 NHWC view untouched."""
+    check_guards(raw, case)
+    v = view.cpu().view(torch.int16)
+    assert bool((v[..., :off] == SENT16).all()) and bool((v[..., off + n:] == SENT16).all()), \
+        f"{case}: wrote outside channels [{off}, {off + n})"
+
+
+def conv_tc(**kw):
+    """dc_conv_tc with the given dc_conv_args fields, synchronised."""
+    L = _lib()
+    a = L.ConvArgs()
+    for k, v in kw.items():
+        setattr(a, k, v)
+    L.check(L.load().dc_conv_tc(ctypes.byref(a), L.stream_ptr()))
+    torch.cuda.synchronize()

@@ -88,6 +88,27 @@ def plane_buffer(x64, plane_stride, width, fill=float("nan"), off=0):
     return buf
 
 
+def assert_planes(buf, want64, plane_stride, off, case, others=True):
+    """Plane p of a bf16 buffer at channels [off + p * plane_stride, + C) equals plane p of split(want64), bit for bit
+    (-0 == +0); others: every channel outside the three ranges still holds the sentinel of exact_net.guarded."""
+    from exact_net import SENT16
+    g = buf.detach().cpu()
+    C = want64.shape[-1]
+    want = split64(want64.cpu())
+    for p in range(3):
+        got = g[..., off + p * plane_stride:off + p * plane_stride + C].float()
+        bad = ~(got == want[p].float())
+        if bool(bad.any()):
+            idx = tuple(int(v) for v in bad.nonzero()[0])
+            raise AssertionError(f"{case}: plane {p}: {int(bad.sum())}/{bad.numel()} differ; first at {idx}: got "
+                                 f"{float(got[idx])!r}, want {float(want[p][idx])!r} (value {float(want64[idx])!r})")
+    if others:
+        keep = torch.ones(g.shape[-1], dtype=torch.bool)
+        for p in range(3):
+            keep[off + p * plane_stride:off + p * plane_stride + C] = False
+        assert bool((g.view(torch.int16)[..., keep] == SENT16).all()), f"{case}: wrote outside its channel ranges"
+
+
 def join(buf, plane_stride, C, off=0):
     """Three bf16 planes of a buffer -> float64 values hi + (mid + lo)."""
     f = buf.double()

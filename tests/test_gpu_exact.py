@@ -19,9 +19,7 @@ import exact_net as en
 
 pytestmark = pytest.mark.gpu
 
-GUARD = 4096                                   # bytes of sentinel before and after every output view
-SENT = 0xA5
-SENT16 = -23131                                # int16 view of the bytes 0xA5 0xA5
+GUARD, SENT, SENT16 = en.GUARD, en.SENT, en.SENT16
 THRESH = 0.3
 FAMILIES = ("auto", "no_pair", "generic")
 
@@ -43,38 +41,12 @@ def _lib():
     return L
 
 
-@pytest.fixture
-def family():
-    """dc_debug_set_conv_family for one test, restored to auto afterwards."""
-    L = _lib()
-    codes = {"auto": L.DC_CONV_FAMILY_AUTO, "no_pair": L.DC_CONV_FAMILY_NO_PAIR, "generic": L.DC_CONV_FAMILY_GENERIC}
-    try:
-        yield lambda name: L.check(L.load().dc_debug_set_conv_family(codes[name]))
-    finally:
-        L.check(L.load().dc_debug_set_conv_family(L.DC_CONV_FAMILY_AUTO))
+family = en.family
 
 
 # ----------------------------------------------------------------------------- buffers
 
-def _guarded(shape, dtype):
-    """(raw uint8 buffer, view of `shape`): the view sits between GUARD sentinel bytes, and is itself sentinel-filled."""
-    n = torch.Size(shape).numel() * torch.empty((), dtype=dtype).element_size()
-    raw = torch.full((n + 2 * GUARD,), SENT, dtype=torch.uint8, device="cuda")
-    return raw, raw[GUARD:GUARD + n].view(dtype).view(shape)
-
-
-def _check_guards(raw, case):
-    r = raw.cpu()
-    assert bool((r[:GUARD] == SENT).all()), f"{case}: wrote before its output buffer"
-    assert bool((r[-GUARD:] == SENT).all()), f"{case}: wrote after its output buffer"
-
-
-def _check_outside(raw, view, off, n, case):
-    """Guards intact and channels [0, off) and [off + n, S) of a bf16 NHWC view untouched."""
-    _check_guards(raw, case)
-    v = view.cpu().view(torch.int16)
-    assert bool((v[..., :off] == SENT16).all()) and bool((v[..., off + n:] == SENT16).all()), \
-        f"{case}: wrote outside channels [{off}, {off + n})"
+_guarded, _check_guards, _check_outside = en.guarded, en.check_guards, en.check_outside
 
 
 def _nan_padded(x64, width, off=0):
@@ -84,14 +56,7 @@ def _nan_padded(x64, width, off=0):
     return buf.cuda()
 
 
-def _conv(**kw):
-    """dc_conv_tc with the given dc_conv_args fields (pool and head outputs have no out= in layers.py)."""
-    L = _lib()
-    a = L.ConvArgs()
-    for k, v in kw.items():
-        setattr(a, k, v)
-    L.check(L.load().dc_conv_tc(ctypes.byref(a), L.stream_ptr()))
-    torch.cuda.synchronize()
+_conv = en.conv_tc
 
 
 def _head_weights(feat64, seed):
