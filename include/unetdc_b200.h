@@ -16,6 +16,7 @@
  *   dc_rolling_ball              rolling_ball_correction_rgb  utils/data_loader.py:11-24
  *   dc_resize_linear_u8          the two cv2.resize calls     quantify_droplets_batch.py:44, :57
  *   dc_label_stats               quantify                     quantify_droplets_batch.py:81-95
+ *   dc_table_csv                 df.to_csv of the per-image tables  quantify_droplets_batch.py:62-63
  *   dc_overlay_stencil           cv2.findContours + cv2.drawContours of the overlays
  *                                                           quantify_droplets_batch.py:74-79
  *   dc_roi_mask / dc_radial_density / dc_spatial_density
@@ -50,7 +51,7 @@ extern "C" {
 /* Bumped whenever a struct or signature in this header changes, or an entry point's return code for some arguments
  * does; dc_version() returns the value the library was built with and the Python binding refuses to load a library
  * that disagrees. */
-#define DC_ABI_VERSION 208
+#define DC_ABI_VERSION 209
 
 const char* dc_last_error(void);
 int dc_version(void);
@@ -354,6 +355,58 @@ typedef struct dc_label_args {
 int dc_label_workspace_bytes(int B, int H, int W, size_t* bytes);
 /* Shape limits (DC_EINVAL otherwise): B <= 65535, H*W < 2^31, H <= 65535 * 128 (rows of 128-row tiles in gridDim.y). */
 int dc_label_stats(const dc_label_args_t* args, void* stream);
+
+/* ------------------------------------------------------------------ droplet table -> CSV text
+ * The per-image CSV files of quantify_droplets_batch.py:62-63 (df.insert(0, "filename", name); df.to_csv(index=False))
+ * written on the device from a dc_label_stats table, byte for byte what pandas writes:
+ *   header   filename,label,area,equivalent_diameter,centroid-0,centroid-1[,area_sqmicron,eq_diam_micron]\n
+ *            (the micron columns exactly when area_um2 and diam_um are both non-NULL)
+ *   rows     <filename field>,<r + 1>,<area>,<eq_diam>,<centroid0>,<centroid1>[,<area_um2>,<diam_um>]\n
+ *   a frame without droplets is the single line "filename\n" (an empty DataFrame with the column inserted).
+ * Integers in decimal; float64 as Python's repr / numpy's str: the shortest digit string that reads back as the same
+ * double (the closest one when several do), positional when the leading digit's decimal exponent is in [-4, 16) with
+ * ".0" when nothing follows the point, else d[.ddd]e+XX / e-XX with at least two exponent digits; "inf" / "-inf";
+ * NaN as an empty field (pandas' na_rep).
+ * names: the filename FIELD of each frame as pandas' csv writer emits it (QUOTE_MINIMAL: quoted, with quotes doubled,
+ * when it contains a comma, a quote or a line break), already encoded; frame b's field is
+ * names[name_offsets[b] .. name_offsets[b+1]).
+ * Output: frame b's file is out[frame_offsets[b] .. frame_offsets[b+1]) (frames back to back); area_sum[b] = the sum of
+ * the frame's area column (summary_per_image.csv's total_area_px).  A frame whose count exceeds `capacity` gets NO text
+ * (an empty range) and area_sum -1: re-run dc_label_stats with room for every droplet, then this call.
+ * Two passes (row lengths, then text) around a per-frame and a per-batch scan; no synchronisation, no allocation, and
+ * nothing is written past out[out_bytes). */
+typedef struct dc_table_csv_args {
+    int B;
+    int capacity;                /* table rows per frame, as dc_label_args.capacity                          */
+    const int32_t* counts;       /* [B]                                                                       */
+    const int64_t* area;         /* [B*capacity] (row r of frame b at b*capacity + r)                         */
+    const double* eq_diam;
+    const double* centroid0;
+    const double* centroid1;
+    const double* area_um2;      /* NULL together with diam_um: no micron columns                            */
+    const double* diam_um;
+    const char* names;           /* escaped, encoded filename fields, back to back                           */
+    const int64_t* name_offsets; /* [B+1]                                                                     */
+    int64_t names_bytes;         /* upper bound of name_offsets[B] - name_offsets[0] (sizes the bound below)  */
+    char* out;
+    int64_t out_bytes;           /* >= dc_table_csv_bounds(...) (DC_EINVAL otherwise)                        */
+    int64_t* frame_offsets;      /* [B+1]                                                                     */
+    int64_t* area_sum;           /* [B]                                                                       */
+    void* workspace;
+    size_t workspace_bytes;
+} dc_table_csv_args_t;
+
+/* out_bytes: enough text for any table of this shape (every row at the widest field widths); workspace_bytes: the
+ * workspace dc_table_csv needs.  micron: 0 / 1. */
+int dc_table_csv_bounds(int B, int capacity, int micron, int64_t names_bytes, int64_t* out_bytes, size_t* workspace_bytes);
+/* Shape limits (DC_EINVAL otherwise): 1 <= B <= 65535, 1 <= capacity < 2^31 - 1. */
+int dc_table_csv(const dc_table_csv_args_t* args, void* stream);
+/* TEST AIDS (host only, no GPU needed), the formatting code dc_table_csv runs, compiled for the host:
+ * format n values (float64 when is_double, else int64) into out, value i at out[offsets[i] .. offsets[i+1]);
+ * returns DC_EINVAL when the text does not fit in cap bytes. */
+int dc_debug_format_values(const void* values, int is_double, int64_t n, char* out, int64_t cap, int64_t* offsets);
+/* dc_table_csv on a table in HOST memory (every pointer of args a host pointer; the workspace is not used). */
+int dc_debug_table_csv_host(const dc_table_csv_args_t* args);
 
 /* ---- overlay stencil --------------------------------------------------------------------------
  * stencil[b,y,x] = 1 exactly where

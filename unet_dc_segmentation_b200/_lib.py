@@ -17,7 +17,7 @@ DC_EPI_STORE, DC_EPI_STORE_POOL, DC_EPI_HEAD, DC_EPI_UPSCATTER = 0, 1, 2, 3
 DC_NUM_LAYERS = 23
 DC_CONV_FAMILY_AUTO, DC_CONV_FAMILY_NO_PAIR, DC_CONV_FAMILY_GENERIC = 0, 1, 2
 DC_PRECISION_BF16, DC_PRECISION_FP32 = 0, 1
-ABI_VERSION = 208          # DC_ABI_VERSION of include/unetdc_b200.h these ctypes structures mirror
+ABI_VERSION = 209          # DC_ABI_VERSION of include/unetdc_b200.h these ctypes structures mirror
 
 EXPORTS = [
     "dc_last_error", "dc_version", "dc_device_check", "dc_conv_tc", "dc_conv_upfused", "dc_debug_upfuse_schedule", "dc_debug_set_upfuse_mode", "dc_debug_set_conv_family", "dc_stem", "dc_model_create",
@@ -27,6 +27,7 @@ EXPORTS = [
     "dc_resize_linear_u8", "dc_overlay_workspace_bytes", "dc_overlay_stencil",
     "dc_roi_workspace_bytes", "dc_roi_mask", "dc_radial_workspace_bytes", "dc_radial_density",
     "dc_spatial_workspace_bytes", "dc_spatial_density",
+    "dc_table_csv_bounds", "dc_table_csv", "dc_debug_format_values", "dc_debug_table_csv_host",
 ]
 
 
@@ -104,6 +105,17 @@ class LabelArgs(Structure):
         ("labels_out", c_void_p), ("capacity", c_int), ("counts", c_void_p),
         ("area", c_void_p), ("centroid0", c_void_p), ("centroid1", c_void_p), ("eq_diam", c_void_p),
         ("area_um2", c_void_p), ("diam_um", c_void_p),
+        ("workspace", c_void_p), ("workspace_bytes", c_size_t),
+    ]
+
+
+class TableCsvArgs(Structure):
+    _fields_ = [
+        ("B", c_int), ("capacity", c_int), ("counts", c_void_p), ("area", c_void_p),
+        ("eq_diam", c_void_p), ("centroid0", c_void_p), ("centroid1", c_void_p),
+        ("area_um2", c_void_p), ("diam_um", c_void_p),
+        ("names", c_void_p), ("name_offsets", c_void_p), ("names_bytes", c_int64),
+        ("out", c_void_p), ("out_bytes", c_int64), ("frame_offsets", c_void_p), ("area_sum", c_void_p),
         ("workspace", c_void_p), ("workspace_bytes", c_size_t),
     ]
 
@@ -190,6 +202,10 @@ def load(build_if_missing: bool = True) -> C.CDLL:
     lib.dc_debug_rolling_ball_bands.argtypes = [c_int, POINTER(c_int), c_int]
     lib.dc_label_workspace_bytes.argtypes = [c_int, c_int, c_int, POINTER(c_size_t)]
     lib.dc_label_stats.argtypes = [POINTER(LabelArgs), c_void_p]
+    lib.dc_table_csv_bounds.argtypes = [c_int, c_int, c_int, c_int64, POINTER(c_int64), POINTER(c_size_t)]
+    lib.dc_table_csv.argtypes = [POINTER(TableCsvArgs), c_void_p]
+    lib.dc_debug_format_values.argtypes = [c_void_p, c_int, c_int64, c_void_p, c_int64, c_void_p]
+    lib.dc_debug_table_csv_host.argtypes = [POINTER(TableCsvArgs)]
     lib.dc_resize_linear_u8.argtypes = [POINTER(ResizeArgs), c_void_p]
     lib.dc_overlay_workspace_bytes.argtypes = [c_int, c_int, c_int, POINTER(c_size_t)]
     lib.dc_overlay_stencil.argtypes = [POINTER(OverlayArgs), c_void_p]

@@ -16,14 +16,18 @@ IMG_SIZE constant) and `--density_maps` (the per-image maps of the reference's s
 rank writes the per-image files of its own frames, and the tables are gathered on rank 0, which writes the reports.
 
 ``main`` runs the FAST path (``run_fast``): frames are decoded by a thread pool, batched, and streamed through
-``DropletPipeline.run_host_pipelined`` -- u8 frames up, u8 masks (+ overlay stencils) and table rows down, nothing
-else crosses PCIe -- while another pool writes the PNG / CSV files.  ``preprocess`` / ``run_batch`` keep the
+``DropletPipeline.run_host_pipelined`` -- u8 frames up, u8 masks (+ overlay stencils) and the per-image CSV files as
+text (formatted on the device by dc_table_csv) down, nothing else crosses PCIe -- while another pool writes the PNG /
+CSV files.  ``write_reports`` builds the reports of both loops from the per-image CSV texts.  ``preprocess`` / ``run_batch`` keep the
 reference's function-by-function shape (per-image round trips) for callers that use them as a library;
 ``--reference_loop`` makes ``main`` use them.
 """
 from __future__ import annotations
 
 import argparse
+import codecs
+import functools
+import io
 import sys
 from pathlib import Path
 
@@ -144,31 +148,80 @@ def combined_csv_text(all_props, csv_texts):
     return header + "".join(t.split("\n", 1)[1] for t in csv_texts)
 
 
-def write_reports(out_dir: Path, per_image_rows, all_props, skip_excel: bool, skip_histogram: bool, csv_texts=None) -> None:
-    """qdb:163-199: summary_per_image.csv, all_droplets.csv (+xlsx or the noexcel copy), stats, histogram."""
+@functools.lru_cache(maxsize=None)
+def concat_upcasts_with_empty_frames() -> bool:
+    """Whether the installed pandas turns the int64 label / area columns into float64 when pd.concat meets a per-image
+    frame without droplets (pandas 3: the empty frame's missing columns count as all-NaN float64 columns; pandas 2
+    left empty frames out when it chose the dtype).  Decided by one tiny concat, the way the reports are built."""
     import pandas as pd
+    empty = pd.DataFrame()
+    empty.insert(0, "filename", "e")
+    full = pd.DataFrame({"label": np.array([1], np.int64), "area": np.array([12], np.int64), "x": [0.5]})
+    full.insert(0, "filename", "f")
+    text = pd.concat([empty, full], ignore_index=True).to_csv(index=False)
+    if text in ("filename,label,area,x\nf,1,12,0.5\n", "filename,label,area,x\nf,1.0,12.0,0.5\n"):
+        return ".0" in text
+    raise RuntimeError(f"pandas {pd.__version__} concatenates the droplet tables in an unknown way: {text!r}")
+
+
+def combined_csv_bytes(texts, fields) -> bytes:
+    """all_droplets.csv -- ``pd.concat(per-image frames, ignore_index=True).to_csv(index=False)`` (qdb:165-166) -- from
+    the per-image CSV files (bytes) without formatting a number again.  fields: each image's filename field as it
+    appears in its file.  When some images have droplets and others not, pandas may write label and area as float64
+    (``concat_upcasts_with_empty_frames``): then ".0" is inserted after both fields of every row, at positions that
+    follow from the filename field's length."""
+    full = [(t, f) for t, f in zip(texts, fields) if not t.startswith(b"filename\n")]
+    if not full:
+        return b"filename\n"
+    header = full[0][0][:full[0][0].index(b"\n") + 1]
+    if len(full) == len(texts) or not concat_upcasts_with_empty_frames():
+        return header + b"".join(t[len(header):] for t, _ in full)
+    dot0 = np.frombuffer(b".0", np.uint8)
+    parts = [header]
+    for t, f in full:
+        buf = np.frombuffer(t, dtype=np.uint8)[len(header):]
+        m = f.count(b"\n")                                     # a quoted field may hold line breaks: every row has m + 1
+        ends = np.flatnonzero(buf == ord("\n"))[m::m + 1]
+        starts = np.concatenate(([0], ends[:-1] + 1))
+        commas = np.flatnonzero(buf == ord(","))
+        k = np.searchsorted(commas, starts + len(f) + 1)         # the comma after the label of every row
+        at = np.stack([commas[k], commas[k + 1]], 1).ravel()       # ... and the one after its area
+        parts.append(np.insert(buf, np.repeat(at, 2), np.tile(dot0, at.size)).tobytes())
+    return b"".join(parts)
+
+
+def write_reports(out_dir: Path, per_image_rows, texts, sizes, skip_excel: bool, skip_histogram: bool,
+                  encoding: str) -> None:
+    """qdb:163-199: summary_per_image.csv, all_droplets.csv (+xlsx or the noexcel copy), stats, histogram, from every
+    image's summary row, CSV file text (bytes in ``encoding``) and size column (f64), in frame order.  The files pandas
+    writes itself are UTF-8; all_droplets.csv, when every image has droplets, is the per-image texts joined as they are
+    (what the reference's concat gives then, written with write_text)."""
+    import pandas as pd
+    from .quantify import csv_field
     summary_df = pd.DataFrame(per_image_rows)
     summary_df.to_csv(out_dir / "summary_per_image.csv", index=False)
-    if not all_props:
+    if not texts:
         return
-    combined = pd.concat(all_props, ignore_index=True)
-    text = combined_csv_text(all_props, csv_texts)
-    if text is not None:
-        (out_dir / "all_droplets.csv").write_text(text)
-    else:
-        combined.to_csv(out_dir / "all_droplets.csv", index=False)
+    fields = [csv_field(r["filename"], encoding) for r in per_image_rows]
+    combined = combined_csv_bytes(texts, fields)
+    as_pandas = combined if codecs.lookup(encoding).name == "utf-8" else combined.decode(encoding).encode("utf-8")
+    every_frame = all(not t.startswith(b"filename\n") for t in texts)
+    (out_dir / "all_droplets.csv").write_bytes(combined if every_frame else as_pandas)
     if not skip_excel:
         try:
             import xlsxwriter  # noqa: F401
+            frame = pd.read_csv(io.BytesIO(as_pandas), dtype={"filename": str}, keep_default_na=False,
+                                float_precision="round_trip")
             with pd.ExcelWriter(out_dir / "all_droplets.xlsx", engine="xlsxwriter") as xw:
-                combined.to_excel(xw, index=False, sheet_name="droplets")
+                frame.to_excel(xw, index=False, sheet_name="droplets")
                 summary_df.to_excel(xw, index=False, sheet_name="per_image")
         except (ImportError, AttributeError):
-            combined.to_csv(out_dir / "all_droplets_noexcel.csv", index=False)
+            (out_dir / "all_droplets_noexcel.csv").write_bytes(as_pandas)
             print("Skipped Excel file; install 'xlsxwriter' if you need .xlsx output.")
-    size_col = "eq_diam_micron" if "eq_diam_micron" in combined.columns else "equivalent_diameter"
-    if size_col in combined.columns:
-        stats = combined[size_col].describe()[["mean", "50%", "std"]].rename({"50%": "median"})
+    if combined != b"filename\n":
+        size_col = "eq_diam_micron" if b",eq_diam_micron\n" in combined[:combined.index(b"\n") + 1] else "equivalent_diameter"
+        column = pd.Series(np.concatenate(sizes), name=size_col)
+        stats = column.describe()[["mean", "50%", "std"]].rename({"50%": "median"})
         stats.to_csv(out_dir / "droplet_size_stats.csv")
         if not skip_histogram:
             try:
@@ -179,7 +232,7 @@ def write_reports(out_dir: Path, per_image_rows, all_props, skip_excel: bool, sk
                 print("Skipped histogram; matplotlib is not installed.")
                 return
             plt.figure(figsize=(6, 4))
-            plt.hist(combined[size_col], bins=40)
+            plt.hist(column, bins=40)
             plt.xlabel("Diameter (µm)" if "micron" in size_col else "Diameter (pixels)")
             plt.ylabel("Count")
             plt.title("Droplet size distribution")
@@ -198,19 +251,12 @@ def _decode(path):
     return im
 
 
-def _table_frame(cols: dict, px_per_um):
-    """Per-image DataFrame with the reference's column contract (qdb:87-94): empty and column-less without droplets."""
-    import pandas as pd
-    from .quantify import COLUMNS, MICRON_COLUMNS
-    if len(cols["label"]) == 0:
-        return pd.DataFrame()
-    return pd.DataFrame({k: cols[k] for k in COLUMNS + (MICRON_COLUMNS if px_per_um else [])})
-
-
 def run_fast(images, mine, model, args, out_dir, mask_dir, overlay_dir):
     """The batched path behind ``main``: the per-image work of qdb:146-160 (preprocess + run_batch) for the frames
     ``mine`` (indices into ``images``), with every device stage batched and the host stages (decode, PNG / CSV
-    writing) in thread pools around it.  Returns (indices, per_image_rows, all_props) in frame order."""
+    writing) in thread pools around it.  The per-image CSV files are formatted on the device (dc_table_csv): no
+    DataFrame and no per-row Python object.  Returns (indices, per_image_rows, texts, sizes) in frame order: the
+    summary row, the CSV file's bytes and the size column of every frame."""
     import collections
     import os
     from concurrent.futures import ThreadPoolExecutor
@@ -221,7 +267,7 @@ def run_fast(images, mine, model, args, out_dir, mask_dir, overlay_dir):
                            img_size=args.img_size)
     nthreads = max(2, min(16, (os.cpu_count() or 4)))
     metas = collections.deque()                      # one entry per batch handed to the pipeline, in order
-    idx, per_image_rows, all_props = [], [], []
+    idx, per_image_rows, texts, sizes = [], [], [], []
 
     with ThreadPoolExecutor(nthreads) as decoders, ThreadPoolExecutor(nthreads) as writers:
         def batches():
@@ -242,43 +288,42 @@ def run_fast(images, mine, model, args, out_dir, mask_dir, overlay_dir):
                 fr = fut.result()
                 if cur and (fr.shape != cur[0].shape or len(cur) == args.batch):
                     metas.append(cur_meta)
-                    yield np.stack(cur)
+                    yield np.stack(cur), [images[j].name for j in cur_meta]
                     cur, cur_meta = [], []
                 cur.append(fr)
                 cur_meta.append(i)
             if cur:
                 metas.append(cur_meta)
-                yield np.stack(cur)
+                yield np.stack(cur), [images[j].name for j in cur_meta]
 
-        def write_image(i, mask, stencil, df):
+        def write_image(i, mask, stencil, text):
             name = images[i].stem
             cv2.imwrite(str(Path(mask_dir) / f"{name}_pred.png"), mask * 255)                 # qdb:58
-            text = df.to_csv(index=False)                                                     # qdb:63
-            (Path(mask_dir).parent / f"{name}_droplets.csv").write_text(text)
+            (Path(mask_dir).parent / f"{name}_droplets.csv").write_bytes(text)                # qdb:62-63
             if overlay_dir is not None:
                 img = cv2.imread(str(images[i]))                                              # qdb:75
                 if img is not None:
                     draw_overlay(img, stencil)                                                # qdb:76-77, from the GPU
                     cv2.imwrite(str(Path(overlay_dir) / f"{name}_overlay.png"), img)          # qdb:78
-            return text
 
         jobs = []
         want_ov = overlay_dir is not None
-        for res in pipe.run_host_pipelined(batches(), dev, copy=True, want_overlay=want_ov):
+        for res in pipe.run_host_pipelined(batches(), dev, copy=True, want_overlay=want_ov, csv=True):
             masks, tables = res[0], res[1]
             stencils = res[2] if want_ov else None
             for b, i in enumerate(metas.popleft()):
-                df = _table_frame(tables[b], args.px_per_micron)
-                df.insert(0, "filename", images[i].name)                                      # qdb:62
-                jobs.append(writers.submit(write_image, i, masks[b], stencils[b] if want_ov else None, df))
+                jobs.append(writers.submit(write_image, i, masks[b], stencils[b] if want_ov else None, tables.texts[b]))
                 idx.append(i)
-                all_props.append(df)
-                per_image_rows.append({"filename": images[i].name, "droplet_count": len(df),
-                                       "total_area_px": df["area"].sum() if not df.empty else 0})   # qdb:67-72
+                texts.append(tables.texts[b])
+                sizes.append(tables.sizes[b])
+                n = int(tables.counts[b])
+                per_image_rows.append({"filename": images[i].name, "droplet_count": n,
+                                       "total_area_px": int(tables.area_sums[b]) if n else 0})    # qdb:67-72
                 if args.density_maps:
                     save_density_maps(str(images[i]), images[i].stem, torch.from_numpy(masks[b]).to(dev)[None], out_dir)
-        csv_texts = [j.result() for j in jobs]
-    return idx, per_image_rows, all_props, csv_texts
+        for j in jobs:
+            j.result()
+    return idx, per_image_rows, texts, sizes
 
 
 def build_parser() -> argparse.ArgumentParser:
@@ -334,7 +379,6 @@ def main(argv=None) -> int:
 
     tensors, meta, idx = [], [], []
     per_image_rows, all_props = [], []
-    csv_texts = None
 
     def flush():
         run_batch(tensors, meta, model, mask_dir, overlay_dir, args.prob_thresh, args.min_area, args.px_per_micron,
@@ -352,15 +396,21 @@ def main(argv=None) -> int:
                 flush()
         if tensors:
             flush()
+        # run_batch wrote its CSVs through pandas (UTF-8); the reports take the same text from its DataFrames
+        encoding = "utf-8"
+        size_col = "eq_diam_micron" if args.px_per_micron else "equivalent_diameter"
+        texts = [df.to_csv(index=False).encode(encoding) for df in all_props]
+        sizes = [df[size_col].to_numpy(np.float64) if size_col in df else np.zeros(0) for df in all_props]
     else:
-        idx, per_image_rows, all_props, csv_texts = run_fast(images, mine, model, args, out_dir, mask_dir, overlay_dir)
+        from .quantify import text_encoding
+        encoding = text_encoding()
+        idx, per_image_rows, texts, sizes = run_fast(images, mine, model, args, out_dir, mask_dir, overlay_dir)
 
-    texts = csv_texts if csv_texts is not None else [None] * len(idx)
-    local = [(i, (row, df, t)) for i, row, df, t in zip(idx, per_image_rows, all_props, texts)]
-    merged = shard.gather_results(local, len(images), dst=0)
+    local = [(i, (row, t, s)) for i, row, t, s in zip(idx, per_image_rows, texts, sizes)]
+    merged = shard.gather_results(local, len(images), dst=0)       # the CSV texts travel, not DataFrames
     if rank == 0:
-        write_reports(out_dir, [m[0] for m in merged], [m[1] for m in merged], args.skip_excel, args.skip_histogram,
-                      csv_texts=[m[2] for m in merged])
+        write_reports(out_dir, [m[0] for m in merged], [m[1] for m in merged], [m[2] for m in merged],
+                      args.skip_excel, args.skip_histogram, encoding)
         print("\n All done. Outputs are in ", out_dir)
     if world > 1:
         import torch.distributed as dist

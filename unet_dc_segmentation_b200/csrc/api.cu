@@ -243,6 +243,18 @@ int dc_label_stats(const dc_label_args_t* args, void* stream) {
     return launch_label_stats(args, (cudaStream_t)stream);
 }
 
+int dc_table_csv(const dc_table_csv_args_t* args, void* stream) {
+    int rc = check_current_device(nullptr);
+    if (rc != DC_OK) return rc;
+    return launch_table_csv(args, (cudaStream_t)stream);
+}
+
+int dc_debug_format_values(const void* values, int is_double, int64_t n, char* out, int64_t cap, int64_t* offsets) {
+    return format_values_host(values, is_double, n, out, cap, offsets);
+}
+
+int dc_debug_table_csv_host(const dc_table_csv_args_t* args) { return table_csv_host(args); }
+
 int dc_overlay_workspace_bytes(int B, int H, int W, size_t* bytes) {
     DC_REQUIRE(bytes && B > 0 && H > 0 && W > 0, DC_EINVAL, "dc_overlay_workspace_bytes: bad argument");
     *bytes = overlay_workspace_bytes(B, H, W);

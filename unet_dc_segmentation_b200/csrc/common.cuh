@@ -37,6 +37,9 @@ int set_conv_family(int family);
 int upfuse_schedule(int* out, int cap);
 int set_upfuse_mode(int mode);
 int launch_label_stats(const dc_label_args_t* a, cudaStream_t stream);
+int launch_table_csv(const dc_table_csv_args_t* a, cudaStream_t stream);
+int table_csv_host(const dc_table_csv_args_t* a);
+int format_values_host(const void* values, int is_double, int64_t n, char* out, int64_t cap, int64_t* offsets);
 int launch_rolling_ball(const dc_rolling_ball_args_t* a, cudaStream_t stream, bool tiled_only);
 int launch_rolling_ball_banded(const dc_rolling_ball_args_t* a, cudaStream_t stream, const char* who);
 int launch_resize_linear_u8(const dc_resize_args_t* a, cudaStream_t stream);

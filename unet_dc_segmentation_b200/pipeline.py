@@ -11,6 +11,7 @@ Stages, all on the current CUDA stream (no host synchronisation until the tables
   dc_forward        stem reads the corrected u8 plane and does the /255 (qdb:45); the last conv's
                      epilogue does out_conv + sigmoid + `> prob_thresh` and writes the u8 mask
   dc_label_stats    labelling, min_area filter, compaction, area / centroid / diameter (+ micron columns)
+  dc_table_csv      (run_host_pipelined(csv=True)) the per-image CSV files as text, formatted on the device
 """
 from __future__ import annotations
 
@@ -24,7 +25,8 @@ from . import _lib
 from .model import UNetDC
 from .morphology import resize_linear_u8_device, rolling_ball_device, rolling_ball_workspace_bytes
 from .overlay import overlay_stencil_device, overlay_workspace_bytes
-from .quantify import DEFAULT_CAPACITY, DropletTables, alloc_tables, label_stats_device, label_workspace_bytes
+from .quantify import (DEFAULT_CAPACITY, CsvTables, DropletTables, alloc_tables, csv_field, csv_text_device,
+                       label_stats_device, label_workspace_bytes, pack_fields, table_csv_bounds, table_csv_device)
 
 
 @contextmanager
@@ -136,7 +138,7 @@ class DropletPipeline:
 
     # ------------------------------------------------------------------ pipelined host entry
     def run_host_pipelined(self, batches, device: torch.device | str = "cuda", copy: bool = True,
-                           want_overlay: bool = False, tables_archive: DropletTables | None = None):
+                           want_overlay: bool = False, tables_archive: DropletTables | None = None, csv: bool = False):
         """Generator over host batches (each u8 [B,H,W] or [B,H,W,3], ideally pinned; all the same shape):
         yields (masks u8 numpy [B,H,W], list of per-image column dicts) per batch, in order.
 
@@ -151,7 +153,12 @@ class DropletPipeline:
         of every mask (u8 [B,H,W], qdb:76-77).  ``tables_archive`` (from ``alloc_tables(total_frames, ...)``): the
         tables stay on the DEVICE, batch after batch in consecutive rows of the archive, and ``None`` is yielded in
         their place -- for jobs whose tables are merged elsewhere (sharded runs gather them to one rank) instead of being
-        read back batch by batch; the archive's capacity applies and is not grown."""
+        read back batch by batch; the archive's capacity applies and is not grown.
+
+        ``csv``: every item of ``batches`` is (images, filenames), and the tables come back as a ``CsvTables`` -- the
+        per-image CSV files (qdb:62-63) formatted on the device by dc_table_csv inside the batch's own stream (and CUDA
+        graph), their counts and area sums, and the one size column the reports need -- in place of the column dicts;
+        only those cross PCIe."""
         dev = torch.device(device)
         if dev.index is None:
             dev = torch.device("cuda", torch.cuda.current_device())
@@ -165,8 +172,10 @@ class DropletPipeline:
         s_outs = (s_out0, s_out1)
         slots = self._slots              # pinned allocations cost milliseconds: made once, reused by later calls
         micron = bool(self.px_per_micron)
+        if csv and tables_archive is not None:
+            raise ValueError("csv=True reads the tables back as text; it cannot keep them in a tables_archive")
 
-        def make_slot(shape):
+        def make_slot(shape, names_cap=0):
             B = shape[0]
             d = {"dev_in": torch.empty(shape, dtype=torch.uint8, device=dev),
                  "masks": torch.empty(tuple(shape[:3]), dtype=torch.uint8, device=dev),
@@ -175,21 +184,44 @@ class DropletPipeline:
                  "tables": alloc_tables(B, self.capacity, micron, dev),
                  "h_masks": torch.empty(tuple(shape[:3]), dtype=torch.uint8).pin_memory(),
                  "h_counts": torch.empty(B, dtype=torch.int32).pin_memory(),
-                 "h_cols": torch.empty((7 if micron else 5, B, self.capacity), dtype=torch.float64).pin_memory(),
+                 "h_cols": torch.empty((1 if csv else 7 if micron else 5, B, self.capacity), dtype=torch.float64).pin_memory(),
                  "ev_in": torch.cuda.Event(), "ev_run": torch.cuda.Event(), "ev_counts": torch.cuda.Event(),
-                 "ev_free": torch.cuda.Event(), "graph": None, "uses": 0}
+                 "ev_free": torch.cuda.Event(), "graph": None, "uses": 0, "names_cap": names_cap}
+            if csv:
+                # text buffer sized for the widest rows of names_cap bytes of filename fields: static for graph replay
+                nbytes, wsb = table_csv_bounds(B, self.capacity, micron, names_cap)
+                d.update({"d_names": torch.empty(names_cap, dtype=torch.uint8, device=dev),
+                          "d_name_off": torch.empty(B + 1, dtype=torch.int64, device=dev),
+                          "d_text": torch.empty(nbytes, dtype=torch.uint8, device=dev),
+                          "d_frame_off": torch.empty(B + 1, dtype=torch.int64, device=dev),
+                          "d_area_sum": torch.empty(B, dtype=torch.int64, device=dev),
+                          "csv_ws": torch.empty(wsb, dtype=torch.uint8, device=dev),
+                          "h_frame_off": torch.empty(B + 1, dtype=torch.int64).pin_memory(),
+                          "h_area_sum": torch.empty(B, dtype=torch.int64).pin_memory()})
             d["ev_free"].record(s_run)
             return d
 
-        def stage(k, host):
+        h_text = [torch.empty(0, dtype=torch.uint8)]     # pinned text read-back buffer, grown on demand
+
+        def stage(k, item):
+            host, names = item if csv else (item, None)
             host = torch.from_numpy(np.ascontiguousarray(host)) if isinstance(host, np.ndarray) else host
+            if csv:
+                if len(names) != host.shape[0]:
+                    raise ValueError(f"{host.shape[0]} images but {len(names)} filenames")
+                name_buf, name_off = pack_fields([csv_field(n) for n in names])
             sl = slots[k % 2]
             if (sl is None or sl["dev_in"].shape != host.shape or sl["tables"].capacity != self.capacity
-                    or (sl["tables"].area_um2 is not None) != micron or (sl["stencil"] is not None) != want_overlay):
-                sl = slots[k % 2] = make_slot(tuple(host.shape))
+                    or (sl["tables"].area_um2 is not None) != micron or (sl["stencil"] is not None) != want_overlay
+                    or ("d_text" in sl) != csv or (csv and name_off[-1] > sl["names_cap"])):
+                names_cap = 2 * int(name_off[-1]) + 256 if csv else 0
+                sl = slots[k % 2] = make_slot(tuple(host.shape), names_cap)
             with torch.cuda.stream(s_in):
                 s_in.wait_event(sl["ev_free"])            # the slot's previous batch has been computed and read back
                 sl["dev_in"].copy_(host, non_blocking=True)
+                if csv:
+                    sl["d_names"][:name_buf.size].copy_(torch.from_numpy(name_buf.copy()), non_blocking=True)
+                    sl["d_name_off"].copy_(torch.from_numpy(name_off), non_blocking=True)
                 sl["ev_in"].record(s_in)
 
         archive_pos = [0]
@@ -207,6 +239,9 @@ class DropletPipeline:
             def work():
                 self.run_device(sl["dev_in"], mask_out=sl["masks"], tables_out=tables_out, want_overlay=want_overlay,
                                 stencil_out=sl["stencil"])
+                if csv:
+                    table_csv_device(tables_out, sl["d_names"], sl["d_name_off"], sl["names_cap"], sl["d_text"],
+                                     sl["d_frame_off"], sl["d_area_sum"], sl["csv_ws"])
             if self.use_graphs and tables_archive is None and sl["graph"] is None and sl["uses"] >= 1:
                 # second use of the slot: every buffer the batch touches exists and is static -> capture once
                 g = torch.cuda.CUDAGraph()
@@ -224,6 +259,9 @@ class DropletPipeline:
             with torch.cuda.stream(s_out):
                 s_out.wait_event(sl["ev_run"])
                 sl["h_counts"].copy_(sl["tables"].counts, non_blocking=True)
+                if csv:
+                    sl["h_frame_off"].copy_(sl["d_frame_off"], non_blocking=True)
+                    sl["h_area_sum"].copy_(sl["d_area_sum"], non_blocking=True)
                 sl["ev_counts"].record(s_out)
                 sl["h_masks"].copy_(sl["masks"], non_blocking=True)
                 if want_overlay:
@@ -245,11 +283,19 @@ class DropletPipeline:
             sl["ev_counts"].synchronize()
             counts = sl["h_counts"].numpy().copy()
             nmax = int(counts.max()) if counts.size else 0
+            if csv:
+                text_dev, frame_off, area_sums = sl["d_text"], sl["h_frame_off"].numpy(), sl["h_area_sum"].numpy()
             if nmax > t.capacity:        # rare: rerun the table with room for everything (counts are exact)
                 with torch.cuda.stream(s_run):
                     t = label_stats_device(sl["masks"], self.min_area, self.px_per_micron, nmax)
                     self.capacity = max(self.capacity, nmax)
+                    if csv:              # the batch's own text left those frames out: format the complete table
+                        text_dev, off_dev, asum_dev = csv_text_device(t, sl["d_names"], sl["d_name_off"], sl["names_cap"])
                 s_run.synchronize()
+                if csv:
+                    frame_off, area_sums = off_dev.cpu().numpy(), asum_dev.cpu().numpy()
+            if csv:
+                return finish_csv(sl, s_out, t, counts, nmax, text_dev, frame_off.copy(), area_sums.copy())
             cols_dev = [t.area.view(torch.float64), t.eq_diam, t.centroid0, t.centroid1]
             names = ["area", "equivalent_diameter", "centroid-0", "centroid-1"]
             if micron:
@@ -277,6 +323,28 @@ class DropletPipeline:
                 st = sl["h_stencil"].numpy()
                 return masks, out, (st.copy() if copy else st)
             return masks, out
+
+        def finish_csv(sl, s_out, t, counts, nmax, text_dev, frame_off, area_sums):
+            total = int(frame_off[-1])
+            if h_text[0].numel() < total:
+                h_text[0] = torch.empty(total + total // 2, dtype=torch.uint8).pin_memory()
+            if nmax > sl["h_cols"].shape[2]:
+                sl["h_cols"] = torch.empty((1, counts.size, nmax), dtype=torch.float64).pin_memory()
+            size = t.diam_um if micron else t.eq_diam
+            with torch.cuda.stream(s_out):
+                h_text[0][:total].copy_(text_dev[:total], non_blocking=True)
+                sl["h_cols"][0, :, :nmax].copy_(size[:, :nmax], non_blocking=True)
+                sl["ev_free"].record(s_out)
+            s_out.synchronize()
+            text = h_text[0].numpy()
+            masks = sl["h_masks"].numpy()
+            out = CsvTables([text[frame_off[b]:frame_off[b + 1]].tobytes() for b in range(counts.size)],
+                            counts.astype(np.int64), area_sums,
+                            [sl["h_cols"][0, b, :n].numpy().copy() for b, n in enumerate(counts)])
+            if want_overlay:
+                st = sl["h_stencil"].numpy()
+                return (masks.copy() if copy else masks), out, (st.copy() if copy else st)
+            return (masks.copy() if copy else masks), out
 
         k = 0
         pending = []                      # batch indices staged / computed but not yet yielded

@@ -3,11 +3,15 @@
 ``quantify`` keeps the reference signature and DataFrame contract (columns ``label, area,
 equivalent_diameter, centroid-0, centroid-1`` [+ ``area_sqmicron, eq_diam_micron``]; an empty,
 column-less frame when nothing is left, qdb:87-88).  ``label_stats_device`` is the batched device
-entry the fused pipeline uses; both run ``dc_label_stats``.
+entry the fused pipeline uses; both run ``dc_label_stats``.  ``tables_to_csv`` turns a device table into the
+per-image CSV files (``dc_table_csv``), byte for byte what pandas writes for those DataFrames (qdb:62-63).
 """
 from __future__ import annotations
 
 import ctypes as C
+import csv
+import io
+import locale
 from dataclasses import dataclass
 
 import numpy as np
@@ -155,3 +159,88 @@ def quantify(bin_mask, min_area: int = 1, px_per_um: float | None = None, device
         return pd.DataFrame()                                   # qdb:87-88
     order = COLUMNS + (MICRON_COLUMNS if px_per_um else [])
     return pd.DataFrame({k: cols[k] for k in order})
+
+
+# ------------------------------------------------------------------ table -> CSV text (dc_table_csv)
+def text_encoding() -> str:
+    """The encoding Path.write_text uses (UTF-8 mode: UTF-8; otherwise the locale's)."""
+    enc = io.text_encoding(None)
+    return locale.getencoding() if enc == "locale" else enc
+
+
+def csv_field(name: str, encoding: str | None = None) -> bytes:
+    """`name` as the filename field of pandas' to_csv (csv QUOTE_MINIMAL: quoted, quotes doubled, when it holds a comma,
+    a quote or a line break), encoded as Path.write_text would (``encoding`` None) or in ``encoding``."""
+    buf = io.StringIO()
+    csv.writer(buf, lineterminator="\n", quoting=csv.QUOTE_MINIMAL).writerow([name, ""])
+    return buf.getvalue()[:-2].encode(encoding or text_encoding())
+
+
+def pack_fields(fields) -> tuple[np.ndarray, np.ndarray]:
+    """Filename fields (bytes) -> (u8 buffer, int64 offsets [B+1]) as dc_table_csv takes them."""
+    offsets = np.zeros(len(fields) + 1, dtype=np.int64)
+    offsets[1:] = np.cumsum([len(f) for f in fields])
+    return np.frombuffer(b"".join(fields) or b"\0", dtype=np.uint8), offsets
+
+
+def table_csv_bounds(B: int, capacity: int, micron: bool, names_bytes: int) -> tuple[int, int]:
+    """(text bytes that always suffice, workspace bytes) for dc_table_csv."""
+    out, ws = C.c_int64(), C.c_size_t()
+    _lib.check(_lib.load().dc_table_csv_bounds(B, capacity, int(micron), names_bytes, C.byref(out), C.byref(ws)))
+    return int(out.value), int(ws.value)
+
+
+def table_csv_device(t: "DropletTables", names: torch.Tensor, name_offsets: torch.Tensor, names_bytes: int,
+                     out: torch.Tensor, frame_offsets: torch.Tensor, area_sum: torch.Tensor, workspace: torch.Tensor):
+    """Enqueue dc_table_csv on the current stream (no synchronisation, no allocation): frame b's file text lands in
+    out[frame_offsets[b]:frame_offsets[b+1]], its area sum in area_sum[b].  names / name_offsets: device copies of
+    pack_fields(); names_bytes: the largest names total these buffers will hold (sizes the bound)."""
+    B = t.counts.shape[0]
+    micron = t.area_um2 is not None
+    args = _lib.TableCsvArgs(
+        B, t.capacity, t.counts.data_ptr(), t.area.data_ptr(), t.eq_diam.data_ptr(), t.centroid0.data_ptr(),
+        t.centroid1.data_ptr(), t.area_um2.data_ptr() if micron else None, t.diam_um.data_ptr() if micron else None,
+        names.data_ptr(), name_offsets.data_ptr(), int(names_bytes), out.data_ptr(), out.numel(),
+        frame_offsets.data_ptr(), area_sum.data_ptr(), workspace.data_ptr(), workspace.numel())
+    _lib.check(_lib.load().dc_table_csv(C.byref(args), _lib.stream_ptr(t.counts.device)))
+
+
+@dataclass
+class CsvTables:
+    """Per-image CSV files of one batch, read back to the host."""
+    texts: list                   # bytes per image: the file quantify_droplets_batch.py:63 writes
+    counts: np.ndarray            # int64 [B] droplets per image
+    area_sums: np.ndarray         # int64 [B] sum of the area column (summary_per_image.csv's total_area_px)
+    sizes: list                   # f64 per image: eq_diam_micron with micron columns, else equivalent_diameter
+
+
+def csv_text_device(t: "DropletTables", names: torch.Tensor, name_offsets: torch.Tensor, names_bytes: int):
+    """dc_table_csv into fresh device buffers on the current stream: (text u8, frame_offsets int64 [B+1], area_sum)."""
+    dev = t.counts.device
+    B = t.counts.shape[0]
+    nbytes, wsb = table_csv_bounds(B, t.capacity, t.area_um2 is not None, names_bytes)
+    out = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+    off = torch.empty(B + 1, dtype=torch.int64, device=dev)
+    asum = torch.empty(B, dtype=torch.int64, device=dev)
+    ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
+    table_csv_device(t, names, name_offsets, names_bytes, out, off, asum, ws)
+    return out, off, asum
+
+
+def tables_to_csv(t: "DropletTables", filenames) -> CsvTables:
+    """Device droplet table + one filename per image -> the per-image CSV files as bytes (synchronises).  A table whose
+    capacity some image exceeds raises DC_ECAPACITY (re-run label_stats_device with room for every droplet)."""
+    counts = t.counts.cpu().numpy().astype(np.int64)
+    if counts.size and int(counts.max()) > t.capacity:
+        raise _lib.DcError(_lib.DC_ECAPACITY, f"droplet table capacity {t.capacity} < {int(counts.max())} droplets")
+    buf, offs = pack_fields([csv_field(f) for f in filenames])
+    dev = t.counts.device
+    with torch.cuda.device(dev):
+        names = torch.from_numpy(buf.copy()).to(dev)
+        name_off = torch.from_numpy(offs).to(dev)
+        out, off, asum = csv_text_device(t, names, name_off, int(offs[-1]))
+    off = off.cpu().numpy()
+    text = out[:int(off[-1])].cpu().numpy()
+    size = t.diam_um if t.area_um2 is not None else t.eq_diam
+    sizes = [size[b, :n].cpu().numpy() for b, n in enumerate(counts)]
+    return CsvTables([text[off[b]:off[b + 1]].tobytes() for b in range(counts.size)], counts, asum.cpu().numpy(), sizes)
