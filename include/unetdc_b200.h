@@ -51,7 +51,7 @@ extern "C" {
 /* Bumped whenever a struct or signature in this header changes, or an entry point's return code for some arguments
  * does; dc_version() returns the value the library was built with and the Python binding refuses to load a library
  * that disagrees. */
-#define DC_ABI_VERSION 209
+#define DC_ABI_VERSION 210
 
 const char* dc_last_error(void);
 int dc_version(void);
@@ -168,16 +168,12 @@ int dc_conv_upfused(const dc_upfuse_args_t* args, void* stream);
  * operand is the classes' [64 co][64 ci] tiles stacked, rows [0, N/2) in the first CTA's half of the blob and
  * [N/2, N) in the second's.  Returns the number of MMAs (38) or a negative DC_E* code. */
 int dc_debug_upfuse_schedule(int* out, int cap);
-/* TEST / MEASUREMENT AID, never called on the product path: which windows dc_conv_upfused shares between classes
- * (0, the default: N = 256 / 128 / 64 MMAs as the windows allow; 1: no sharing, one N = 64 MMA per class and tap;
- * 2: sharing in the x chunks only; 3: only the four-class windows).  Weights must be packed for the mode in force
- * (dc_debug_upfuse_schedule follows it).  Process-wide. */
-int dc_debug_set_upfuse_mode(int mode);
 
 /* TEST AID, never called on the product path: pins which kernel family dc_conv_tc picks for layers that have a
  * choice, so that the fallback kernels stay under test.  AUTO (the default): CTA-pair halo kernel where it fits,
- * else single-CTA halo, else per-tap.  Process-wide; not thread-safe against concurrent launches. */
-enum { DC_CONV_FAMILY_AUTO = 0, DC_CONV_FAMILY_NO_PAIR = 1, DC_CONV_FAMILY_GENERIC = 2 };
+ * else single-CTA halo, else per-tap.  GENERIC: always the per-tap kernel.  Any other value (1 included) is
+ * DC_EINVAL.  Process-wide; not thread-safe against concurrent launches. */
+enum { DC_CONV_FAMILY_AUTO = 0, DC_CONV_FAMILY_GENERIC = 2 };
 int dc_debug_set_conv_family(int family);
 
 /* First layer (Cin = 3, models/model_2.py:10 first conv) + BatchNorm + ReLU on tcgen05: the im2col tile is

@@ -406,7 +406,7 @@ def _lib():
 def family():
     """dc_debug_set_conv_family for one test, restored to auto afterwards (import it into a test module to use it)."""
     L = _lib()
-    codes = {"auto": L.DC_CONV_FAMILY_AUTO, "no_pair": L.DC_CONV_FAMILY_NO_PAIR, "generic": L.DC_CONV_FAMILY_GENERIC}
+    codes = {"auto": L.DC_CONV_FAMILY_AUTO, "generic": L.DC_CONV_FAMILY_GENERIC}
     try:
         yield lambda name: L.check(L.load().dc_debug_set_conv_family(codes[name]))
     finally:

@@ -72,6 +72,9 @@ def test_workspace_queries_and_argument_errors_need_no_gpu():
     with pytest.raises(_lib.DcError) as ei:
         _lib.check(lib.dc_rolling_ball_workspace_bytes(1, -1, 8, 1, C.byref(n)))
     assert ei.value.code == _lib.DC_EINVAL
+    for family in (-1, 1, 3):           # the family numbers are ABI: AUTO = 0, GENERIC = 2, 1 is unassigned
+        assert lib.dc_debug_set_conv_family(family) == _lib.DC_EINVAL
+    assert lib.dc_debug_set_conv_family(_lib.DC_CONV_FAMILY_AUTO) == _lib.DC_OK
 
 
 NO_GPU_CHECK = r"""

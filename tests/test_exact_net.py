@@ -113,24 +113,18 @@ def _upf_want(x, skip, comp, skipw):
     return y[0].permute(1, 2, 0).numpy()
 
 
-@pytest.mark.parametrize("mode", [0, 1, 2, 3])
-def test_upf_model_level1_exact(mode):
+def test_upf_model_level1_exact():
     """The numpy replay of one tile pair of conv_upfused2_kernel (tests/upf_model.py) gives the exact result."""
     import upf_model as um
-    from unet_dc_segmentation_b200 import _lib, model as M
+    from unet_dc_segmentation_b200 import model as M
     from unet_dc_segmentation_b200.model import compose_upconv
     wu, bu, wd, bd = en.upfused_operands(64, 3, "dense")
     comp, skipw, _ = compose_upconv(wu.float(), bu.float(), wd.float(), bd.float())
     x, skip = en.acts((20, 12, 128), 4), en.acts((40, 24, 64), 5)
-    lib = _lib.load()
-    _lib.check(lib.dc_debug_set_upfuse_mode(mode))
-    try:
-        blob = M.pack_upfused(comp, skipw).float().numpy()
-    finally:
-        _lib.check(lib.dc_debug_set_upfuse_mode(0))
+    blob = M.pack_upfused(comp, skipw).float().numpy()
     got = np.zeros((40, 24, 64), np.float32)
     for tiles in ([(0, 0), (0, 8)], [(16, 0), (16, 8)]):
-        acc = um.level1_tile_pair(x.float().numpy(), skip.float().numpy(), blob, tiles, mode)
+        acc = um.level1_tile_pair(x.float().numpy(), skip.float().numpy(), blob, tiles)
         for c, (h0, w0) in enumerate(tiles):
             um.scatter_level1(acc[c], h0, w0, got)
     np.testing.assert_array_equal(got, _upf_want(x, skip, comp, skipw))

@@ -15,7 +15,7 @@ def conv_family():
     """dc_debug_set_conv_family for the duration of one test (the product path never calls it)."""
     from unet_dc_segmentation_b200 import _lib
     lib = _lib.load()
-    codes = {"auto": _lib.DC_CONV_FAMILY_AUTO, "no_pair": _lib.DC_CONV_FAMILY_NO_PAIR, "generic": _lib.DC_CONV_FAMILY_GENERIC}
+    codes = {"auto": _lib.DC_CONV_FAMILY_AUTO, "generic": _lib.DC_CONV_FAMILY_GENERIC}
     yield lambda name: _lib.check(lib.dc_debug_set_conv_family(codes[name]))
     _lib.check(lib.dc_debug_set_conv_family(_lib.DC_CONV_FAMILY_AUTO))
 
@@ -54,7 +54,7 @@ CONV_CASES = [
     (1, 16, 16, 256, 512, 8),     # two N tiles
     (2, 8, 8, 512, 1024, 16),     # dilation > map: only the centre tap is in bounds
     (1, 16, 32, 1024, 512, 1),    # long K
-    (3, 40, 24, 192, 64, 3),      # Cin not a power of two, odd dilation
+    (3, 40, 24, 192, 64, 3),      # Cin not a power of two, odd dilation; single-CTA halo kernel, weights streamed
     (2, 48, 24, 128, 64, 1),      # dec1.0 shape: halo kernel, two chunks, weights resident
     (1, 40, 40, 64, 128, 2),      # enc2.0 shape: halo kernel, BN = 128, dilation 2
     (1, 32, 16, 64, 64, 4),       # halo kernel, dilation 4
@@ -90,23 +90,19 @@ def test_conv3x3_generic_path_forced(cuda_device, conv_family, B, H, W, cin, cou
     test_conv3x3_store(cuda_device, B, H, W, cin, cout, d)
 
 
-@pytest.mark.parametrize("B,H,W,cin,cout,d", [(2, 16, 32, 64, 64, 1), (2, 48, 24, 128, 64, 1), (1, 40, 40, 64, 128, 2),
-                                               (2, 16, 16, 128, 128, 2), (3, 40, 24, 192, 64, 3)])
-def test_conv3x3_single_cta_halo_forced(cuda_device, conv_family, B, H, W, cin, cout, d):
-    """DC_CONV_FAMILY_NO_PAIR keeps the single-CTA halo kernel (resident and streamed weights) covered."""
-    conv_family("no_pair")
-    test_conv3x3_store(cuda_device, B, H, W, cin, cout, d)
-
-
-@pytest.mark.parametrize("family", ["generic", "no_pair"])
+@pytest.mark.parametrize("family", ["generic", "single_cta"])
 def test_fused_epilogues_on_the_fallback_kernels(cuda_device, conv_family, family):
-    """Pool, head and transposed-conv epilogues through the per-tap kernel and the single-CTA halo kernel (one or two
-    halves per tile: an epilogue group can be left without a half of its own in the head epilogue)."""
-    conv_family(family)
-    test_conv3x3_store_pool(cuda_device, 1, 16, 32, 64, 1)
-    test_conv3x3_store_pool(cuda_device, 2, 24, 48, 128, 2)
-    test_head_epilogue(cuda_device)
-    test_upconv2x2(cuda_device, 1, 8, 16, 128, 64)
+    """Pool, head and transposed-conv epilogues through the per-tap kernel (forced), and pool and head through the
+    single-CTA halo kernel, which AUTO picks for 256 -> 64 at dilation 1."""
+    if family == "generic":
+        conv_family("generic")
+        _store_pool(1, 16, 32, 64, 64, 1)
+        _store_pool(2, 24, 48, 128, 128, 2)
+        _head(64)
+        test_upconv2x2(cuda_device, 1, 8, 16, 128, 64)
+    else:
+        _store_pool(2, 24, 32, 256, 64, 1)
+        _head(256)
 
 
 def test_conv3x3_no_relu_and_channel_slices(cuda_device):
@@ -125,14 +121,13 @@ def test_conv3x3_no_relu_and_channel_slices(cuda_device):
     assert bool((out[..., :64].float() == 7.0).all()), "wrote outside its channel slice"
 
 
-@pytest.mark.parametrize("B,H,W,c,d", [(1, 16, 32, 64, 1), (2, 24, 48, 128, 2), (1, 16, 16, 256, 4)])
-def test_conv3x3_store_pool(cuda_device, B, H, W, c, d):
+def _store_pool(B, H, W, cin, cout, d):
     import torch
     import torch.nn.functional as F
     from unet_dc_segmentation_b200 import layers
     from unet_dc_segmentation_b200.model import pack_conv3x3
-    w, b = _rand_layer(c, c, 77 + c)
-    x = _rand_act(B, H, W, c, 3 + c)
+    w, b = _rand_layer(cin, cout, 77 + cin)
+    x = _rand_act(B, H, W, cin, 3 + cin)
     full = F.relu(F.conv2d(x.float().permute(0, 3, 1, 2), w, b, padding=d, dilation=d))
     got, pooled = layers.conv3x3(x.cuda(), pack_conv3x3(w).cuda(), b.cuda(), dilation=d, pool=True)
     torch.cuda.synchronize()
@@ -140,6 +135,11 @@ def test_conv3x3_store_pool(cuda_device, B, H, W, c, d):
     # the pooled tensor must be EXACTLY the 2x2 max of the bf16 full-res tensor the kernel wrote
     want_pool = F.max_pool2d(got.float().cpu().permute(0, 3, 1, 2), 2).permute(0, 2, 3, 1)
     assert torch.equal(pooled.float().cpu(), want_pool)
+
+
+@pytest.mark.parametrize("B,H,W,c,d", [(1, 16, 32, 64, 1), (2, 24, 48, 128, 2), (1, 16, 16, 256, 4)])
+def test_conv3x3_store_pool(cuda_device, B, H, W, c, d):
+    _store_pool(B, H, W, c, c, d)
 
 
 @pytest.mark.parametrize("B,H,W,cin,cout", [(1, 8, 16, 128, 64), (2, 12, 20, 256, 128), (1, 8, 8, 1024, 512)])
@@ -285,16 +285,16 @@ def test_conv3x3_parity_class_kernel(cuda_device, B, H, W):
     assert torch.equal(mask.cpu(), (prob.cpu() > 0.3).to(torch.uint8))
 
 
-def test_head_epilogue(cuda_device):
+def _head(cin):
     import torch
     import torch.nn.functional as F
     from unet_dc_segmentation_b200 import layers
     from unet_dc_segmentation_b200.model import pack_conv3x3
-    w, b = _rand_layer(64, 64, 31)
+    w, b = _rand_layer(cin, 64, 31)
     g = torch.Generator().manual_seed(2)
     hw = torch.randn(64, generator=g) * 0.3
     hb = -0.2
-    x = _rand_act(2, 24, 32, 64, 13)
+    x = _rand_act(2, 24, 32, cin, 13)
     feat = F.relu(F.conv2d(x.float().permute(0, 3, 1, 2), w, b, padding=1))
     want = torch.sigmoid((feat * hw.view(1, -1, 1, 1)).sum(1) + hb)
     prob, mask = layers.conv3x3_head(x.cuda(), pack_conv3x3(w).cuda(), b.cuda(), hw.cuda(), hb, 0.3)
@@ -302,6 +302,10 @@ def test_head_epilogue(cuda_device):
     err = (prob.cpu() - want).abs().max()
     assert float(err) < 2e-3, f"head prob max err {float(err)}"             # no bf16 rounding of the features here
     assert torch.equal(mask.cpu(), (prob.cpu() > 0.3).to(torch.uint8))     # mask is exactly `prob > thresh`
+
+
+def test_head_epilogue(cuda_device):
+    _head(64)
 
 
 @pytest.mark.parametrize("kind", ["f32_nchw", "u8_gray", "u8_hwc"])

@@ -21,7 +21,7 @@ pytestmark = pytest.mark.gpu
 
 GUARD, SENT, SENT16 = en.GUARD, en.SENT, en.SENT16
 THRESH = 0.3
-FAMILIES = ("auto", "no_pair", "generic")
+FAMILIES = ("auto", "generic")
 
 CONV_CASES = [
     (1, 8, 16, 64, 64, 1), (2, 16, 32, 64, 64, 1), (1, 24, 40, 64, 128, 2), (2, 16, 16, 128, 128, 2),
@@ -125,18 +125,18 @@ def test_conv_store_exact_random(cuda_device, B, H, W, cin, cout, d, relu, kind,
                 seed=seed)
 
 
-def _pool_case(B, H, W, c, d, kind, case, par=False):
+def _pool_case(B, H, W, cin, c, d, kind, case, par=False):
     from unet_dc_segmentation_b200.model import pack_conv3x3, pack_par3x3
     L = _lib()
-    x64, w64, b64, pre = _conv_ref(B, H, W, c, c, d, kind, 7)
+    x64, w64, b64, pre = _conv_ref(B, H, W, cin, c, d, kind, 7)
     want = pre.clamp(min=0)
-    x = _nan_padded(x64, c + 64)
+    x = _nan_padded(x64, cin + 64)
     raw, out = _guarded((B, H, W, c + 32), torch.bfloat16)
     praw, pooled = _guarded((B, H // 2, W // 2, c), torch.bfloat16)
     wp, bias = pack_conv3x3(w64).cuda(), b64.float().cuda()
     wpar = pack_par3x3(w64.float()).cuda() if par else None
-    _conv(kind=L.DC_KIND_CONV3X3, epilogue=L.DC_EPI_STORE_POOL, relu=1, B=B, H=H, W=W, Cin=c, Cout=c, dilation=d,
-          in_=x.data_ptr(), in_stride=c + 64, weight=wp.data_ptr(), bias=bias.data_ptr(), out=out.data_ptr(),
+    _conv(kind=L.DC_KIND_CONV3X3, epilogue=L.DC_EPI_STORE_POOL, relu=1, B=B, H=H, W=W, Cin=cin, Cout=c, dilation=d,
+          in_=x.data_ptr(), in_stride=cin + 64, weight=wp.data_ptr(), bias=bias.data_ptr(), out=out.data_ptr(),
           out_stride=c + 32, out_offset=16, pool_out=pooled.data_ptr(), pool_stride=c,
           weight_par=wpar.data_ptr() if par else None)
     en.assert_exact(out[..., 16:16 + c], want, f"{case}: full-res output")
@@ -146,21 +146,21 @@ def _pool_case(B, H, W, c, d, kind, case, par=False):
     _check_guards(praw, f"{case}: pooled output")
 
 
-def _head_case(B, H, W, d, case, par=False):
+def _head_case(B, H, W, cin, d, case, par=False):
     from unet_dc_segmentation_b200.model import pack_conv3x3, pack_par3x3
     L = _lib()
-    x64, w64, b64, pre = _conv_ref(B, H, W, 64, 64, d, "sparse", 11)
+    x64, w64, b64, pre = _conv_ref(B, H, W, cin, 64, d, "sparse", 11)
     feat = pre.clamp(min=0)
     hw, hb = _head_weights(feat, 3)
     logits = feat @ hw + hb
-    x = _nan_padded(x64, 128)
+    x = _nan_padded(x64, cin + 64)
     wp, bias = pack_conv3x3(w64).cuda(), b64.float().cuda()
     wpar = pack_par3x3(w64.float()).cuda() if par else None
     hwd = hw.float().cuda()
     praw, prob = _guarded((B, H, W), torch.float32)
     mraw, mask = _guarded((B, H, W), torch.uint8)
-    _conv(kind=L.DC_KIND_CONV3X3, epilogue=L.DC_EPI_HEAD, relu=1, B=B, H=H, W=W, Cin=64, Cout=64, dilation=d,
-          in_=x.data_ptr(), in_stride=128, weight=wp.data_ptr(), bias=bias.data_ptr(), head_w=hwd.data_ptr(), head_b=hb,
+    _conv(kind=L.DC_KIND_CONV3X3, epilogue=L.DC_EPI_HEAD, relu=1, B=B, H=H, W=W, Cin=cin, Cout=64, dilation=d,
+          in_=x.data_ptr(), in_stride=cin + 64, weight=wp.data_ptr(), bias=bias.data_ptr(), head_w=hwd.data_ptr(), head_b=hb,
           thresh=THRESH, prob_out=prob.data_ptr(), mask_out=mask.data_ptr(), weight_par=wpar.data_ptr() if par else None)
     en.assert_probs(prob, mask, logits, THRESH, case)
     _check_guards(praw, f"{case}: prob")
@@ -169,11 +169,13 @@ def _head_case(B, H, W, d, case, par=False):
 
 @pytest.mark.parametrize("fam", FAMILIES)
 def test_pool_and_head_epilogues_exact(cuda_device, family, fam):
+    """256 -> 64 at dilation 1 is a single-CTA halo layer (conv_halo_kernel) in AUTO."""
     family(fam)
-    for B, H, W, c, d in [(1, 16, 32, 64, 1), (2, 24, 48, 128, 2), (1, 16, 16, 256, 4), (1, 18, 34, 64, 1)]:
-        _pool_case(B, H, W, c, d, "dense" if c > 64 else "sparse", f"pool {c} d{d} {B}x{H}x{W} family={fam}")
-    for B, H, W, d in [(2, 24, 32, 1), (1, 17, 29, 1), (2, 16, 8, 2)]:
-        _head_case(B, H, W, d, f"head {B}x{H}x{W} d{d} family={fam}")
+    for B, H, W, cin, c, d in [(1, 16, 32, 64, 64, 1), (2, 24, 48, 128, 128, 2), (1, 16, 16, 256, 256, 4),
+                               (1, 18, 34, 64, 64, 1), (2, 24, 32, 256, 64, 1)]:
+        _pool_case(B, H, W, cin, c, d, "dense" if cin > 64 else "sparse", f"pool {cin}->{c} d{d} {B}x{H}x{W} family={fam}")
+    for B, H, W, cin, d in [(2, 24, 32, 64, 1), (1, 17, 29, 64, 1), (2, 16, 8, 64, 2), (1, 24, 40, 256, 1)]:
+        _head_case(B, H, W, cin, d, f"head {cin}->64 {B}x{H}x{W} d{d} family={fam}")
 
 
 @pytest.mark.parametrize("B,H,W", PARITY_CASES)
@@ -191,8 +193,8 @@ def test_parity_class_kernel_exact(cuda_device, B, H, W):
           out_offset=16, weight_par=wpar.data_ptr())
     en.assert_exact(out[..., 16:80], pre, f"{case}: store")
     _check_outside(raw, out, 16, 64, case)
-    _pool_case(B, H, W, 64, 1, "dense", f"{case}: pool", par=True)
-    _head_case(B, H, W, 1, f"{case}: head", par=True)
+    _pool_case(B, H, W, 64, 64, 1, "dense", f"{case}: pool", par=True)
+    _head_case(B, H, W, 64, 1, f"{case}: head", par=True)
 
 
 @pytest.mark.parametrize("fam", FAMILIES)
@@ -218,7 +220,7 @@ def test_upconv_exact(cuda_device, family, fam, B, H, W, cin, cout):
     _check_outside(raw, out, 16, cout, case)
 
 
-def _upfused_case(C, B, H, W, kind, relu, case, mode=0, bias9_edit=None):
+def _upfused_case(C, B, H, W, kind, relu, case, bias9_edit=None):
     """dc_conv_upfused on integer operands against the unfused float64 chain.  x is read at channels [0, 2C) of a
     2C + 64 wide buffer, skip at [64, 64 + C) of a C + 128 wide one; everything else is NaN."""
     from unet_dc_segmentation_b200.model import compose_upconv, pack_upfused, pack_upfused_wide
@@ -234,41 +236,32 @@ def _upfused_case(C, B, H, W, kind, relu, case, mode=0, bias9_edit=None):
         bias9[bias9_edit] += 1.0
     ws = None
     if C == 64:
-        L.check(lib.dc_debug_set_upfuse_mode(mode))
-        try:
-            wx = pack_upfused(comp, skipw).cuda()
-        except BaseException:
-            L.check(lib.dc_debug_set_upfuse_mode(0))
-            raise
+        wx = pack_upfused(comp, skipw).cuda()
     else:
         wx, ws = (t.cuda() for t in pack_upfused_wide(comp, skipw))
-    try:
-        x = _nan_padded(x64, 2 * C + 64)
-        skip = _nan_padded(s64, C + 128, off=64)
-        raw, out = _guarded((B, 2 * H, 2 * W, C + 32), torch.bfloat16)
-        b9 = bias9.cuda()
-        a = L.UpfuseArgs()
-        a.B, a.H, a.W, a.channels = B, H, W, C
-        a.x, a.x_stride = x.data_ptr(), 2 * C + 64
-        a.skip, a.skip_stride = skip.data_ptr() + 2 * 64, C + 128
-        a.weight, a.bias9, a.relu = wx.data_ptr(), b9.data_ptr(), int(relu)
-        if ws is not None:
-            a.weight_skip = ws.data_ptr()
-        a.out, a.out_stride, a.out_offset = out.data_ptr(), C + 32, 16
-        L.check(lib.dc_conv_upfused(ctypes.byref(a), L.stream_ptr()))
-        torch.cuda.synchronize()
-    finally:
-        L.check(lib.dc_debug_set_upfuse_mode(0))
+    x = _nan_padded(x64, 2 * C + 64)
+    skip = _nan_padded(s64, C + 128, off=64)
+    raw, out = _guarded((B, 2 * H, 2 * W, C + 32), torch.bfloat16)
+    b9 = bias9.cuda()
+    a = L.UpfuseArgs()
+    a.B, a.H, a.W, a.channels = B, H, W, C
+    a.x, a.x_stride = x.data_ptr(), 2 * C + 64
+    a.skip, a.skip_stride = skip.data_ptr() + 2 * 64, C + 128
+    a.weight, a.bias9, a.relu = wx.data_ptr(), b9.data_ptr(), int(relu)
+    if ws is not None:
+        a.weight_skip = ws.data_ptr()
+    a.out, a.out_stride, a.out_offset = out.data_ptr(), C + 32, 16
+    L.check(lib.dc_conv_upfused(ctypes.byref(a), L.stream_ptr()))
+    torch.cuda.synchronize()
     en.assert_exact(out[..., 16:16 + C], want, case)
     _check_outside(raw, out, 16, C, case)
 
 
-@pytest.mark.parametrize("mode", [0, 1, 2, 3])
 @pytest.mark.parametrize("B,H,W", UPFUSED_CASES)
-def test_upfused_level1_exact(cuda_device, mode, B, H, W):
-    """conv_upfused2_kernel (C = 64) under every MMA schedule mode (blob repacked for the mode, mode restored)."""
+def test_upfused_level1_exact(cuda_device, B, H, W):
+    """conv_upfused2_kernel (C = 64)."""
     for relu, kind in ((True, "dense"), (False, "sparse")):
-        _upfused_case(64, B, H, W, kind, relu, f"upfused C=64 {B}x{H}x{W} {kind} relu={relu} mode={mode}", mode=mode)
+        _upfused_case(64, B, H, W, kind, relu, f"upfused C=64 {B}x{H}x{W} {kind} relu={relu}")
 
 
 @pytest.mark.parametrize("C,B,H,W", WIDE_CASES)
@@ -378,25 +371,21 @@ def _forward(m, in_kind, x, B, H, W, want_prob=True, want_mask=True):
 
 def _schedules():
     """(label, setup(model, lib)) of every schedule: default, the switch combinations, fully unfused; then all of them
-    under the two forced kernel families and under upfuse modes 1-3."""
+    with the per-tap kernel forced."""
     base = [("default", {})]
     base += [(f"parity={layers} fused={levels}", {"parity_layers": layers, "fuse_levels": levels}) for layers, levels in SWITCHES]
     base += [("unfused", {"fuse_level1": False, "parity_level1": False, "fuse_levels": ()})]
-    out = [(lbl, attrs, "auto", 0) for lbl, attrs in base]
-    out += [(lbl, attrs, fam, 0) for fam in ("no_pair", "generic") for lbl, attrs in base]
-    out += [(lbl, attrs, "auto", mode) for mode in (1, 2, 3) for lbl, attrs in base if attrs.get("fuse_level1", True)]
-    return out
+    return [(lbl, attrs, fam) for fam in FAMILIES for lbl, attrs in base]
 
 
-def _run_schedule(m, attrs, fam, mode, fn):
+def _run_schedule(m, attrs, fam, fn):
     import unet_dc_segmentation_b200 as pkg
     L = _lib()
     lib = L.load()
-    codes = {"auto": L.DC_CONV_FAMILY_AUTO, "no_pair": L.DC_CONV_FAMILY_NO_PAIR, "generic": L.DC_CONV_FAMILY_GENERIC}
+    codes = {"auto": L.DC_CONV_FAMILY_AUTO, "generic": L.DC_CONV_FAMILY_GENERIC}
     for k, v in attrs.items():
         setattr(m, k, v)
     try:
-        L.check(lib.dc_debug_set_upfuse_mode(mode))
         L.check(lib.dc_debug_set_conv_family(codes[fam]))
         m.invalidate()
         if attrs.get("fuse_level1") is False:
@@ -404,7 +393,6 @@ def _run_schedule(m, attrs, fam, mode, fn):
         return fn()
     finally:
         L.check(lib.dc_debug_set_conv_family(L.DC_CONV_FAMILY_AUTO))
-        L.check(lib.dc_debug_set_upfuse_mode(0))
         for k in attrs:
             setattr(m, k, getattr(pkg.UNetDC, k))
         m.invalidate()
@@ -420,9 +408,9 @@ def test_forward_every_schedule_exact(cuda_device, refs, shape):
     rgb = u8.cuda()
     mu = _model("unetdc", en.u8_stem(sd), dil)
     first = None
-    for lbl, attrs, fam, mode in _schedules():
-        case = f"forward {B}x{H}x{W} schedule {lbl} family={fam} upfuse_mode={mode}"
-        prob, mask = _run_schedule(mu, attrs, fam, mode, lambda: _forward(mu, 2, rgb, B, H, W))
+    for lbl, attrs, fam in _schedules():
+        case = f"forward {B}x{H}x{W} schedule {lbl} family={fam}"
+        prob, mask = _run_schedule(mu, attrs, fam, lambda: _forward(mu, 2, rgb, B, H, W))
         en.assert_probs(prob[:, 0], mask, logits[:, 0], THRESH, case)
         if first is None:
             first = (prob, mask)
@@ -443,7 +431,7 @@ def test_forward_other_networks_exact(cuda_device, refs, name):
         x = x64.float().contiguous().cuda()
         prob, mask = _forward(m, 0, x, B, H, W)
         en.assert_probs(prob, mask, logits, THRESH, f"{name} {shape} default")
-        p2, m2 = _run_schedule(m, {"fuse_level1": False, "parity_level1": False, "fuse_levels": ()}, "auto", 0,
+        p2, m2 = _run_schedule(m, {"fuse_level1": False, "parity_level1": False, "fuse_levels": ()}, "auto",
                                lambda: _forward(m, 0, x, B, H, W))
         assert torch.equal(prob, p2) and torch.equal(mask, m2), f"{name} {shape}: unfused schedule differs"
 

@@ -210,12 +210,10 @@ def test_split_head_real(cuda_device, cin, d):
 # ----------------------------------------------------------------------------- real-valued bf16 layers
 
 # (B, H, W, Cin, Cout, dilation, family, K order): pair kernel (auto, d <= 4, BN 64 / 128 / 256 resident or streamed),
-# single-CTA halo (no_pair, Cout = BN <= 128), per-tap kernel (generic; auto at dilation 8 / 16)
+# single-CTA halo (auto, Cout = 64 with long K), per-tap kernel (generic; auto at dilation 8 / 16)
 BF16_CASES = [(1, 16, 16, 64, 64, 1, "auto", "chunk"), (2, 24, 40, 128, 128, 2, "auto", "chunk"),
               (1, 32, 24, 64, 128, 4, "auto", "chunk"), (1, 16, 32, 256, 256, 1, "auto", "chunk"),
-              (1, 12, 20, 512, 512, 3, "auto", "chunk"),
-              (1, 16, 16, 64, 64, 1, "no_pair", "chunk"), (2, 24, 40, 128, 128, 2, "no_pair", "chunk"),
-              (1, 12, 20, 256, 64, 3, "no_pair", "chunk"), (1, 40, 24, 1024, 128, 1, "no_pair", "chunk"),
+              (1, 12, 20, 512, 512, 3, "auto", "chunk"), (1, 12, 20, 256, 64, 3, "auto", "chunk"),
               (1, 16, 16, 64, 64, 1, "generic", "tap"), (2, 24, 40, 128, 256, 2, "generic", "tap"),
               (1, 16, 16, 256, 512, 8, "auto", "tap"), (2, 8, 8, 512, 512, 16, "auto", "tap"),
               (1, 16, 32, 1024, 512, 1, "generic", "tap")]

@@ -248,7 +248,7 @@ def test_pack_upfused_wide_layout():
 
 def test_upf_schedule_issue_code_matches_its_tables():
     """The straight-line MMA issue code of csrc/upf_schedule.inc (literal descriptor offsets) against the definitions:
-    per (mode, chunk kind, group) every MMA reads the window of its table entry (x chunk: (r*10 + c)*8; skip chunk:
+    per (chunk kind, group) every MMA reads the window of its table entry (x chunk: (r*10 + c)*8; skip chunk:
     column-parity plane (c & 1), row r, column c >> 1 of a 9-wide plane), takes its weights from the next free 32-row
     sub-tile of the group's ring slot, writes the accumulator of its first class with N = 64 * classes, and only the
     first MMA to touch a class in a tile's first chunk may overwrite."""
@@ -256,15 +256,16 @@ def test_upf_schedule_issue_code_matches_its_tables():
     from pathlib import Path
     txt = (Path(__file__).resolve().parent.parent / "unet_dc_segmentation_b200" / "csrc" / "upf_schedule.inc").read_text()
     ops = {}
-    for m in re.finditer(r"upf_(u|s)_op<(\d)>\(int i\) \{\s*switch \(i\) \{(.*?)default", txt, re.S):
-        ops[(m.group(1), int(m.group(2)))] = [tuple(int(v) for v in t) for t in
-                                              re.findall(r"UpfOp\{(\d+), (\d+), (\d+), (\d+)\}", m.group(3))]
-    assert len(ops) == 8
+    for m in re.finditer(r"upf_(u|s)_op\(int i\) \{\s*switch \(i\) \{(.*?)default", txt, re.S):
+        ops[m.group(1)] = [tuple(int(v) for v in t) for t in re.findall(r"UpfOp\{(\d+), (\d+), (\d+), (\d+)\}", m.group(2))]
+    assert len(ops) == 2
     plane = (9 * 34 * 128) >> 4
-    for m in re.finditer(r"upf_issue_group<(\d), (\d), (\d)>\(.*?\) \{(.*?)\n\}", txt, re.S):
-        mode, kind, g = int(m.group(1)), int(m.group(2)), int(m.group(3))
-        calls = re.findall(r"umma_bf16_2sm\(d \+ (\d+)u, a \+ (\d+)ull, b \+ (\d+)ull, 0x([0-9a-f]+)u, ([^)]*)\);", m.group(4))
-        table = ops[("u" if kind == 0 else "s", mode)]
+    groups = 0
+    for m in re.finditer(r"upf_issue_group<(\d), (\d)>\(.*?\) \{(.*?)\n\}", txt, re.S):
+        kind, g = int(m.group(1)), int(m.group(2))
+        groups += 1
+        calls = re.findall(r"umma_bf16_2sm\(d \+ (\d+)u, a \+ (\d+)ull, b \+ (\d+)ull, 0x([0-9a-f]+)u, ([^)]*)\);", m.group(3))
+        table = ops["u" if kind == 0 else "s"]
         # the group's entries: groups are consecutive runs of the table whose classes add up to 4
         runs, cur, tot = [], [], 0
         for o in table:
@@ -285,3 +286,4 @@ def test_upf_schedule_issue_code_matches_its_tables():
                 sub += ncls
         if kind != 1 and g == 0:
             assert any("fresh" in c[4] for c in calls)
+    assert groups == 4 + 2 * 9          # x chunk; skip chunk after the x chunks and on its own

@@ -34,22 +34,16 @@ def _want(x, skip, comp, skipw, bias9):
     return y[0].permute(1, 2, 0).numpy()
 
 
-@pytest.mark.parametrize("mode", [0, 1, 2, 3])
-def test_level1_model(mode):
+def test_level1_model():
     """Level 1 (C = 64): image of 20 x 12 half-resolution pixels = tiles (0,0), (0,8) (ragged) and (16,0), (16,8):
     every border class, zero fill on all four sides, both CTAs of a pair."""
-    from unet_dc_segmentation_b200 import _lib, model as M
+    from unet_dc_segmentation_b200 import model as M
     comp, skipw, bias9 = _layer(64, 1)
     x, skip = _acts(64, 20, 12, 2)
-    lib = _lib.load()
-    _lib.check(lib.dc_debug_set_upfuse_mode(mode))
-    try:
-        blob = M.pack_upfused(comp, skipw).float().numpy()
-    finally:
-        _lib.check(lib.dc_debug_set_upfuse_mode(0))
+    blob = M.pack_upfused(comp, skipw).float().numpy()
     got = np.zeros((40, 24, 64), np.float32)
     for tiles in ([(0, 0), (0, 8)], [(16, 0), (16, 8)]):
-        acc = um.level1_tile_pair(x.numpy(), skip.numpy(), blob, tiles, mode)
+        acc = um.level1_tile_pair(x.numpy(), skip.numpy(), blob, tiles)
         for c, (h0, w0) in enumerate(tiles):
             um.scatter_level1(acc[c], h0, w0, got)
     want = _want(x, skip, comp, skipw, bias9)

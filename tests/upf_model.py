@@ -22,11 +22,11 @@ PLANE16 = (S_W * S_H * 128) >> 4         # plane size in descriptor units (16 by
 INC = Path(__file__).resolve().parent.parent / "unet_dc_segmentation_b200" / "csrc" / "upf_schedule.inc"
 
 
-def issue_code(mode: int, kind: int):
+def issue_code(kind: int):
     """[(group, [(d, a, b, N, fresh_at_k0), ...])] parsed from the generated issue functions."""
     txt = INC.read_text()
     out = []
-    for m in re.finditer(rf"upf_issue_group<{mode}, {kind}, (\d)>\(.*?\) \{{(.*?)\n\}}", txt, re.S):
+    for m in re.finditer(rf"upf_issue_group<{kind}, (\d)>\(.*?\) \{{(.*?)\n\}}", txt, re.S):
         calls = re.findall(r"umma_bf16_2sm\(d \+ (\d+)u, a \+ (\d+)ull, b \+ (\d+)ull, 0x([0-9a-f]+)u, ([^)]*)\);", m.group(2))
         out.append((int(m.group(1)), [(int(d), int(a), int(b), ((int(i, 16) >> 17) & 0x3F) << 3, "fresh" in acc)
                                       for d, a, b, i, acc in calls]))
@@ -66,7 +66,7 @@ def window(region_flat_rows, start_row16, sbo_rows):
     return np.stack([region_flat_rows[s + g * sbo_rows + r] for g in range(16) for r in range(8)])      # [128, 64]
 
 
-def level1_tile_pair(x, skip, blob, tiles, mode=0):
+def level1_tile_pair(x, skip, blob, tiles):
     """conv_upfused2_kernel for one pair of tiles [(h0, w0) of CTA 0, (h0, w0) of CTA 1]; x [H,W,128], skip [2H,2W,64],
     blob [2, 2176, 64] (model.pack_upfused).  Returns per CTA the four accumulators [4 slots][128 px][64]."""
     acc = np.zeros((2, 256, 128), np.float32)             # [cta][tmem column = slot * 64 + co][lane = pixel]
@@ -78,7 +78,7 @@ def level1_tile_pair(x, skip, blob, tiles, mode=0):
             flat = [x_region(x, h0, w0, chunk).reshape(-1, 64) for h0, w0 in tiles]
         else:
             flat = [skip_planes(skip, h0, w0, 0).reshape(-1, 64) for h0, w0 in tiles]
-        for g, calls in issue_code(mode, kind):
+        for g, calls in issue_code(kind):
             slot_rows = [blob[c, row:row + 128].astype(np.float32) for c in range(2)]      # this group's ring slot per CTA
             row += 128
             per_k = len(calls) // 4

@@ -45,45 +45,36 @@ def timed(fn, n=7):
     return statistics.median(ts[2:])
 
 
-from unet_dc_segmentation_b200 import _lib                                      # noqa: E402
-t2 = timed(two)
-print(f"B {B} H {H} W {W}: upconv1 + dec1.0 as two launches {t2:.3f} ms")
-modes = [int(v) for v in sys.argv[4].split(",")] if len(sys.argv) > 4 else [0, 1, 2, 3]
-for mode in modes:
-    _lib.check(_lib.load().dc_debug_set_upfuse_mode(mode))
-    fw = pack_upfused(comp, skipw).to(dev)
-    out2.zero_()
-    tf = timed(fused)
-    d = (out.float() - out2.float()).abs()
-    print(f"  mode {mode}: fused {tf:.3f} ms, max |diff| {float(d.max()):.4f} mean {float(d.mean()):.5f}")
-_lib.check(_lib.load().dc_debug_set_upfuse_mode(0))
+t2, tf = timed(two), timed(fused)
+d = (out.float() - out2.float()).abs()
+print(f"B {B} H {H} W {W}: upconv1 + dec1.0 as two launches {t2:.3f} ms, fused {tf:.3f} ms, "
+      f"max |diff| {float(d.max()):.4f} mean {float(d.mean()):.5f}")
 
 
 # ---- levels 2..4 at the benchmark shapes: upconv + dec.0 as two launches against conv_upfused_wide_kernel
 from unet_dc_segmentation_b200.model import pack_upfused_wide                    # noqa: E402
-if len(sys.argv) <= 4:
-    for C, Hh in ((128, 256), (256, 128), (512, 64)):
-        wu = torch.randn(2 * C, C, 2, 2, generator=g) / (2 * C) ** 0.5
-        bu = torch.randn(C, generator=g) * 0.3
-        wd = torch.randn(C, 2 * C, 3, 3, generator=g) / (3.0 * (2 * C) ** 0.5)
-        bd = torch.randn(C, generator=g) * 0.1
-        comp, skipw, fb = compose_upconv(wu, bu, wd, bd)
-        wx, ws = (t.to(dev) for t in pack_upfused_wide(comp, skipw))
-        fb = fb.to(dev)
-        pu, pd = pack_upconv(wu).to(dev), pack_conv3x3(wd).to(dev)
-        bu_d, bd_d = bu.to(dev), bd.to(dev)
-        x = torch.randn((B, Hh, Hh, 2 * C), device=dev).bfloat16()
-        cat = torch.randn((B, 2 * Hh, 2 * Hh, 2 * C), device=dev).bfloat16()
-        o1 = torch.empty((B, 2 * Hh, 2 * Hh, C), dtype=torch.bfloat16, device=dev)
-        o2 = torch.empty_like(o1)
+for C, Hh in ((128, 256), (256, 128), (512, 64)):
+    wu = torch.randn(2 * C, C, 2, 2, generator=g) / (2 * C) ** 0.5
+    bu = torch.randn(C, generator=g) * 0.3
+    wd = torch.randn(C, 2 * C, 3, 3, generator=g) / (3.0 * (2 * C) ** 0.5)
+    bd = torch.randn(C, generator=g) * 0.1
+    comp, skipw, fb = compose_upconv(wu, bu, wd, bd)
+    wx, ws = (t.to(dev) for t in pack_upfused_wide(comp, skipw))
+    fb = fb.to(dev)
+    pu, pd = pack_upconv(wu).to(dev), pack_conv3x3(wd).to(dev)
+    bu_d, bd_d = bu.to(dev), bd.to(dev)
+    x = torch.randn((B, Hh, Hh, 2 * C), device=dev).bfloat16()
+    cat = torch.randn((B, 2 * Hh, 2 * Hh, 2 * C), device=dev).bfloat16()
+    o1 = torch.empty((B, 2 * Hh, 2 * Hh, C), dtype=torch.bfloat16, device=dev)
+    o2 = torch.empty_like(o1)
 
-        def two():
-            layers.upconv2x2(x, pu, bu_d, out=cat, out_offset=0)
-            layers.conv3x3(cat, pd, bd_d, out=o1)
+    def two():
+        layers.upconv2x2(x, pu, bu_d, out=cat, out_offset=0)
+        layers.conv3x3(cat, pd, bd_d, out=o1)
 
-        def fusedw():
-            layers.upconv_conv3x3(x, cat, wx, fb, skip_offset=C, out=o2, weight_skip=ws)
+    def fusedw():
+        layers.upconv_conv3x3(x, cat, wx, fb, skip_offset=C, out=o2, weight_skip=ws)
 
-        t2, tf = timed(two), timed(fusedw)
-        d = (o1.float() - o2.float()).abs()
-        print(f"C {C} ({Hh}^2 -> {2 * Hh}^2): two launches {t2:.3f} ms, fused {tf:.3f} ms, max |diff| {float(d.max()):.4f} mean {float(d.mean()):.5f}")
+    t2, tf = timed(two), timed(fusedw)
+    d = (o1.float() - o2.float()).abs()
+    print(f"C {C} ({Hh}^2 -> {2 * Hh}^2): two launches {t2:.3f} ms, fused {tf:.3f} ms, max |diff| {float(d.max()):.4f} mean {float(d.mean()):.5f}")

@@ -15,12 +15,12 @@ DC_EINVAL, DC_ECUDA, DC_EDEVICE, DC_ECAPACITY, DC_EWORKSPACE = -1, -2, -3, -4, -
 DC_KIND_CONV3X3, DC_KIND_UPCONV2 = 0, 1
 DC_EPI_STORE, DC_EPI_STORE_POOL, DC_EPI_HEAD, DC_EPI_UPSCATTER = 0, 1, 2, 3
 DC_NUM_LAYERS = 23
-DC_CONV_FAMILY_AUTO, DC_CONV_FAMILY_NO_PAIR, DC_CONV_FAMILY_GENERIC = 0, 1, 2
+DC_CONV_FAMILY_AUTO, DC_CONV_FAMILY_GENERIC = 0, 2
 DC_PRECISION_BF16, DC_PRECISION_FP32 = 0, 1
-ABI_VERSION = 209          # DC_ABI_VERSION of include/unetdc_b200.h these ctypes structures mirror
+ABI_VERSION = 210          # DC_ABI_VERSION of include/unetdc_b200.h these ctypes structures mirror
 
 EXPORTS = [
-    "dc_last_error", "dc_version", "dc_device_check", "dc_conv_tc", "dc_conv_upfused", "dc_debug_upfuse_schedule", "dc_debug_set_upfuse_mode", "dc_debug_set_conv_family", "dc_stem", "dc_model_create",
+    "dc_last_error", "dc_version", "dc_device_check", "dc_conv_tc", "dc_conv_upfused", "dc_debug_upfuse_schedule", "dc_debug_set_conv_family", "dc_stem", "dc_model_create",
     "dc_model_destroy", "dc_forward_workspace_bytes", "dc_forward", "dc_forward_num_launches", "dc_forward_profile",
     "dc_rolling_ball_workspace_bytes", "dc_rolling_ball", "dc_rolling_ball_tiled", "dc_rolling_ball_banded", "dc_rolling_ball_max_radius",
     "dc_rolling_ball_tiled_max_radius", "dc_debug_rolling_ball_plan", "dc_debug_rolling_ball_bands", "dc_label_workspace_bytes", "dc_label_stats",
@@ -181,7 +181,6 @@ def load(build_if_missing: bool = True) -> C.CDLL:
     lib.dc_conv_tc.argtypes = [POINTER(ConvArgs), c_void_p]
     lib.dc_conv_upfused.argtypes = [POINTER(UpfuseArgs), c_void_p]
     lib.dc_debug_upfuse_schedule.argtypes = [POINTER(c_int), c_int]
-    lib.dc_debug_set_upfuse_mode.argtypes = [c_int]
     lib.dc_debug_set_conv_family.argtypes = [c_int]
     lib.dc_stem.argtypes = [POINTER(StemArgs), c_void_p]
     lib.dc_model_create.argtypes = [POINTER(c_void_p), c_int, POINTER(ModelDesc)]

@@ -160,8 +160,6 @@ int dc_debug_set_conv_family(int family) { return set_conv_family(family); }
 
 int dc_debug_upfuse_schedule(int* out, int cap) { return upfuse_schedule(out, cap); }
 
-int dc_debug_set_upfuse_mode(int mode) { return set_upfuse_mode(mode); }
-
 int dc_device_check(int device, int* sm_count) {
     cudaDeviceProp prop;
     DC_CUDA(cudaGetDeviceProperties(&prop, device));

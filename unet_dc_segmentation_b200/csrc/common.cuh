@@ -35,7 +35,6 @@ int launch_stem(const dc_stem_args_t* a, cudaStream_t stream, const float* bias_
 int launch_conv_upfused(const dc_upfuse_args_t* a, cudaStream_t stream, const float* bias9_host);
 int set_conv_family(int family);
 int upfuse_schedule(int* out, int cap);
-int set_upfuse_mode(int mode);
 int launch_label_stats(const dc_label_args_t* a, cudaStream_t stream);
 int launch_table_csv(const dc_table_csv_args_t* a, cudaStream_t stream);
 int table_csv_host(const dc_table_csv_args_t* a);

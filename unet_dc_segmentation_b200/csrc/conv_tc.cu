@@ -23,10 +23,10 @@
 // Kernels (they share the roles and the epilogue; DESIGN.md 3.1 has the measurements):
 //   conv_tc_kernel     generic: one TMA box per (tap, 64-channel chunk), A re-fetched per tap from L2.
 //                      Used for dilation 8 / 16 (enc4, bottleneck) and the transposed convs.
-//   conv_halo_kernel   single CTA: ONE haloed activation region (16+2d) x (8*NH+2d) pixels x 64 ch per tile and
+//   conv_halo_kernel   single CTA: ONE haloed activation region (16+2d) x (16+2d) pixels x 64 ch per tile and
 //                      chunk; the nine taps are nine UMMA descriptors into that region (start = base +
-//                      (ky*d*RW + kx*d) rows, stride between 8-pixel groups = RW rows).  Weights resident in
-//                      shared memory, or streamed per (tap, chunk).  Fallback of the pair kernel.
+//                      (ky*d*RW + kx*d) rows, stride between 8-pixel groups = RW rows).  Cout = 64 layers with
+//                      long K at dilation <= 4, weights streamed (the pair kernel does not stream at N = 64).
 //   conv_halo2_kernel  the same on a CTA pair (cta_group::2): M = 256 MMAs over two SMs, each SM holds half of the
 //                      weight rows and its own pixel tile.  Runs every 3x3 layer with dilation <= 4.
 //   stem_tc_kernel     first layer (Cin = 3): im2col tile built by producer warps, K = 9 -> 16 or 27 -> 32.
@@ -54,8 +54,6 @@ constexpr int EPI_WARP0 = 4;
 
 // Kernel-family override for the tests (dc_debug_set_conv_family): the product path never changes it.
 int g_kernel_family = DC_CONV_FAMILY_AUTO;
-// Test / measurement override of the MMA schedule of conv_upfused2_kernel (dc_debug_set_upfuse_mode); 0 on the product path.
-int g_upfuse_mode = 0;
 
 // cudaFuncAttributeMaxDynamicSharedMemorySize is per (function, device): set once per device, not per launch.
 template <class K>
@@ -688,7 +686,6 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) conv_tc_split_kernel(const __g
 constexpr int HT_H = 16, HT_W = 8;      // 16 x 8 output patch: each 8-pixel row is one UMMA 8-row group
 // NHALF = 2: two patches side by side (16 x 16 pixels) share one haloed region and accumulate into separate
 // TMEM tiles -- two independent MMA chains hide the latency of back-to-back accumulating MMAs at N = 64 / 128.
-// NHALF = 1 is kept for layers whose resident weights leave no room for two 16-wide regions.
 constexpr int HALO_MAX_STAGES = 8;
 constexpr int HALO_BAR_BYTES = 512;     // 4 x 8 stage barriers + TMEM / weight barriers + TMEM slot
 constexpr int HALO_BIAS_BYTES = 4096 + 256;   // bias (<= 1024 channels) + out_conv weights
@@ -707,29 +704,30 @@ __device__ __forceinline__ uint64_t umma_desc_sw128_strided(uint32_t smem_addr, 
     return d;
 }
 
-// WRES = true : the weights of the whole layer are loaded once and stay in shared memory (9*Cin*BN*2 bytes).
-// WRES = false: they do not fit (Cin*BN large), so (tap, chunk) slices stream through a ring of p.nbstages
-//               BN x 64 tiles; each slice still feeds HT_NHALF * 4 MMAs and the activations are still loaded
-//               once per chunk instead of once per tap, which is what keeps these layers off the L2 roofline.
-template <int BN, int HT_NHALF, bool WRES>
+// Cout = 64 layers with long K at dilation <= 4, whose weights do not fit next to the pair kernel's regions (and the
+// pair kernel does not stream weights at N = 64): two 8-wide halves per tile, the weights streamed through a ring of
+// p.nbstages 64 x 64 (tap, chunk) slices.  Each slice still feeds 2 x 4 MMAs and the activations are still loaded
+// once per chunk instead of once per tap, which is what keeps these layers off the L2 roofline.
+constexpr int HALO_BN = 64, HALO_NHALF = 2;
+constexpr int HALO_W_TILE_BYTES = HALO_BN * KCHUNK * 2;      // one (tap, chunk) slice of the weights
+
 __global__ void __launch_bounds__(NUM_THREADS, 1) conv_halo_kernel(const __grid_constant__ ConvParams p) {
-    constexpr int HT_TW = HT_W * HT_NHALF;
-    constexpr int W_TILE_BYTES = BN * KCHUNK * 2;     // one (tap, chunk) slice of the weights
-    constexpr int TMEM_COLS = 2 * HT_NHALF * BN;
+    constexpr int BN = HALO_BN;
+    constexpr int HT_TW = HT_W * HALO_NHALF;
+    constexpr int W_TILE_BYTES = HALO_W_TILE_BYTES;
+    constexpr int TMEM_COLS = 2 * HALO_NHALF * BN;
 
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-    const int n_wtiles = WRES ? 9 * p.kchunks : p.nbstages;
-    uint8_t* w_res = smem;                                             // resident weights, or the weight ring
-    uint8_t* a_ring = smem + n_wtiles * W_TILE_BYTES;                  // haloed activation regions
+    uint8_t* w_ring = smem;                                            // the weight ring
+    uint8_t* a_ring = smem + p.nbstages * W_TILE_BYTES;                // haloed activation regions
     uint64_t* full_bar = reinterpret_cast<uint64_t*>(a_ring + p.nstages * p.region_stride);
     uint64_t* empty_bar = full_bar + HALO_MAX_STAGES;
     uint64_t* bfull_bar = empty_bar + HALO_MAX_STAGES;
     uint64_t* bempty_bar = bfull_bar + HALO_MAX_STAGES;
     uint64_t* tfull_bar = bempty_bar + HALO_MAX_STAGES;
     uint64_t* tempty_bar = tfull_bar + 2;
-    uint64_t* w_bar = tempty_bar + 2;
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(w_bar + 1);
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty_bar + 2);
     float* bias_s = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(full_bar) + HALO_BAR_BYTES);
     uint8_t* stg_s = reinterpret_cast<uint8_t*>(full_bar) + HALO_BAR_BYTES + HALO_BIAS_BYTES;
 
@@ -748,7 +746,6 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) conv_halo_kernel(const __grid_
             mbar_init(&bfull_bar[s], 1); mbar_init(&bempty_bar[s], 1);
         }
         for (int s = 0; s < 2; ++s) { mbar_init(&tfull_bar[s], 1); mbar_init(&tempty_bar[s], 4 * EPI_GROUPS); }
-        mbar_init(w_bar, 1);
         fence_barrier_init();
     }
     if (warp == 2) {
@@ -774,18 +771,11 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) conv_halo_kernel(const __grid_
 
     if (warp == 0) {
         // ------------------------------------------------------------------ TMA producer (warp-uniform loop)
-        if (WRES) {
-            if (elect_one()) {
-                mbar_expect_tx(w_bar, (uint32_t)(n_wtiles * W_TILE_BYTES));
-                for (int j = 0; j < n_wtiles; ++j) tma_load_2d(w_res + j * W_TILE_BYTES, &p.tmB, w_bar, j * KCHUNK, 0);
-            }
-            __syncwarp();
-        }
         int stage = 0, bstage = 0;
         uint32_t phase = 0, bphase = 0;
         for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
             const TileCoord t = decode_tile<HT_H, HT_TW>(p, tile, BN);
-            const uint32_t tap_mask = WRES ? 0u : tile_tap_mask(t);
+            const uint32_t tap_mask = tile_tap_mask(t);
             for (int kc = 0; kc < p.kchunks; ++kc) {
                 mbar_wait(&empty_bar[stage], phase ^ 1u);
                 if (elect_one()) {
@@ -795,18 +785,16 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) conv_halo_kernel(const __grid_
                 }
                 __syncwarp();
                 if (++stage == NST) { stage = 0; phase ^= 1u; }
-                if (!WRES) {
-                    for (int tap = 0; tap < 9; ++tap) {
-                        if (!((tap_mask >> tap) & 1u)) continue;
-                        mbar_wait(&bempty_bar[bstage], bphase ^ 1u);
-                        if (elect_one()) {
-                            mbar_expect_tx(&bfull_bar[bstage], W_TILE_BYTES);
-                            tma_load_2d(w_res + bstage * W_TILE_BYTES, &p.tmB, &bfull_bar[bstage],
-                                        (tap * p.kchunks + kc) * KCHUNK, 0);
-                        }
-                        __syncwarp();
-                        if (++bstage == NBS) { bstage = 0; bphase ^= 1u; }
+                for (int tap = 0; tap < 9; ++tap) {
+                    if (!((tap_mask >> tap) & 1u)) continue;
+                    mbar_wait(&bempty_bar[bstage], bphase ^ 1u);
+                    if (elect_one()) {
+                        mbar_expect_tx(&bfull_bar[bstage], W_TILE_BYTES);
+                        tma_load_2d(w_ring + bstage * W_TILE_BYTES, &p.tmB, &bfull_bar[bstage],
+                                    (tap * p.kchunks + kc) * KCHUNK, 0);
                     }
+                    __syncwarp();
+                    if (++bstage == NBS) { bstage = 0; bphase ^= 1u; }
                 }
             }
         }
@@ -814,13 +802,12 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) conv_halo_kernel(const __grid_
         // ------------------------------------------------------------------ MMA issuer (warp-uniform loop)
         const uint32_t idesc = umma_idesc_bf16(TILE_M, BN);
         const uint32_t sbo = (uint32_t)p.region_w * 128u;
-        const uint32_t w_addr = smem_u32(w_res);
+        const uint32_t w_addr = smem_u32(w_ring);
         const uint32_t tap_dy_bytes = (uint32_t)(p.dil * p.region_w) * 128u;     // one tap row down
         const uint32_t tap_dx_bytes = (uint32_t)p.dil * 128u;                    // one tap column right
         int stage = 0, bstage = 0;
         uint32_t phase = 0, bphase = 0;
         int it = 0;
-        if (WRES) mbar_wait(w_bar, 0);
         for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x, ++it) {
             const TileCoord t = decode_tile<HT_H, HT_TW>(p, tile, BN);
             const int as = it & 1;
@@ -828,68 +815,43 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) conv_halo_kernel(const __grid_
             const uint32_t tap_mask = tile_tap_mask(t);
             mbar_wait(&tempty_bar[as], aphase ^ 1u);
             tc_fence_after();
-            const uint32_t d_tmem = tmem_base + (uint32_t)(as * HT_NHALF * BN);
+            const uint32_t d_tmem = tmem_base + (uint32_t)(as * HALO_NHALF * BN);
             uint32_t accumulate = 0;
             for (int kc = 0; kc < p.kchunks; ++kc) {
                 mbar_wait(&full_bar[stage], phase);
                 tc_fence_after();
                 const uint32_t region = smem_u32(a_ring + stage * p.region_stride);
-                if (WRES) {
-                    const uint32_t w_chunk = w_addr + (uint32_t)(kc * W_TILE_BYTES);
-                    const uint32_t w_tap_stride = (uint32_t)(p.kchunks * W_TILE_BYTES);
+#pragma unroll 1
+                for (int tap = 0; tap < 9; ++tap) {
+                    if (!((tap_mask >> tap) & 1u)) continue;
+                    mbar_wait(&bfull_bar[bstage], bphase);
+                    tc_fence_after();
+                    const uint32_t a_addr = region + (uint32_t)(tap / 3) * tap_dy_bytes + (uint32_t)(tap % 3) * tap_dx_bytes;
+                    const uint64_t adesc = umma_desc_sw128_strided(a_addr, sbo);
+                    const uint64_t bdesc = umma_desc_sw128(w_addr + (uint32_t)(bstage * W_TILE_BYTES));
                     if (elect_one()) {
 #pragma unroll
-                        for (int tap = 0; tap < 9; ++tap) {
-                            if (!((tap_mask >> tap) & 1u)) continue;
-                            const uint32_t a_addr = region + (uint32_t)(tap / 3) * tap_dy_bytes + (uint32_t)(tap % 3) * tap_dx_bytes;
-                            const uint64_t adesc = umma_desc_sw128_strided(a_addr, sbo);
-                            const uint64_t bdesc = umma_desc_sw128(w_chunk + (uint32_t)tap * w_tap_stride);
+                        for (int k = 0; k < KCHUNK / 16; ++k) {
 #pragma unroll
-                            for (int k = 0; k < KCHUNK / 16; ++k) {
-#pragma unroll
-                                for (int half = 0; half < HT_NHALF; ++half)   // right patch = 8 region rows (1024 B) further
-                                    umma_bf16(d_tmem + (uint32_t)(half * BN), adesc + (uint64_t)(2 * k + 64 * half),
-                                              bdesc + (uint64_t)(2 * k), idesc, accumulate);
-                                accumulate = 1;
-                            }
+                            for (int half = 0; half < HALO_NHALF; ++half)   // right patch = 8 region rows (1024 B) further
+                                umma_bf16(d_tmem + (uint32_t)(half * BN), adesc + (uint64_t)(2 * k + 64 * half),
+                                          bdesc + (uint64_t)(2 * k), idesc, (k == 0) ? accumulate : 1u);
                         }
-                        umma_commit(&empty_bar[stage]);
+                        umma_commit(&bempty_bar[bstage]);
                     }
                     __syncwarp();
                     accumulate = 1;
-                } else {
-#pragma unroll 1
-                    for (int tap = 0; tap < 9; ++tap) {
-                        if (!((tap_mask >> tap) & 1u)) continue;
-                        mbar_wait(&bfull_bar[bstage], bphase);
-                        tc_fence_after();
-                        const uint32_t a_addr = region + (uint32_t)(tap / 3) * tap_dy_bytes + (uint32_t)(tap % 3) * tap_dx_bytes;
-                        const uint64_t adesc = umma_desc_sw128_strided(a_addr, sbo);
-                        const uint64_t bdesc = umma_desc_sw128(w_addr + (uint32_t)(bstage * W_TILE_BYTES));
-                        if (elect_one()) {
-#pragma unroll
-                            for (int k = 0; k < KCHUNK / 16; ++k) {
-#pragma unroll
-                                for (int half = 0; half < HT_NHALF; ++half)
-                                    umma_bf16(d_tmem + (uint32_t)(half * BN), adesc + (uint64_t)(2 * k + 64 * half),
-                                              bdesc + (uint64_t)(2 * k), idesc, (k == 0) ? accumulate : 1u);
-                            }
-                            umma_commit(&bempty_bar[bstage]);
-                        }
-                        __syncwarp();
-                        accumulate = 1;
-                        if (++bstage == NBS) { bstage = 0; bphase ^= 1u; }
-                    }
-                    if (elect_one()) umma_commit(&empty_bar[stage]);
-                    __syncwarp();
+                    if (++bstage == NBS) { bstage = 0; bphase ^= 1u; }
                 }
+                if (elect_one()) umma_commit(&empty_bar[stage]);
+                __syncwarp();
                 if (++stage == NST) { stage = 0; phase ^= 1u; }
             }
             if (elect_one()) umma_commit(&tfull_bar[as]);
             __syncwarp();
         }
     } else if (warp >= EPI_WARP0) {
-        run_epilogue<BN, HT_H, HT_W, HT_NHALF>(p, warp & 3, lane, (warp - EPI_WARP0) >> 2, tmem_base, tfull_bar, tempty_bar, bias_s, stg_s);
+        run_epilogue<BN, HT_H, HT_W, HALO_NHALF>(p, warp & 3, lane, (warp - EPI_WARP0) >> 2, tmem_base, tfull_bar, tempty_bar, bias_s, stg_s);
     }
 
     tc_fence_before();
@@ -1138,20 +1100,17 @@ constexpr size_t UPF_SMEM = UPF_RING * UPF_GROUP_BYTES + 2 * UPF_U_BYTES + 2 * U
                             UPF_BIAS_BYTES + EPI_STAGE_TOTAL;
 static_assert(UPF_SMEM <= 227 * 1024, "conv_upfused2_kernel: shared memory");
 
-struct UpfOp;
-template <int MODE> inline UpfOp upf_u_op(int i);           // host: MMA i of one K = 16 step of an x chunk / the skip chunk
-template <int MODE> inline UpfOp upf_s_op(int i);
-template <int MODE> inline int upf_u_count();
-template <int MODE> inline int upf_s_count();
-// device: the 4 x (MMAs of group G) of chunk kind KIND (0 = x, 1 = skip); d = accumulator base, a = descriptor of the
-// region's first row, b = descriptor of the group's ring slot; fresh = overwrite at the tile's first K step
-template <int MODE, int KIND, int G>
+// upf_schedule.inc defines, host side, upf_u_op(i) / upf_s_op(i) = MMA i of one K = 16 step of an x chunk / the skip
+// chunk and upf_u_count() / upf_s_count(); device side, the specialisations of upf_issue_group below.
+// upf_issue_group<KIND, G> issues the 4 x (MMAs of group G) of chunk kind KIND (0 = x, 1 = skip); d = accumulator base,
+// a = descriptor of the region's first row, b = descriptor of the group's ring slot; fresh = overwrite at the tile's
+// first K step
+template <int KIND, int G>
 __device__ __forceinline__ void upf_issue_group(uint32_t d, uint64_t a, uint64_t b, bool fresh);
 #include "upf_schedule.inc"
 constexpr int UPF_GROUPS_PER_TILE = 2 * 4 + 9;
 constexpr int UPF_ROWS_PER_RANK = UPF_GROUPS_PER_TILE * UPF_GROUP_ROWS;      // 2176 weight rows per CTA of the pair
 
-template <int MODE>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1)
 conv_upfused2_kernel(const __grid_constant__ ConvParams p) {
     constexpr int BN = 64;
@@ -1266,7 +1225,7 @@ conv_upfused2_kernel(const __grid_constant__ ConvParams p) {
         mbar_wait(&bfull_bar[bg], bphase);                                                                          \
         tc_fence_after();                                                                                           \
         if (elect_one()) {                                                                                          \
-            upf_issue_group<MODE, KIND, G>(d_tmem, ADESC, bdesc_ring + (uint64_t)(bg * (UPF_GROUP_BYTES >> 4)), FRESH); \
+            upf_issue_group<KIND, G>(d_tmem, ADESC, bdesc_ring + (uint64_t)(bg * (UPF_GROUP_BYTES >> 4)), FRESH);       \
             umma_commit_2sm(&bempty_bar[bg]);                                                                       \
         }                                                                                                           \
         __syncwarp();                                                                                               \
@@ -1558,7 +1517,6 @@ constexpr size_t PAR_SMEM = PAR_RING * UPF_GROUP_BYTES + PAR_STAGES * 2 * UPF_PL
                             PAR_BIAS_BYTES + EPI_STAGE_TOTAL;
 static_assert(PAR_SMEM <= 227 * 1024, "conv_par2_kernel: shared memory");
 
-template <int MODE>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1)
 conv_par2_kernel(const __grid_constant__ ConvParams p) {
     constexpr int BN = 64;
@@ -1660,7 +1618,7 @@ conv_par2_kernel(const __grid_constant__ ConvParams p) {
         mbar_wait(&bfull_bar[bg], bphase);                                                                          \
         tc_fence_after();                                                                                           \
         if (elect_one()) {                                                                                          \
-            upf_issue_group<MODE, 2, G>(d_tmem, areg, bdesc_ring + (uint64_t)(bg * (UPF_GROUP_BYTES >> 4)), true);  \
+            upf_issue_group<2, G>(d_tmem, areg, bdesc_ring + (uint64_t)(bg * (UPF_GROUP_BYTES >> 4)), true);        \
             umma_commit_2sm(&bempty_bar[bg]);                                                                       \
         }                                                                                                           \
         __syncwarp();                                                                                               \
@@ -2042,15 +2000,10 @@ static int launch_conv_par(const dc_conv_args_t* a, cudaStream_t stream, const f
     const int n_pairs = (p.m_tiles + 1) / 2;
     const int max_clusters = num_sms() / 2;
     const int grid = 2 * (n_pairs < max_clusters ? n_pairs : max_clusters);
-#define DC_PAR_CASE(mode)                                                                                    \
-    if (g_upfuse_mode == mode) {                                                                             \
-        static unsigned long long attr_done = 0;                                                             \
-        int rc = set_max_smem_once(conv_par2_kernel<mode>, (int)PAR_SMEM, &attr_done);                       \
-        if (rc != DC_OK) return rc;                                                                          \
-        conv_par2_kernel<mode><<<grid, NUM_THREADS, PAR_SMEM, stream>>>(p);                                  \
-    }
-    DC_PAR_CASE(0) DC_PAR_CASE(1) DC_PAR_CASE(2) DC_PAR_CASE(3)
-#undef DC_PAR_CASE
+    static unsigned long long attr_done = 0;
+    int rc = set_max_smem_once(conv_par2_kernel, (int)PAR_SMEM, &attr_done);
+    if (rc != DC_OK) return rc;
+    conv_par2_kernel<<<grid, NUM_THREADS, PAR_SMEM, stream>>>(p);
     DC_CUDA(cudaGetLastError());
     return DC_OK;
 }
@@ -2155,45 +2108,26 @@ int launch_conv_tc(const dc_conv_args_t* a, cudaStream_t stream, const float* bi
         }
         }
     }
-    if (!split && !halo && !up && a->Cout == BN && BN <= 128 && a->dilation <= 4) {
+    if (!split && !halo && !up && a->Cout == HALO_BN && a->dilation <= 4) {
+        // Cout = 64 layers whose weights do not fit next to the pair kernel's regions: conv_halo_kernel streams them.
         // TMA and the MMA unit both take the swizzle phase from absolute address bits, so a region only needs
         // TMA's 128 B alignment, not a 1024 B one: regions are packed back to back
-        const size_t w_tile = (size_t)BN * KCHUNK * 2;
-        const size_t w_bytes = (size_t)9 * (a->Cin / KCHUNK) * w_tile;
-        const size_t budget = 227 * 1024 - 1024 /* alignment slack */ - HALO_BAR_BYTES - HALO_BIAS_BYTES -
-                              EPI_STAGE_TOTAL /* epilogue transpose buffers */;
-        // Preference order (measured, profiles/): two halves (two independent MMA chains) beat one; resident weights
-        // beat streamed ones, and at BN = 64 a streamed slice carries only 256 MMA-cycles, too little to cover the
-        // L2 latency with the ring that fits -- so BN = 64 takes resident/1 half before anything streamed.
-        static const int order128[4][2] = {{2, 0}, {2, 1}, {1, 0}, {1, 1}};     // {nhalf, pass}; pass 1 = streamed
-        static const int order64[4][2] = {{2, 0}, {1, 0}, {2, 1}, {1, 1}};
-        for (int oi = 0; oi < 4 && !halo; ++oi) {
-            {
-                const int nhalf = (BN == 128 ? order128 : order64)[oi][0];
-                const int pass = (BN == 128 ? order128 : order64)[oi][1];
-                const int rw = HT_W * nhalf + 2 * a->dilation, rh = HT_H + 2 * a->dilation;
-                const size_t region_stride = (size_t)rw * rh * KCHUNK * 2;
-                size_t wsm = w_bytes;
-                int nb = 0;
-                if (pass == 1) {
-                    if (budget < 2 * region_stride + 4 * w_tile) continue;
-                    const size_t room = budget - 2 * region_stride;
-                    nb = (int)(room / w_tile);
-                    if (nb > HALO_MAX_STAGES) nb = HALO_MAX_STAGES;
-                    wsm = (size_t)nb * w_tile;
-                }
-                const long long nst = wsm < budget ? (long long)((budget - wsm) / region_stride) : 0;
-                if (nst >= 2) {
-                    halo = true;
-                    halo_wres = pass == 0;
-                    halo_nhalf = nhalf;
-                    p.region_w = rw; p.region_h = rh; p.region_stride = (int)region_stride;
-                    p.nstages = nst > HALO_MAX_STAGES ? HALO_MAX_STAGES : (int)nst;
-                    p.nbstages = nb;
-                    halo_smem = wsm + (size_t)p.nstages * region_stride + 1024 + HALO_BAR_BYTES + HALO_BIAS_BYTES + EPI_STAGE_TOTAL;
-                }
-            }
-        }
+        constexpr size_t budget = 227 * 1024 - 1024 /* alignment slack */ - HALO_BAR_BYTES - HALO_BIAS_BYTES -
+                                  EPI_STAGE_TOTAL /* epilogue transpose buffers */;
+        constexpr size_t max_region = (size_t)(HT_W * HALO_NHALF + 2 * 4) * (HT_H + 2 * 4) * KCHUNK * 2;    // dilation 4
+        static_assert(budget >= 2 * max_region + 4 * HALO_W_TILE_BYTES, "conv_halo_kernel: two regions and a 4-slice ring");
+        const int rw = HT_W * HALO_NHALF + 2 * a->dilation, rh = HT_H + 2 * a->dilation;
+        const size_t region_stride = (size_t)rw * rh * KCHUNK * 2;
+        int nb = (int)((budget - 2 * region_stride) / HALO_W_TILE_BYTES);
+        if (nb > HALO_MAX_STAGES) nb = HALO_MAX_STAGES;
+        const size_t wsm = (size_t)nb * HALO_W_TILE_BYTES;
+        const int nst = (int)((budget - wsm) / region_stride);
+        halo = true;
+        halo_nhalf = HALO_NHALF;
+        p.region_w = rw; p.region_h = rh; p.region_stride = (int)region_stride;
+        p.nstages = nst > HALO_MAX_STAGES ? HALO_MAX_STAGES : nst;
+        p.nbstages = nb;
+        halo_smem = wsm + (size_t)p.nstages * region_stride + 1024 + HALO_BAR_BYTES + HALO_BIAS_BYTES + EPI_STAGE_TOTAL;
     }
     if (g_kernel_family == DC_CONV_FAMILY_GENERIC) halo = halo_pair = false;      // test-only override (dc_debug_set_conv_family)
     {
@@ -2269,16 +2203,10 @@ int launch_conv_tc(const dc_conv_args_t* a, cudaStream_t stream, const float* bi
     }
     if (halo) {
         const int grid = p.total_tiles < num_sms() ? p.total_tiles : num_sms();
-#define DC_HALO_CASE(bn, nh, wr)                                                                                     \
-        if (BN == bn && halo_nhalf == nh && halo_wres == wr) {                                                       \
-            static unsigned long long attr_done = 0;                                                                 \
-            int rc_ = set_max_smem_once(conv_halo_kernel<bn, nh, wr>, 227 * 1024, &attr_done);                       \
-            if (rc_ != DC_OK) return rc_;                                                                            \
-            conv_halo_kernel<bn, nh, wr><<<grid, NUM_THREADS, halo_smem, stream>>>(p);                               \
-        }
-        DC_HALO_CASE(64, 1, true) DC_HALO_CASE(64, 2, true) DC_HALO_CASE(128, 1, true) DC_HALO_CASE(128, 2, true)
-        DC_HALO_CASE(64, 1, false) DC_HALO_CASE(64, 2, false) DC_HALO_CASE(128, 1, false) DC_HALO_CASE(128, 2, false)
-#undef DC_HALO_CASE
+        static unsigned long long attr_done = 0;
+        int rc = set_max_smem_once(conv_halo_kernel, 227 * 1024, &attr_done);
+        if (rc != DC_OK) return rc;
+        conv_halo_kernel<<<grid, NUM_THREADS, halo_smem, stream>>>(p);
         DC_CUDA(cudaGetLastError());
         return DC_OK;
     }
@@ -2426,56 +2354,35 @@ int launch_conv_upfused(const dc_upfuse_args_t* a, cudaStream_t stream, const fl
     const int n_pairs = (p.m_tiles + 1) / 2;
     const int max_clusters = num_sms() / 2;
     const int grid = 2 * (n_pairs < max_clusters ? n_pairs : max_clusters);
-#define DC_UPF_CASE(mode)                                                                                    \
-    if (g_upfuse_mode == mode) {                                                                             \
-        static unsigned long long attr_done = 0;                                                             \
-        int rc = set_max_smem_once(conv_upfused2_kernel<mode>, (int)UPF_SMEM, &attr_done);                   \
-        if (rc != DC_OK) return rc;                                                                          \
-        conv_upfused2_kernel<mode><<<grid, NUM_THREADS, UPF_SMEM, stream>>>(p);                              \
-    }
-    DC_UPF_CASE(0) DC_UPF_CASE(1) DC_UPF_CASE(2) DC_UPF_CASE(3)
-#undef DC_UPF_CASE
+    static unsigned long long attr_done = 0;
+    int rc = set_max_smem_once(conv_upfused2_kernel, (int)UPF_SMEM, &attr_done);
+    if (rc != DC_OK) return rc;
+    conv_upfused2_kernel<<<grid, NUM_THREADS, UPF_SMEM, stream>>>(p);
     DC_CUDA(cudaGetLastError());
     return DC_OK;
 }
 
 // The MMA schedule of conv_upfused2_kernel for the host-side weight packer: one row {chunk (0, 1 = x channels,
 // 2 = skip), window row, window column, first class, classes} per MMA, in issue order.
-template <int MODE>
-int upfuse_schedule_of(int* out, int cap) {
-    const int nu = upf_u_count<MODE>(), ns = upf_s_count<MODE>();
+int upfuse_schedule(int* out, int cap) {
+    const int nu = upf_u_count(), ns = upf_s_count();
     const int n = 2 * nu + ns;
     DC_REQUIRE(out && cap >= 5 * n, DC_EINVAL, "dc_debug_upfuse_schedule: need room for %d ints", 5 * n);
     int* o = out;
     for (int kc = 0; kc < 2; ++kc)
         for (int i = 0; i < nu; ++i) {
-            const UpfOp op = upf_u_op<MODE>(i);
+            const UpfOp op = upf_u_op(i);
             *o++ = kc; *o++ = op.r; *o++ = op.c; *o++ = op.cls0; *o++ = op.ncls;
         }
     for (int i = 0; i < ns; ++i) {
-        const UpfOp op = upf_s_op<MODE>(i);
+        const UpfOp op = upf_s_op(i);
         *o++ = 2; *o++ = op.r; *o++ = op.c; *o++ = op.cls0; *o++ = op.ncls;
     }
     return n;
 }
 
-int upfuse_schedule(int* out, int cap) {
-    switch (g_upfuse_mode) {
-        case 1: return upfuse_schedule_of<1>(out, cap);
-        case 2: return upfuse_schedule_of<2>(out, cap);
-        case 3: return upfuse_schedule_of<3>(out, cap);
-        default: return upfuse_schedule_of<0>(out, cap);
-    }
-}
-
-int set_upfuse_mode(int mode) {
-    DC_REQUIRE(mode >= 0 && mode < UPF_MODES, DC_EINVAL, "dc_debug_set_upfuse_mode: %d", mode);
-    g_upfuse_mode = mode;
-    return DC_OK;
-}
-
 int set_conv_family(int family) {
-    DC_REQUIRE(family >= DC_CONV_FAMILY_AUTO && family <= DC_CONV_FAMILY_GENERIC, DC_EINVAL, "dc_debug_set_conv_family: %d", family);
+    DC_REQUIRE(family == DC_CONV_FAMILY_AUTO || family == DC_CONV_FAMILY_GENERIC, DC_EINVAL, "dc_debug_set_conv_family: %d", family);
     g_kernel_family = family;
     return DC_OK;
 }
