@@ -25,8 +25,17 @@ Replays walk K in each kernel's order (conv_tc.cu):
   transposed conv (split)          (term, chunk, k16), one tap              ``upconv_steps``
   conv_halo_kernel / halo2         (chunk, tap, k16), resident or streamed  ``conv_steps(order="chunk")``
   stem_tc_kernel                   one or two K = 16 slices of c * 9 + tap  ``stem_steps``
+  conv_upfused2_kernel             per parity class: (x chunk 0, x chunk 1, skip), group G of the generated issue code,
+                                   k16, the group's calls on the class's slot      ``upf_walks(UPF_CHUNKS)``
+  conv_upfused_wide_kernel<BN>     per class: [x chunk 2g, x chunk 2g + 1, skip chunk g] for g < C / 64, tap, k16
+                                                                                   ``wide_walks``
+  conv_par2_kernel                 the skip chunk of the same schedule alone        ``upf_walks(PAR_CHUNKS)``
 A tap the kernels skip (tap_offset, tile_tap_mask) or read as TMA zero fill is a step of zero products, which leaves
-the accumulator unchanged (probe ``identity``), so the replay does not need the tile geometry.
+the accumulator unchanged (probe ``identity``), so the replay does not need the tile geometry.  ``class_acc`` replays the
+parity-class walks; their epilogues are ``store_border_bf16`` (the fused kernels: the interior bias row, then a second
+fp32 add of the border-class difference), ``store_bf16`` / ``pool_bf16`` / ``head_logit`` (conv_par2_kernel's STORE,
+STORE_POOL and HEAD).  With these walks every kernel of the default bf16 forward is accounted for bit for bit
+(tests/test_gpu_tc_accum.py test_bf16_forward_chain), as is every kernel of the fp32 forward.
 """
 from __future__ import annotations
 
@@ -177,12 +186,146 @@ def stem_steps(cols, wk):
         yield cols[..., k:k + 16], wk[:, k:k + 16].T
 
 
+# ----------------------------------------------------------------------------- K walks of the parity-class kernels
+# conv_upfused2_kernel, conv_upfused_wide_kernel and conv_par2_kernel compute the four output parity classes (py, px) of
+# a half-resolution tile in separate accumulators.  A walk is, per class cls = py * 2 + px, the list of the items
+# (source, 64-channel chunk, tap, k16) the kernel adds into that class's accumulator, in issue order; source "x" is the
+# half-resolution input of the composed transposed conv (tap (a, b) reads x at (h + py + a - 1, w + px + b - 1)), "s"
+# the skip / full-resolution input sampled at stride 2 (tap (ky, kx) reads it at (2h + py + ky - 1, 2w + px + kx - 1)).
+# Every class's walk has the same length and starts with the step the kernel issues with accumulate = 0.
+
+def upf_walks(chunks, reverse_groups=False):
+    """The walks of the generated issue code (csrc/upf_schedule.inc): chunks = [(issue kind, schedule chunk, fresh)]
+    in the kernel's order -- conv_upfused2_kernel [(0, 0, True), (0, 1, False), (1, 2, False)] (``UPF_CHUNKS``),
+    conv_par2_kernel [(2, 2, True)] (``PAR_CHUNKS``); `fresh` is the argument the kernel passes for that chunk.  Within
+    a chunk: group G of the issue code, then k16, then the calls of the group at that k16 (upf_model.issue_code),
+    matched to the rows of model.upfuse_schedule() (window (r, c), slots slot0 .. slot0 + n - 1, slot s = class
+    s ^ (s >> 1)); class (py, px) reads tap (r - py, c - px).  Asserts that the first item of every class is the only
+    one issued with accumulate = 0.  reverse_groups: the groups of each chunk in the opposite order (a wrong walk the
+    tests must tell apart)."""
+    import upf_model as um
+    from unet_dc_segmentation_b200.model import upfuse_schedule
+    sched = upfuse_schedule()
+    walks = {cls: [] for cls in range(4)}
+    fresh_at = {cls: [] for cls in range(4)}
+    for kind, chunk, fresh_arg in chunks:
+        ops = [row for row in sched if row[0] == chunk]
+        groups, i = [], 0
+        for _, calls in um.issue_code(kind):
+            per_k = len(calls) // 4
+            assert per_k * 4 == len(calls)
+            groups.append((calls, ops[i:i + per_k]))
+            i += per_k
+        assert i == len(ops), "issue code and schedule disagree on the number of MMAs"
+        for calls, gops in (reversed(groups) if reverse_groups else groups):
+            per_k = len(gops)
+            for k in range(4):
+                for (d, _, _, n, fresh), (_, r, c, slot0, nslots) in zip(calls[k * per_k:(k + 1) * per_k], gops):
+                    assert (d, n) == (64 * slot0, 64 * nslots), "issue code and schedule disagree on the slots"
+                    for slot in range(slot0, slot0 + nslots):
+                        cls = slot ^ (slot >> 1)
+                        tap = (r - (cls >> 1), c - (cls & 1))
+                        assert all(0 <= t <= (1 if chunk < 2 else 2) for t in tap), (chunk, r, c, cls)
+                        fresh_at[cls].append(fresh and fresh_arg)
+                        walks[cls].append(("s" if chunk == 2 else "x", chunk % 2, tap, k))
+    if not reverse_groups:
+        for cls in range(4):
+            assert fresh_at[cls][0] and not any(fresh_at[cls][1:]), f"class {cls}: accumulate = 0 not on its first MMA only"
+    assert len({len(w) for w in walks.values()}) == 1
+    return walks
+
+
+UPF_CHUNKS = ((0, 0, True), (0, 1, False), (1, 2, False))         # conv_upfused2_kernel: x chunk 0, x chunk 1, skip
+PAR_CHUNKS = ((2, 2, True),)                                      # conv_par2_kernel: the skip chunk alone
+
+
+def wide_walks(C, reverse_groups=False):
+    """conv_upfused_wide_kernel: [x chunk 2g, x chunk 2g + 1, skip chunk g] for g < C / 64; an x chunk over taps
+    (a, b) = (tap >> 1, tap & 1), a skip chunk over taps (ky, kx) = (tap / 3, tap % 3), k16 inside the tap (the MMA
+    warp's loops: chunk, tap, k, class of the pass).  The same walk for every class."""
+    items = []
+    for g in (reversed(range(C // 64)) if reverse_groups else range(C // 64)):
+        for chunk in (2 * g, 2 * g + 1):
+            items += [("x", chunk, (t >> 1, t & 1), k) for t in range(4) for k in range(4)]
+        items += [("s", g, (t // 3, t % 3), k) for t in range(9) for k in range(4)]
+    return {cls: items for cls in range(4)}
+
+
+def composed_walks(C, order):
+    """The composed layer walked as the unfused kernels would: "tap" (tap, chunk, k16) or "chunk" (chunk, tap, k16),
+    the x half before the skip half, taps in their natural order (wrong walks the tests must tell apart)."""
+    xt = [(a, b) for a in range(2) for b in range(2)]
+    st = [(ky, kx) for ky in range(3) for kx in range(3)]
+    if order == "tap":
+        items = [("x", ch, t, k) for t in xt for ch in range(2 * C // 64) for k in range(4)]
+        items += [("s", ch, t, k) for t in st for ch in range(C // 64) for k in range(4)]
+    else:
+        assert order == "chunk"
+        items = [("x", ch, t, k) for ch in range(2 * C // 64) for t in xt for k in range(4)]
+        items += [("s", ch, t, k) for ch in range(C // 64) for t in st for k in range(4)]
+    return {cls: items for cls in range(4)}
+
+
+def skip_first(walks):
+    """A walk with its skip items moved ahead of the x items (a wrong walk the tests must tell apart)."""
+    return {cls: [i for i in w if i[0] == "s"] + [i for i in w if i[0] == "x"] for cls, w in walks.items()}
+
+
+def class_steps(x, skip, comp, skipw, walks):
+    """MMA steps of the four classes at once (class as the leading dimension): x [B, Hh, Wh, Cx] half-resolution
+    NHWC (None for conv_par2_kernel), skip [B, 2 Hh, 2 Wh, C] (float64 of bf16 values, zero padded like TMA's fill);
+    comp [4 cls][2][2][Co][Cx] and skipw [3][3][Co][C] bf16 values (model.compose_upconv; conv_par2_kernel: skipw =
+    the 3x3 weights as [ky][kx][co][ci]).  Yields (a [4, B, Hh, Wh, 16], b [4, 1, 1, 1, 16, Co])."""
+    B, H2, W2, _ = skip.shape
+    Hh, Wh = H2 // 2, W2 // 2
+    sp = F.pad(skip, (0, 0, 1, 1, 1, 1))
+    win = {("s", r, c): sp[:, r:r + 2 * Hh:2, c:c + 2 * Wh:2] for r in range(4) for c in range(4)}
+    if x is not None:
+        xp = F.pad(x, (0, 0, 1, 1, 1, 1))
+        win.update({("x", r, c): xp[:, r:r + Hh, c:c + Wh] for r in range(3) for c in range(3)})
+    for items in zip(*(walks[cls] for cls in range(4))):
+        As, Bs = [], []
+        for cls, (src, chunk, (ty, tx), k) in enumerate(items):
+            c0 = chunk * 64 + 16 * k
+            As.append(win[(src, (cls >> 1) + ty, (cls & 1) + tx)][..., c0:c0 + 16])
+            w = comp[cls, ty, tx] if src == "x" else skipw[ty, tx]
+            Bs.append(w[:, c0:c0 + 16].T)
+        yield torch.stack(As), torch.stack(Bs).view(4, 1, 1, 1, 16, -1)
+
+
+def interleave(acc):
+    """[4 classes, B, Hh, Wh, N] -> [B, 2 Hh, 2 Wh, N]: class (py, px) at output pixel (2h + py, 2w + px)."""
+    _, B, Hh, Wh, N = acc.shape
+    return acc.view(2, 2, B, Hh, Wh, N).permute(2, 3, 0, 4, 1, 5).reshape(B, 2 * Hh, 2 * Wh, N)
+
+
+def class_acc(x, skip, comp, skipw, walks, m=MEASURED):
+    """The fp32 accumulators of a parity-class layer at full resolution [B, 2 Hh, 2 Wh, Co]."""
+    return interleave(run_steps(class_steps(x, skip, comp, skipw, walks), m))
+
+
 def assert_normal_products(xs, ws):
     """Every non-zero product of an activation plane and a weight plane is a normal fp32 number (the model's range):
     min |x| * min |w| over the non-zero values bounds the smallest product from below."""
     def lo(ts):
         return min(float(t[t != 0].abs().min()) for t in ts if bool((t != 0).any()))
     assert lo(xs) * lo(ws) >= NORMAL_MIN, f"products down to {lo(xs) * lo(ws)!r}, below the model's range"
+
+
+def upfused_real_operands(C, B, Hh, Wh, seed):
+    """A real-valued fused decoder level: x [B, Hh, Wh, 2C] and skip [B, 2Hh, 2Wh, C] ReLU-like activations (bf16
+    values, float64) and model.compose_upconv of He-scaled fp32 weights and real biases: (x, skip, comp, skipw, bias9)
+    with comp / skipw the bf16 blobs as float64 and bias9 the fp32 class table as float64."""
+    from unet_dc_segmentation_b200.model import compose_upconv
+    g = torch.Generator().manual_seed(seed)
+    x = (torch.randn(B, Hh, Wh, 2 * C, generator=g).clamp(min=0) * 1.7).bfloat16().double()
+    skip = (torch.randn(B, 2 * Hh, 2 * Wh, C, generator=g).clamp(min=0) * 1.7).bfloat16().double()
+    wu = torch.randn(2 * C, C, 2, 2, generator=g) * (2.0 / (4 * 2 * C)) ** 0.5
+    bu = torch.randn(C, generator=g) * 0.1
+    wd = torch.randn(C, 2 * C, 3, 3, generator=g) * (2.0 / (9 * 2 * C)) ** 0.5
+    bd = torch.randn(C, generator=g) * 0.1
+    comp, skipw, bias9 = compose_upconv(wu.float(), bu.float(), wd.float(), bd.float())
+    return x, skip, comp.double(), skipw.double(), bias9.double()
 
 
 def real_operands(B, H, W, cin, cout, seed, upconv=False):
@@ -208,6 +351,32 @@ def store_bf16(acc, bias, relu):
     if relu:
         x = x.clamp(min=0)
     return x.float().bfloat16().double()
+
+
+def store_border_bf16(acc, bias9, relu):
+    """The fused kernels' epilogue (run_epilogue, UPF with border_bias): acc [B, 2 Hh, 2 Wh, Co] at full resolution,
+    bias9 [9, Co] fp32 (model.compose_upconv; row = row class * 3 + column class, class 0 / 1 / 2 = first / interior /
+    last output row or column).  Every pixel gets the fp32 add of the interior row 4; a pixel of another class then
+    gets a second fp32 add of fp32(bias9[class] - bias9[4]) (two roundings, not one add of bias9[class]).  Then
+    cvt.rn(.relu) to bf16."""
+    _, H, W, _ = acc.shape
+    b9 = bias9.float()
+    x = (acc.float() + b9[4]).double()
+    rc = torch.ones(H, dtype=torch.long, device=acc.device)
+    cc = torch.ones(W, dtype=torch.long, device=acc.device)
+    rc[0], rc[-1] = 0, 2
+    cc[0], cc[-1] = 0, 2
+    cls = rc[:, None] * 3 + cc[None, :]                                # [H, W]
+    delta = (b9 - b9[4]).double()[cls]                                 # [H, W, Co], fp32 values
+    x = torch.where((cls != 4)[..., None], (x.float() + delta.float()).double(), x)
+    if relu:
+        x = x.clamp(min=0)
+    return x.float().bfloat16().double()
+
+
+def pool_bf16(y):
+    """2x2 max pool of stored bf16 values (NHWC float64): the pool epilogues take the max of the bf16-rounded values."""
+    return F.max_pool2d(y.permute(0, 3, 1, 2), 2).permute(0, 2, 3, 1)
 
 
 def store_split(acc, bias, relu):

@@ -8,9 +8,11 @@ candidate models (tc_accum_model.CANDIDATES) it rules out, and together they mus
 Layers: real-valued operands (ReLU-like activations, He-scaled weights, real biases), which the exact tier of
 test_gpu_exact.py / test_gpu_fp32.py cannot use, each stored output equal to the model's replay of the kernel's K walk
 and epilogue, inside sentinel guards, with unread channels holding bf16 NaN: the split kernel's epilogues, the bf16
-per-tap / halo / pair kernels, the unfused bf16 transposed conv and the stem.  Forward: the calibrated network's fp32
-forward as a chain of single-layer launches, every layer equal to the model's replay of its own GPU input, and m(x)
-bit-identical to the chain.  The replay runs in torch float64 on the GPU as a plain reference."""
+per-tap / halo / pair kernels (STORE and STORE_POOL), the unfused bf16 transposed conv, the stem, conv_par2_kernel
+(STORE, STORE_POOL, HEAD) and the fused upconv + conv kernels (conv_upfused2_kernel, conv_upfused_wide_kernel).
+Forward: the calibrated network's fp32 forward and its default bf16 forward, each as a chain of single-layer launches,
+every layer equal to the model's replay of its own GPU input, and m(x) bit-identical to the chain.  The replay runs in
+torch float64 on the GPU as a plain reference."""
 
 import pytest
 import torch
@@ -19,6 +21,7 @@ import exact_net as en
 import split_model as sm
 import tc_accum_model as tm
 from exact_net import family  # noqa: F401  (fixture)
+from test_gpu_exact import PARITY_CASES, UPFUSED_CASES, WIDE_CASES
 from test_gpu_fp32 import CONV_CASES, POOL_CASES
 
 pytestmark = pytest.mark.gpu
@@ -403,3 +406,287 @@ def test_fp32_forward_chain(cuda_device, B, H, W):
     err = {k: float((v.double().cpu() - p64).abs().max()) for k, v in
            (("GPU forward = model forward", prob), ("six terms, exact sums", six), ("CPU fp32 network", cpu))}
     print(f"{B}x{H}x{W}: max |dp| vs float64: " + ", ".join(f"{k} {v:.3e}" for k, v in err.items()))
+
+
+# ----------------------------------------------------------------------------- real-valued parity-class and fused layers
+
+def _nan_buf(x64, width, off):
+    """bf16 NHWC [..., width] on the device: x64 at channels [off, off + C), bf16 NaN everywhere else."""
+    buf = torch.full(tuple(x64.shape[:-1]) + (width,), float("nan"), dtype=torch.bfloat16)
+    buf[..., off:off + x64.shape[-1]] = x64.bfloat16()
+    return buf.cuda()
+
+
+@pytest.mark.parametrize("i", range(len(PARITY_CASES)))
+def test_bf16_par2_real(cuda_device, i):
+    """conv_par2_kernel (weight_par) on a real-valued 64 -> 64 layer: STORE without ReLU into a slice, STORE_POOL with
+    ReLU and HEAD, each equal to the model's replay of the parity-class walk (tc_accum_model.upf_walks(PAR_CHUNKS))."""
+    from unet_dc_segmentation_b200.model import pack_conv3x3, pack_par3x3
+    L = _L()
+    B, H, W = PARITY_CASES[i]
+    x, w, b = tm.real_operands(B, H, W, 64, 64, seed=1300 + i)
+    x = x.bfloat16().double()
+    ws = w.permute(2, 3, 0, 1).bfloat16().double()
+    tm.assert_normal_products([x], [ws])
+    acc = tm.class_acc(None, x.cuda(), None, ws.cuda(), tm.upf_walks(tm.PAR_CHUNKS))
+    xin = _nan_buf(x, 128, 32)
+    wp, wpar, bias = pack_conv3x3(w).cuda(), pack_par3x3(w.float()).cuda(), b.float().cuda()
+    common = dict(kind=L.DC_KIND_CONV3X3, B=B, H=H, W=W, Cin=64, Cout=64, dilation=1, in_=xin[..., 32:].data_ptr(),
+                  in_stride=128, weight=wp.data_ptr(), bias=bias.data_ptr(), weight_par=wpar.data_ptr())
+    case = f"real par2 {B}x{H}x{W}"
+    raw, out = en.guarded((B, H, W, 128), torch.bfloat16)
+    en.conv_tc(epilogue=L.DC_EPI_STORE, relu=0, out=out.data_ptr(), out_stride=128, out_offset=32, **common)
+    en.assert_exact(out[..., 32:96], tm.store_bf16(acc, b.cuda(), False).cpu(), f"{case}: store")
+    en.check_outside(raw, out, 32, 64, f"{case}: store")
+    raw, out = en.guarded((B, H, W, 128), torch.bfloat16)
+    praw, pooled = en.guarded((B, H // 2, W // 2, 64), torch.bfloat16)
+    en.conv_tc(epilogue=L.DC_EPI_STORE_POOL, relu=1, out=out.data_ptr(), out_stride=128, out_offset=32,
+               pool_out=pooled.data_ptr(), pool_stride=64, **common)
+    y = tm.store_bf16(acc, b.cuda(), True).cpu()
+    en.assert_exact(out[..., 32:96], y, f"{case}: store_pool")
+    en.check_outside(raw, out, 32, 64, f"{case}: store_pool")
+    en.assert_exact(pooled, tm.pool_bf16(y), f"{case}: pooled")
+    en.check_guards(praw, f"{case}: pooled")
+    feat = tm.store_split(acc, b.cuda(), True)
+    g = torch.Generator().manual_seed(1400 + i)
+    hw = (torch.randn(64, generator=g) * 0.3).float()
+    hb = float(torch.tensor(-float((feat.cpu() @ hw.double()).mean())).float())
+    logits = tm.head_logit(feat, hw.cuda(), hb).cpu()
+    hwd = hw.cuda()
+    praw, prob = en.guarded((B, H, W), torch.float32)
+    mraw, mask = en.guarded((B, H, W), torch.uint8)
+    en.conv_tc(epilogue=L.DC_EPI_HEAD, relu=1, head_w=hwd.data_ptr(), head_b=hb, thresh=THRESH,
+               prob_out=prob.data_ptr(), mask_out=mask.data_ptr(), **common)
+    en.assert_probs(prob, mask, logits, THRESH, f"{case}: head")
+    en.check_guards(praw, f"{case}: head")
+    en.check_guards(mraw, f"{case}: head")
+
+
+def _upfused_real(C, B, Hh, Wh, seed, relu):
+    """dc_conv_upfused on a real-valued level: x at channels [0, 2C) of a 2C + 64 wide buffer, skip at [64, 64 + C) of a
+    C + 128 wide one (NaN elsewhere), the output in a slice; equal to the model's walk and border-class epilogue."""
+    import ctypes
+    from unet_dc_segmentation_b200.model import pack_upfused, pack_upfused_wide
+    L = _L()
+    x, s, comp, skipw, bias9 = tm.upfused_real_operands(C, B, Hh, Wh, seed)
+    tm.assert_normal_products([x, s], [comp, skipw])
+    walks = tm.upf_walks(tm.UPF_CHUNKS) if C == 64 else tm.wide_walks(C)
+    want = tm.store_border_bf16(tm.class_acc(x.cuda(), s.cuda(), comp.cuda(), skipw.cuda(), walks), bias9.cuda(), relu).cpu()
+    ws = None
+    if C == 64:
+        wx = pack_upfused(comp.bfloat16(), skipw.bfloat16()).cuda()
+    else:
+        wx, ws = (t.cuda() for t in pack_upfused_wide(comp.bfloat16(), skipw.bfloat16()))
+    xin, skip = _nan_buf(x, 2 * C + 64, 0), _nan_buf(s, C + 128, 64)
+    raw, out = en.guarded((B, 2 * Hh, 2 * Wh, C + 32), torch.bfloat16)
+    b9 = bias9.float().cuda()
+    a = L.UpfuseArgs()
+    a.B, a.H, a.W, a.channels = B, Hh, Wh, C
+    a.x, a.x_stride = xin.data_ptr(), 2 * C + 64
+    a.skip, a.skip_stride = skip.data_ptr() + 2 * 64, C + 128
+    a.weight, a.bias9, a.relu = wx.data_ptr(), b9.data_ptr(), int(relu)
+    if ws is not None:
+        a.weight_skip = ws.data_ptr()
+    a.out, a.out_stride, a.out_offset = out.data_ptr(), C + 32, 16
+    L.check(L.load().dc_conv_upfused(ctypes.byref(a), L.stream_ptr()))
+    torch.cuda.synchronize()
+    case = f"real upfused C={C} {B}x{Hh}x{Wh} relu={relu}"
+    en.assert_exact(out[..., 16:16 + C], want, case)
+    en.check_outside(raw, out, 16, C, case)
+
+
+@pytest.mark.parametrize("i", range(len(UPFUSED_CASES)))
+def test_bf16_upfused_real(cuda_device, i):
+    """conv_upfused2_kernel (C = 64): tiles of 16 x 8 half-resolution pixels, ragged in either axis, B > 1."""
+    B, Hh, Wh = UPFUSED_CASES[i]
+    _upfused_real(64, B, Hh, Wh, 1100 + i, i % 2 == 0)
+
+
+@pytest.mark.parametrize("i", range(len(WIDE_CASES)))
+def test_bf16_upfused_wide_real(cuda_device, i):
+    """conv_upfused_wide_kernel: C = 128 (BN = 128, two classes per pass), 256 and 512 (BN = 256, one class per pass)."""
+    C, B, Hh, Wh = WIDE_CASES[i]
+    _upfused_real(C, B, Hh, Wh, 1200 + i, i % 2 == 0)
+
+
+def _bf16_order(fam, d):
+    """K order of a bf16 3x3 layer outside conv_par2_kernel: the pair / halo kernels in auto at dilation <= 4, else the
+    per-tap kernel (launch_conv_tc)."""
+    return "chunk" if fam == "auto" and d <= 4 else "tap"
+
+
+# enc2.3, enc3.3, enc4.3 of the default network (pair kernel, pair kernel, per-tap kernel in auto)
+POOL_BF16_CASES = [(2, 24, 40, 128, 2), (1, 32, 24, 256, 4), (2, 16, 16, 512, 8)]
+
+
+@pytest.mark.parametrize("fam", ["auto", "generic"])
+@pytest.mark.parametrize("i", range(len(POOL_BF16_CASES)))
+def test_bf16_pool_real(cuda_device, family, fam, i):
+    """STORE_POOL of the bf16 pair / halo / per-tap kernels: the full-resolution store and the 2x2 max of it."""
+    from unet_dc_segmentation_b200.model import pack_conv3x3
+    L = _L()
+    B, H, W, c, d = POOL_BF16_CASES[i]
+    family(fam)
+    x, w, b = tm.real_operands(B, H, W, c, c, seed=1500 + i)
+    x = x.bfloat16().double()
+    wp = pack_conv3x3(w)
+    ws = wp.double().reshape(c, 9, c)
+    tm.assert_normal_products([x], [ws])
+    y = tm.store_bf16(tm.run_steps(tm.conv_steps([x.cuda()], [ws.cuda()], d, order=_bf16_order(fam, d))), b.cuda(), True).cpu()
+    xin = _nan_buf(x, c + 64, 32)
+    raw, out = en.guarded((B, H, W, 2 * c), torch.bfloat16)
+    praw, pooled = en.guarded((B, H // 2, W // 2, c + 64), torch.bfloat16)
+    bias = b.float().cuda()
+    en.conv_tc(kind=L.DC_KIND_CONV3X3, epilogue=L.DC_EPI_STORE_POOL, relu=1, B=B, H=H, W=W, Cin=c, Cout=c, dilation=d,
+               in_=xin[..., 32:].data_ptr(), in_stride=c + 64, weight=wp.cuda().data_ptr(), bias=bias.data_ptr(),
+               out=out.data_ptr(), out_stride=2 * c, out_offset=c, pool_out=pooled.data_ptr(), pool_stride=c + 64)
+    case = f"real bf16 pool {c} d{d} {B}x{H}x{W} {fam}"
+    en.assert_exact(out[..., c:2 * c], y, case)
+    en.check_outside(raw, out, c, c, case)
+    en.assert_exact(pooled[..., :c], tm.pool_bf16(y), f"{case}: pooled")
+    en.check_outside(praw, pooled, 0, c, f"{case}: pooled")
+
+
+# ----------------------------------------------------------------------------- the bf16 forward as a chain of layers
+
+def _bf16_blobs(m):
+    """The packed bf16 model's blobs by role (model._Packed: per layer [parity blob], weight, bias; the head; the fused
+    level-1 blob and bias9; per wide level x weights, skip weights, bias9)."""
+    from unet_dc_segmentation_b200.model import _LAYER_ORDER
+    it = iter(m.packed().blobs)
+    wts, bss, par = [], [], {}
+    for i, (name, idx) in enumerate(_LAYER_ORDER):
+        if m.parity_level1 and idx == 3 and name in m.parity_layers:
+            par[i] = next(it)
+        wts.append(next(it))
+        bss.append(next(it))
+    hw, hb = next(it), next(it)
+    fused = {1: (next(it), None, next(it))}
+    for lvl in (2, 3, 4):
+        fused[lvl] = (next(it), next(it), next(it))
+    assert next(it, None) is None and set(par) == {1, 21} and tuple(par[1].shape) == (2, 1152, 64)
+    return wts, bss, par, hw, float(hb[0]), fused
+
+
+@pytest.mark.parametrize("fam", ["auto", "generic"])
+@pytest.mark.parametrize("B,H,W", [(1, 64, 64), (2, 48, 80)])
+def test_bf16_forward_chain(cuda_device, family, fam, B, H, W):
+    """The calibrated network's default bf16 forward run as dc_forward runs it (forward_impl, csrc/api.cu): the stem,
+    enc1.3 STORE_POOL (conv_par2_kernel in auto), enc2-4 and the bottleneck, upconv + dec.0 fused for levels 4-2
+    (conv_upfused_wide_kernel) and level 1 (conv_upfused2_kernel), each dec.3, dec1.3 HEAD (conv_par2_kernel in auto),
+    one launch at a time from the model's own blobs.  Every layer equals the model's replay of its own GPU input bit for
+    bit, and predict_u8 (u8 grey stem) and m(x) (fp32 stem) give exactly the chain's probabilities and mask.  Under
+    family generic conv_par2_kernel and the pair / halo kernels are off (launch_conv_tc), the fused kernels are not."""
+    import ctypes
+    import numpy as np
+    import test_gpu_fp32 as t32
+    from unet_dc_segmentation_b200 import UNetDC
+    from unet_dc_segmentation_b200.model import fused_level_blobs, pack_upfused, pack_upfused_wide
+    L = _L()
+    family(fam)
+    sd = t32._calibrated()
+    m = UNetDC()
+    m.load_state_dict(sd)
+    m = m.cuda().eval()
+    wts, bss, par, hw, hb, fused = _bf16_blobs(m)
+    sdd = {k: v.detach().cuda() for k, v in m.state_dict().items()}
+    dil = m.dilations
+    u8 = t32._frames(B, max(H, W), 60)[:, :H, :W].contiguous()
+    x32 = torch.from_numpy(u8.numpy().astype("float32") / np.float32(255))[:, None].expand(B, 3, H, W).contiguous()
+
+    def buf(h, w, c):
+        return torch.full((B, h, w, c), float("nan"), dtype=torch.bfloat16, device="cuda")
+
+    def conv(i, epi, relu, h, w, cin, cout, d, src, dst=None, pool=None, prob=None, mask=None):
+        wpar = par.get(i)
+        kw = dict(kind=L.DC_KIND_CONV3X3, epilogue=epi, relu=relu, B=B, H=h, W=w, Cin=cin, Cout=cout, dilation=d,
+                  in_=src.data_ptr(), in_stride=src.shape[-1], weight=wts[i].data_ptr(), bias=bss[i].data_ptr(),
+                  weight_par=wpar.data_ptr() if wpar is not None else None)
+        if dst is not None:
+            kw.update(out=dst.data_ptr(), out_stride=dst.shape[-1], out_offset=0)
+        if pool is not None:
+            kw.update(pool_out=pool.data_ptr(), pool_stride=cout)
+        if epi == L.DC_EPI_HEAD:
+            kw.update(head_w=hw.data_ptr(), head_b=hb, thresh=THRESH, prob_out=prob.data_ptr(), mask_out=mask.data_ptr())
+        en.conv_tc(**kw)
+        xs, bias = src[..., :cin].double(), bss[i].double()
+        w64 = wts[i].double().reshape(cout, 3, 3, cin)
+        if wpar is not None and fam == "auto" and d == 1:               # launch_conv_tc's test for conv_par2_kernel
+            acc = tm.class_acc(None, xs, None, w64.permute(1, 2, 0, 3), tm.upf_walks(tm.PAR_CHUNKS))
+        else:
+            acc = tm.run_steps(tm.conv_steps([xs], [w64.reshape(cout, 9, cin)], d, order=_bf16_order(fam, d)))
+        case = f"bf16 chain {B}x{H}x{W} {fam} layer {i}"
+        if epi == L.DC_EPI_HEAD:
+            logit = tm.head_logit(tm.store_split(acc, bias, True), hw, hb).cpu()
+            en.assert_probs(prob, mask, logit, THRESH, case)
+            return
+        y = tm.store_bf16(acc, bias, relu).cpu()
+        en.assert_exact(dst, y, case)
+        if pool is not None:
+            en.assert_exact(pool, tm.pool_bf16(y), f"{case}: pooled")
+
+    def upfused(lvl, h, w, c, src, skip, dst):
+        wx, wsk, b9 = fused[lvl]
+        comp, skipw, bias9 = fused_level_blobs(sdd, lvl, m._bn_eps(f"dec{lvl}", 1))
+        if lvl == 1:
+            assert torch.equal(pack_upfused(comp, skipw), wx)
+        else:
+            assert all(torch.equal(p, q) for p, q in zip(pack_upfused_wide(comp, skipw), (wx, wsk)))
+        assert torch.equal(bias9, b9)
+        a = L.UpfuseArgs()
+        a.B, a.H, a.W, a.channels = B, h // 2, w // 2, c
+        a.x, a.x_stride, a.skip, a.skip_stride = src.data_ptr(), 2 * c, skip.data_ptr(), c
+        a.weight, a.bias9, a.relu = wx.data_ptr(), b9.data_ptr(), 1
+        if wsk is not None:
+            a.weight_skip = wsk.data_ptr()
+        a.out, a.out_stride, a.out_offset = dst.data_ptr(), c, 0
+        L.check(L.load().dc_conv_upfused(ctypes.byref(a), L.stream_ptr()))
+        torch.cuda.synchronize()
+        xs, ss = src.double(), skip.double()
+        tm.assert_normal_products([xs, ss], [comp.double(), skipw.double()])
+        walks = tm.upf_walks(tm.UPF_CHUNKS) if lvl == 1 else tm.wide_walks(c)
+        acc = tm.class_acc(xs, ss, comp.double(), skipw.double(), walks)
+        en.assert_exact(dst, tm.store_border_bf16(acc, bias9.double(), True).cpu(), f"bf16 chain {B}x{H}x{W} {fam} fused level {lvl}")
+
+    def chain(in_kind):
+        a = [buf(H >> l, W >> l, 64 << l) for l in range(5)]
+        cat = [buf(H >> l, W >> l, 64 << l) for l in range(4)]          # fused levels: the skip half alone
+        pool = [buf(H >> (l + 1), W >> (l + 1), 64 << l) for l in range(4)]
+        dev = u8.cuda() if in_kind == 1 else x32.cuda()
+        s = L.StemArgs(in_kind, B, H, W, 64, dil[0], dev.data_ptr(), wts[0].data_ptr(), bss[0].data_ptr(), a[0].data_ptr(),
+                       64, 0)
+        L.check(L.load().dc_stem(ctypes.byref(s), L.stream_ptr()))
+        torch.cuda.synchronize()
+        x64 = u8.double()[:, None] if in_kind == 1 else x32.bfloat16().double()
+        acc = tm.run_steps(tm.stem_steps(tm.stem_cols(x64, dil[0]).cuda(), tm.stem_weights(wts[0].double(), in_kind)))
+        en.assert_exact(a[0], tm.store_bf16(acc, bss[0].double(), True).cpu(), f"bf16 chain {B}x{H}x{W} stem {in_kind}")
+        conv(1, L.DC_EPI_STORE_POOL, 1, H, W, 64, 64, dil[0], a[0], cat[0], pool[0])
+        for l in range(1, 4):
+            h, w, c = H >> l, W >> l, 64 << l
+            conv(2 * l, L.DC_EPI_STORE, 1, h, w, c // 2, c, dil[l], pool[l - 1], a[l])
+            conv(2 * l + 1, L.DC_EPI_STORE_POOL, 1, h, w, c, c, dil[l], a[l], cat[l], pool[l])
+        bott = buf(H >> 4, W >> 4, 1024)
+        conv(8, L.DC_EPI_STORE, 1, H >> 4, W >> 4, 512, 1024, dil[4], pool[3], a[4])
+        conv(9, L.DC_EPI_STORE, 1, H >> 4, W >> 4, 1024, 1024, dil[4], a[4], bott)
+        src = bott
+        prob = torch.full((B, H, W), float("nan"), device="cuda")
+        mask = torch.full((B, H, W), 7, dtype=torch.uint8, device="cuda")
+        for l in (3, 2, 1, 0):
+            h, w, c = H >> l, W >> l, 64 << l
+            ad = buf(h, w, c)
+            upfused(l + 1, h, w, c, src, cat[l], ad)
+            if l > 0:
+                src = buf(h, w, c)
+                conv(12 + 3 * (3 - l), L.DC_EPI_STORE, 1, h, w, c, c, 1, ad, src)
+            else:
+                conv(21, L.DC_EPI_HEAD, 1, h, w, c, c, 1, ad, prob=prob, mask=mask)
+        return prob, mask
+
+    prob, mask = chain(1)
+    mk, pr = m.predict_u8(u8.cuda(), THRESH, return_prob=True)
+    assert torch.equal(pr[:, 0], prob) and torch.equal(mk, mask), "predict_u8 differs from the layer chain"
+    prob0, _ = chain(0)
+    assert torch.equal(m(x32.cuda())[:, 0], prob0), "m(x) differs from the layer chain"
+    p64 = sm.network(sd, x32)
+    err = {k: float((v.double().cpu() - p64).abs().max()) for k, v in (("u8 grey entry", prob), ("fp32 entry", prob0))}
+    print(f"{B}x{H}x{W} {fam}: bf16 forward max |dp| vs float64: " + ", ".join(f"{k} {v:.3e}" for k, v in err.items()))

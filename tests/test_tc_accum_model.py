@@ -158,3 +158,121 @@ def test_teeth_k_order():
     assert not torch.equal(_bf16_layer(M, "tap"), _bf16_layer(M, "chunk"))
     reordered = _split_layer(M, terms=tuple(reversed(sm.TERMS)))
     assert not torch.equal(reordered, _split_layer(M))
+
+
+# ----------------------------------------------------------------------------- parity-class and fused kernels
+
+def _par_weights(w):
+    """conv_par2_kernel's B operands: the 3x3 weights as bf16 [ky][kx][co][ci] (float64)."""
+    return w.permute(2, 3, 0, 1).bfloat16().double()
+
+
+@pytest.mark.parametrize("reverse", [False, True])
+def test_par2_walk_covers_the_layer(reverse):
+    """On integer operands every sum is exact: the walk (and its epilogues) must give the plain float64 conv, so it
+    visits every (class, tap, channel) product once.  The reversed-group walk covers the same products."""
+    x = en.acts((2, 16, 32, 64), 21)
+    w = en.conv_weight(64, 64, "dense", 22)
+    b = en.biases(64, 23)
+    acc = tm.class_acc(None, x, None, _par_weights(w), tm.upf_walks(tm.PAR_CHUNKS, reverse_groups=reverse))
+    y = tm.store_bf16(acc, b, True)
+    assert torch.equal(y, en.bf16(en.conv3x3_ref(x, w, b, 1, True)).double())
+    assert torch.equal(tm.pool_bf16(y), en.bf16(tm.pool_bf16(en.conv3x3_ref(x, w, b, 1, True))).double())
+    assert torch.equal(tm.store_bf16(acc, b, False), en.bf16(en.conv3x3_ref(x, w, b, 1, False)).double())
+
+
+def _upfused_exact(C, B, Hh, Wh, walks, relu):
+    from unet_dc_segmentation_b200.model import compose_upconv
+    wu, bu, wd, bd = en.upfused_operands(C, 40 + C, "dense")
+    x, s = en.acts((B, Hh, Wh, 2 * C), C + 1), en.acts((B, 2 * Hh, 2 * Wh, C), C + 2)
+    en.assert_bound(lambda *o: en.upfused_ref(*o, relu=False), x, s, wu, bu, wd, bd)
+    comp, skipw, bias9 = compose_upconv(wu.float(), bu.float(), wd.float(), bd.float())
+    got = tm.store_border_bf16(tm.class_acc(x, s, comp.double(), skipw.double(), walks), bias9.double(), relu)
+    assert torch.equal(got, en.bf16(en.upfused_ref(x, s, wu, bu, wd, bd, relu)).double())
+
+
+@pytest.mark.parametrize("relu", [False, True])
+def test_upfused_walk_covers_the_layer(relu):
+    """conv_upfused2_kernel's walk and border-class epilogue give the unfused chain upconv -> cat -> conv exactly on
+    integer operands (3 x 5 half-resolution pixels: every border class)."""
+    _upfused_exact(64, 2, 3, 5, tm.upf_walks(tm.UPF_CHUNKS), relu)
+
+
+@pytest.mark.parametrize("C", [128, 256])
+def test_wide_walk_covers_the_layer(C):
+    _upfused_exact(C, 1, 3, 2, tm.wide_walks(C), True)
+
+
+def test_walks_visit_every_product_once():
+    """Each walk is a permutation of the composed layer's (source, chunk, tap, k16) items, for every class."""
+    for walks, C in ((tm.upf_walks(tm.UPF_CHUNKS), 64), (tm.wide_walks(128), 128), (tm.wide_walks(512), 512)):
+        want = sorted(tm.composed_walks(C, "tap")[0])
+        assert all(sorted(w) == want for w in walks.values())
+    want = sorted(i for i in tm.composed_walks(64, "tap")[0] if i[0] == "s")
+    assert all(sorted(w) == want for w in tm.upf_walks(tm.PAR_CHUNKS).values())
+
+
+# The operands of one case of each new GPU test in test_gpu_tc_accum.py, as the GPU test replays them.
+
+def _par2_layer(walk):
+    """PARITY_CASES[0] of test_bf16_par2_real (1 x 32 x 16, seed 1300, STORE without ReLU)."""
+    x, w, b = tm.real_operands(1, 32, 16, 64, 64, seed=1300)
+    x = x.bfloat16().double()
+    if walk in ("tap", "chunk"):
+        ws = w.permute(0, 2, 3, 1).reshape(64, 9, 64).bfloat16().double()
+        acc = tm.run_steps(tm.conv_steps([x], [ws], 1, order=walk))
+    else:
+        acc = tm.class_acc(None, x, None, _par_weights(w), tm.upf_walks(tm.PAR_CHUNKS, reverse_groups=walk == "reversed"))
+    return tm.store_bf16(acc, b, False)
+
+
+def _fused_layer(C, B, Hh, Wh, seed, walk):
+    x, s, comp, skipw, bias9 = tm.upfused_real_operands(C, B, Hh, Wh, seed)
+    kernel = (lambda rev=False: tm.upf_walks(tm.UPF_CHUNKS, rev)) if C == 64 else (lambda rev=False: tm.wide_walks(C, rev))
+    walks = {"kernel": kernel, "reversed": lambda: kernel(True), "skip first": lambda: tm.skip_first(kernel()),
+             "tap": lambda: tm.composed_walks(C, "tap"), "chunk": lambda: tm.composed_walks(C, "chunk")}[walk]()
+    return tm.store_border_bf16(tm.class_acc(x, s, comp, skipw, walks), bias9, True)
+
+
+@pytest.mark.parametrize("walk", ["tap", "chunk", "reversed"])
+def test_teeth_par2_walk(walk):
+    """conv_par2_kernel's walk predicts different bits from the unfused kernels' orders on the same layer and from its
+    own groups reversed."""
+    assert not torch.equal(_par2_layer(walk), _par2_layer("kernel"))
+
+
+@pytest.mark.parametrize("walk", ["tap", "chunk", "reversed", "skip first"])
+@pytest.mark.parametrize("C,B,Hh,Wh,seed", [(64, 1, 40, 24, 1102), (128, 1, 16, 8, 1200)])
+def test_teeth_fused_walks(C, B, Hh, Wh, seed, walk):
+    """The fused kernels' walks predict different bits from the composed layer walked (tap, chunk) or (chunk, tap),
+    from their groups reversed and from the skip chunk first (UPFUSED_CASES[2] of test_bf16_upfused_real and
+    WIDE_CASES[0] of test_bf16_upfused_wide_real)."""
+    assert not torch.equal(_fused_layer(C, B, Hh, Wh, seed, walk), _fused_layer(C, B, Hh, Wh, seed, "kernel"))
+
+
+def test_teeth_border_bias():
+    """The fused epilogue's two fp32 adds on border pixels predict different bits from one add of bias9[class]."""
+    x, s, comp, skipw, bias9 = tm.upfused_real_operands(64, 1, 40, 24, 1102)
+    acc = tm.class_acc(x, s, comp, skipw, tm.upf_walks(tm.UPF_CHUNKS))
+    H, W = acc.shape[1:3]
+    rc = torch.tensor([0] + [1] * (H - 2) + [2])
+    cc = torch.tensor([0] + [1] * (W - 2) + [2])
+    one_add = tm.store_bf16(acc, bias9[rc[:, None] * 3 + cc[None, :]], True)
+    assert not torch.equal(tm.store_border_bf16(acc, bias9, True), one_add)
+
+
+# The bits the walks predict on those operands, which test_gpu_tc_accum.py holds the kernels to on a B200: a change to
+# a walk (two groups swapped, the skip chunk moved, another tap or k16 nesting) changes them.
+PINNED = {"par2": "ef6174e68876276b", "upfused 64": "7249aba3d67337ac", "upfused wide 128": "6c5ff951040a396b"}
+
+
+def _fingerprint(y):
+    import hashlib
+    return hashlib.sha256(y.float().bfloat16().view(torch.int16).numpy().tobytes()).hexdigest()[:16]
+
+
+def test_walk_predictions_pinned():
+    got = {"par2": _fingerprint(_par2_layer("kernel")),
+           "upfused 64": _fingerprint(_fused_layer(64, 1, 40, 24, 1102, "kernel")),
+           "upfused wide 128": _fingerprint(_fused_layer(128, 1, 16, 8, 1200, "kernel"))}
+    assert got == PINNED

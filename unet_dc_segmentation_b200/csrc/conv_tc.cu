@@ -1063,7 +1063,8 @@ conv_halo2_kernel(const __grid_constant__ ConvParams p) {
 // ConvTranspose2d(128, 64, 2, stride 2) -> cat([up, skip]) -> Conv2d(128, 64, 3, padding 1) + BN + ReLU
 // (reference models/model_2.py:29, :76-77) as ONE kernel that never materialises `up`.  A 2x2/stride-2 transposed
 // conv followed by a 3x3 conv is, for the output pixels of one parity class (py, px) = (y & 1, x & 1), a 2x2-tap conv
-// over the HALF-resolution tensor x with composed weights (the host folds Wu into Wd in fp32: model.py compose_upconv)
+// over the HALF-resolution tensor x with composed weights (the host composes Wu with Wd in fp64 and rounds the result
+// to bf16 once: model.py compose_upconv)
 // -- K = 4 x 128 instead of 9 x 64 -- plus the ordinary 3x3 over the skip half sampled at stride 2.  Taps of the 3x3
 // that fall outside the upsampled image contribute nothing, bias of the transposed conv included: TMA's zero fill does
 // that for the data, the border-class bias of the epilogue for the bias.
