@@ -166,7 +166,7 @@ def assert_probs(prob, mask, logits64, thresh, case, names=("b", "y", "x")):
             raise AssertionError(f"{case}: {int(bad.sum())}/{bad.numel()} probabilities off by > 1e-6; first at ({where}): "
                                  f"got {float(p[idx])!r}, want {float(want[idx])!r} (logit {float(logits64[idx])!r})")
     if mask is not None:
-        w0 = want if want.dim() == 3 else want[:, 0]
+        w0 = want[:, 0] if want.dim() == 4 else want
         m = mask.detach().cpu()
         bad = (m != (w0 > thresh).to(torch.uint8)) & ((w0 - thresh).abs() > 1e-6)
         if bool(bad.any()):

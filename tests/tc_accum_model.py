@@ -35,7 +35,8 @@ the accumulator unchanged (probe ``identity``), so the replay does not need the 
 parity-class walks; their epilogues are ``store_border_bf16`` (the fused kernels: the interior bias row, then a second
 fp32 add of the border-class difference), ``store_bf16`` / ``pool_bf16`` / ``head_logit`` (conv_par2_kernel's STORE,
 STORE_POOL and HEAD).  With these walks every kernel of the default bf16 forward is accounted for bit for bit
-(tests/test_gpu_tc_accum.py test_bf16_forward_chain), as is every kernel of the fp32 forward.
+(tests/test_gpu_tc_accum.py test_bf16_forward_chain, and at full frame size at sampled sites,
+tests/test_gpu_tc_accum_fullsize.py), as is every kernel of the fp32 forward.
 """
 from __future__ import annotations
 
@@ -123,21 +124,92 @@ def run_steps(steps, m=MEASURED):
     return acc
 
 
+# ----------------------------------------------------------------------------- sites
+# A replay at sites computes the outputs of chosen pixels only: sites = (b, y, x), three long tensors of equal length S
+# on the maps' device, and the steps' A operands are [S, 16] instead of [B, H, W, 16].  The windows are gathered from
+# the device buffers in their own type (bf16, u8) and only then converted to float64, so a full-size map is never
+# held as float64.
+
+def _at(x, b, y, xx):
+    """NHWC x at pixels (b, y, xx) as float64 [S, C], zero where (y, xx) lies outside the map (the kernels' zero fill)."""
+    _, H, W, _ = x.shape
+    inside = ((y >= 0) & (y < H) & (xx >= 0) & (xx < W))[:, None]
+    v = x[b, y.clamp(0, H - 1), xx.clamp(0, W - 1)].double()
+    return torch.where(inside, v, torch.zeros((), dtype=torch.float64, device=v.device))
+
+
+def class_sites(sites):
+    """Half-resolution sites (b, h, w) -> the 4 S full-resolution pixels (b, 2h + py, 2w + px), class cls = py * 2 + px
+    major: the order of class_acc's rows at sites, and the 2 x 2 block of each pooled pixel (pool_bf16 blocks=True)."""
+    b, h, w = sites
+    cls = torch.arange(4, device=b.device)[:, None]
+    return b.repeat(4), (2 * h + (cls >> 1)).flatten(), (2 * w + (cls & 1)).flatten()
+
+
+SMALL_MAP = 4096            # a check of at most this many pixels (frames x h x w) replays every one of them
+PRODUCT_BUDGET = 2 ** 34    # MMA products up to which a layer's seeded random interior sites are added
+
+
+def select_sites(shape, d, tile, frames, cost, seed=0, budget=PRODUCT_BUDGET, small=SMALL_MAP):
+    """The sites (b, y, x) at which a layer is replayed: map shape = (B, h, w), dilation d, the kernel's tile grid
+    tile = (rows, columns) on that map, the frames to check, and cost = the MMA products one site replays.  A map of
+    at most `small` pixels in those frames: every pixel.  Otherwise, in every frame, the union of the border ring; the
+    rows and columns where a dilated tap crosses the edge (d - 1, d, h - d - 1, h - d); one pixel of every tile, its
+    in-tile position rotating with the tile index so that every (y mod rows, x mod columns) occurs (positions that no
+    tile reaches, on maps of fewer tiles than positions, are added in tile 0); and seeded random interior pixels of the
+    frames, as many as keep the layer within `budget` products (none if the rest is already past it).  CPU tensors,
+    sorted by (b, y, x), without repeats."""
+    _, h, w = shape
+    th, tw = tile
+    fr = torch.tensor(list(frames), dtype=torch.long)
+    if len(frames) * h * w <= small:
+        b, y, x = torch.meshgrid(fr, torch.arange(h), torch.arange(w), indexing="ij")
+        return b.flatten(), y.flatten(), x.flatten()
+    rows = sorted({0, h - 1} | {r for r in (d - 1, d, h - d - 1, h - d) if 0 <= r < h})
+    cols = sorted({0, w - 1} | {c for c in (d - 1, d, w - d - 1, w - d) if 0 <= c < w})
+    ys = [torch.full((w,), r) for r in rows] + [torch.arange(h)] * len(cols)
+    xs = [torch.arange(w)] * len(rows) + [torch.full((h,), c) for c in cols]
+    nty, ntx = -(-h // th), -(-w // tw)
+    k = torch.arange(nty * ntx)
+    ty, tx, pos = k // ntx, k % ntx, k % (th * tw)
+    ys.append(ty * th + (pos // tw) % (h - ty * th).clamp(max=th))     # a partial tile: the position wrapped into it
+    xs.append(tx * tw + (pos % tw) % (w - tx * tw).clamp(max=tw))
+    y, x = torch.cat(ys), torch.cat(xs)
+    seen = set(((y % th) * tw + x % tw).tolist())
+    miss = torch.tensor([p for p in range(th * tw) if p not in seen and p // tw < h and p % tw < w], dtype=torch.long)
+    y, x = torch.cat([y, miss // tw]), torch.cat([x, miss % tw])
+    key = torch.unique(y * w + x)
+    key = (fr[:, None] * (h * w) + key[None, :]).flatten()
+    n_rand = max(0, budget // max(cost, 1) - key.numel())
+    if n_rand and h > 2 and w > 2:
+        g = torch.Generator().manual_seed(seed)
+        rb = fr[torch.randint(0, len(frames), (n_rand,), generator=g)]
+        ry = torch.randint(1, h - 1, (n_rand,), generator=g)
+        rx = torch.randint(1, w - 1, (n_rand,), generator=g)
+        key = torch.cat([key, (rb * h + ry) * w + rx])
+    key = torch.unique(key)
+    return key // (h * w), key // w % h, key % w
+
+
 # ----------------------------------------------------------------------------- K walks of the kernels
 
-def _windows(x, d):
-    """The nine dilated 3x3 taps of NHWC x (zero padded), tap = ky * 3 + kx."""
+def _windows(x, d, sites=None):
+    """The nine dilated 3x3 taps of NHWC x (zero padded), tap = ky * 3 + kx, as float64: [B, H, W, C] maps, or [S, C]
+    at sites."""
+    if sites is not None:
+        b, y, xx = sites
+        return [_at(x, b, y + (t // 3 - 1) * d, xx + (t % 3 - 1) * d) for t in range(9)]
     _, H, W, _ = x.shape
-    xp = F.pad(x, (0, 0, d, d, d, d))
+    xp = F.pad(x.double(), (0, 0, d, d, d, d))
     return [xp[:, (t // 3) * d:(t // 3) * d + H, (t % 3) * d:(t % 3) * d + W, :] for t in range(9)]
 
 
-def conv_steps(xs, ws, d, terms=((0, 0),), order="tap"):
-    """MMA steps of a 3x3 layer.  xs: activation planes (NHWC float64 of bf16 values, Cin channels each); ws: weight
-    planes [Cout, 9, Cin] of bf16 values.  order "tap": (tap, term, chunk, k16), the per-tap kernels; "chunk":
-    (chunk, tap, k16), the halo and pair kernels (one term)."""
+def conv_steps(xs, ws, d, terms=((0, 0),), order="tap", sites=None):
+    """MMA steps of a 3x3 layer.  xs: activation planes (NHWC of bf16 values, Cin channels each); ws: weight planes
+    [Cout, 9, Cin] of bf16 values.  order "tap": (tap, term, chunk, k16), the per-tap kernels; "chunk": (chunk, tap,
+    k16), the halo and pair kernels (one term).  sites: the output pixels (b, y, x) to replay (None: all)."""
     cin = xs[0].shape[-1]
-    wins = [_windows(x, d) for x in xs]
+    wins = [_windows(x, d, sites) for x in xs]
     if order == "tap":
         for tap in range(9):
             for pa, pb in terms:
@@ -151,19 +223,21 @@ def conv_steps(xs, ws, d, terms=((0, 0),), order="tap"):
                     yield wins[0][tap][..., c:c + 16], ws[0][:, tap, c:c + 16].T
 
 
-def upconv_steps(xs, ws, terms=((0, 0),)):
-    """MMA steps of the transposed conv (GEMM N = 4 Cout): (term, chunk, k16); ws planes [4 Cout, Cin]."""
+def upconv_steps(xs, ws, terms=((0, 0),), sites=None):
+    """MMA steps of the transposed conv (GEMM N = 4 Cout): (term, chunk, k16); ws planes [4 Cout, Cin].  sites: the
+    input pixels (b, h, w) to replay (None: all)."""
     cin = xs[0].shape[-1]
+    xs = [x.double() if sites is None else _at(x, *sites) for x in xs]
     for pa, pb in terms:
         for c in range(0, cin, 16):
             yield xs[pa][..., c:c + 16], ws[pb][:, c:c + 16].T
 
 
-def stem_cols(x, d):
-    """stem_tc_kernel's im2col tile: NCHW x (3 channels, or 1 for u8 grey) -> [B, H, W, 32 or 16], K index c * 9 + tap
-    (stem_px_raw), zero padded."""
-    B, C, H, W = x.shape
-    cols = torch.stack(_windows(x.permute(0, 2, 3, 1), d), -1).reshape(B, H, W, C * 9)
+def stem_cols(x, d, sites=None):
+    """stem_tc_kernel's im2col tile: NCHW x (3 channels, or 1 for u8 grey) -> [B, H, W, 32 or 16] (or [S, 32 or 16] at
+    sites), K index c * 9 + tap (stem_px_raw), zero padded."""
+    C = x.shape[1]
+    cols = torch.stack(_windows(x.permute(0, 2, 3, 1), d, sites), -1).flatten(-2)
     return F.pad(cols, (0, (16 if C == 1 else 32) - C * 9))
 
 
@@ -271,18 +345,25 @@ def skip_first(walks):
     return {cls: [i for i in w if i[0] == "s"] + [i for i in w if i[0] == "x"] for cls, w in walks.items()}
 
 
-def class_steps(x, skip, comp, skipw, walks):
+def class_steps(x, skip, comp, skipw, walks, sites=None):
     """MMA steps of the four classes at once (class as the leading dimension): x [B, Hh, Wh, Cx] half-resolution
-    NHWC (None for conv_par2_kernel), skip [B, 2 Hh, 2 Wh, C] (float64 of bf16 values, zero padded like TMA's fill);
-    comp [4 cls][2][2][Co][Cx] and skipw [3][3][Co][C] bf16 values (model.compose_upconv; conv_par2_kernel: skipw =
-    the 3x3 weights as [ky][kx][co][ci]).  Yields (a [4, B, Hh, Wh, 16], b [4, 1, 1, 1, 16, Co])."""
-    B, H2, W2, _ = skip.shape
-    Hh, Wh = H2 // 2, W2 // 2
-    sp = F.pad(skip, (0, 0, 1, 1, 1, 1))
-    win = {("s", r, c): sp[:, r:r + 2 * Hh:2, c:c + 2 * Wh:2] for r in range(4) for c in range(4)}
-    if x is not None:
-        xp = F.pad(x, (0, 0, 1, 1, 1, 1))
-        win.update({("x", r, c): xp[:, r:r + Hh, c:c + Wh] for r in range(3) for c in range(3)})
+    NHWC (None for conv_par2_kernel), skip [B, 2 Hh, 2 Wh, C] (bf16 values, zero padded like TMA's fill); comp
+    [4 cls][2][2][Co][Cx] and skipw [3][3][Co][C] bf16 values (model.compose_upconv; conv_par2_kernel: skipw = the 3x3
+    weights as [ky][kx][co][ci]).  Yields (a [4, B, Hh, Wh, 16], b [4, 1, 1, 1, 16, Co]); at half-resolution sites
+    (b, h, w): (a [4, S, 16], b [4, 1, 16, Co])."""
+    if sites is None:
+        B, H2, W2, _ = skip.shape
+        Hh, Wh = H2 // 2, W2 // 2
+        sp = F.pad(skip.double(), (0, 0, 1, 1, 1, 1))
+        win = {("s", r, c): sp[:, r:r + 2 * Hh:2, c:c + 2 * Wh:2] for r in range(4) for c in range(4)}
+        if x is not None:
+            xp = F.pad(x.double(), (0, 0, 1, 1, 1, 1))
+            win.update({("x", r, c): xp[:, r:r + Hh, c:c + Wh] for r in range(3) for c in range(3)})
+    else:
+        b, h, w = sites
+        win = {("s", r, c): _at(skip, b, 2 * h + r - 1, 2 * w + c - 1) for r in range(4) for c in range(4)}
+        if x is not None:
+            win.update({("x", r, c): _at(x, b, h + r - 1, w + c - 1) for r in range(3) for c in range(3)})
     for items in zip(*(walks[cls] for cls in range(4))):
         As, Bs = [], []
         for cls, (src, chunk, (ty, tx), k) in enumerate(items):
@@ -290,7 +371,7 @@ def class_steps(x, skip, comp, skipw, walks):
             As.append(win[(src, (cls >> 1) + ty, (cls & 1) + tx)][..., c0:c0 + 16])
             w = comp[cls, ty, tx] if src == "x" else skipw[ty, tx]
             Bs.append(w[:, c0:c0 + 16].T)
-        yield torch.stack(As), torch.stack(Bs).view(4, 1, 1, 1, 16, -1)
+        yield torch.stack(As), torch.stack(Bs).view((4,) + (1,) * (As[0].dim() - 1) + (16, -1))
 
 
 def interleave(acc):
@@ -299,9 +380,11 @@ def interleave(acc):
     return acc.view(2, 2, B, Hh, Wh, N).permute(2, 3, 0, 4, 1, 5).reshape(B, 2 * Hh, 2 * Wh, N)
 
 
-def class_acc(x, skip, comp, skipw, walks, m=MEASURED):
-    """The fp32 accumulators of a parity-class layer at full resolution [B, 2 Hh, 2 Wh, Co]."""
-    return interleave(run_steps(class_steps(x, skip, comp, skipw, walks), m))
+def class_acc(x, skip, comp, skipw, walks, m=MEASURED, sites=None):
+    """The fp32 accumulators of a parity-class layer at full resolution [B, 2 Hh, 2 Wh, Co]; at half-resolution sites
+    [4 S, Co], the pixels of class_sites(sites)."""
+    acc = run_steps(class_steps(x, skip, comp, skipw, walks, sites), m)
+    return interleave(acc) if sites is None else acc.flatten(0, 1)
 
 
 def assert_normal_products(xs, ws):
@@ -353,29 +436,35 @@ def store_bf16(acc, bias, relu):
     return x.float().bfloat16().double()
 
 
-def store_border_bf16(acc, bias9, relu):
+def store_border_bf16(acc, bias9, relu, sites=None, size=None):
     """The fused kernels' epilogue (run_epilogue, UPF with border_bias): acc [B, 2 Hh, 2 Wh, Co] at full resolution,
     bias9 [9, Co] fp32 (model.compose_upconv; row = row class * 3 + column class, class 0 / 1 / 2 = first / interior /
     last output row or column).  Every pixel gets the fp32 add of the interior row 4; a pixel of another class then
     gets a second fp32 add of fp32(bias9[class] - bias9[4]) (two roundings, not one add of bias9[class]).  Then
-    cvt.rn(.relu) to bf16."""
-    _, H, W, _ = acc.shape
+    cvt.rn(.relu) to bf16.  At sites: acc [S, Co] at the full-resolution pixels sites = (b, y, x) of a map of
+    size = (H, W)."""
+    def klass(i, n):                                                   # 0 / 1 / 2: first / interior / last
+        return torch.where(i == n - 1, 2, torch.where(i == 0, 0, 1))
     b9 = bias9.float()
     x = (acc.float() + b9[4]).double()
-    rc = torch.ones(H, dtype=torch.long, device=acc.device)
-    cc = torch.ones(W, dtype=torch.long, device=acc.device)
-    rc[0], rc[-1] = 0, 2
-    cc[0], cc[-1] = 0, 2
-    cls = rc[:, None] * 3 + cc[None, :]                                # [H, W]
-    delta = (b9 - b9[4]).double()[cls]                                 # [H, W, Co], fp32 values
+    if sites is None:
+        _, H, W, _ = acc.shape
+        cls = klass(torch.arange(H, device=acc.device), H)[:, None] * 3 + klass(torch.arange(W, device=acc.device), W)
+    else:
+        H, W = size
+        cls = klass(sites[1], H) * 3 + klass(sites[2], W)              # [S]
+    delta = (b9 - b9[4]).double()[cls]                                 # [H, W, Co] or [S, Co], fp32 values
     x = torch.where((cls != 4)[..., None], (x.float() + delta.float()).double(), x)
     if relu:
         x = x.clamp(min=0)
     return x.float().bfloat16().double()
 
 
-def pool_bf16(y):
-    """2x2 max pool of stored bf16 values (NHWC float64): the pool epilogues take the max of the bf16-rounded values."""
+def pool_bf16(y, blocks=False):
+    """2x2 max pool of stored bf16 values (NHWC float64): the pool epilogues take the max of the bf16-rounded values.
+    blocks: y [4 S, C] holds the 2 x 2 blocks of S pooled pixels (class_sites order) -> [S, C]."""
+    if blocks:
+        return y.unflatten(0, (4, -1)).amax(0)
     return F.max_pool2d(y.permute(0, 3, 1, 2), 2).permute(0, 2, 3, 1)
 
 

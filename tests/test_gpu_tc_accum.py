@@ -20,6 +20,7 @@ import torch
 import exact_net as en
 import split_model as sm
 import tc_accum_model as tm
+import tc_chain as tc
 from exact_net import family  # noqa: F401  (fixture)
 from test_gpu_exact import PARITY_CASES, UPFUSED_CASES, WIDE_CASES
 from test_gpu_fp32 import CONV_CASES, POOL_CASES
@@ -304,99 +305,21 @@ def test_stem_real(cuda_device, in_kind, d):
 
 # ----------------------------------------------------------------------------- the fp32 forward as a chain of layers
 
-def _planes_of(buf, stride, C, off=0):
-    """The three bf16 planes (float64) of channels [off, off + C) of a [B, H, W, 3 * stride] plane buffer."""
-    return [buf[..., p * stride + off:p * stride + off + C].double() for p in range(3)]
-
-
 @pytest.mark.parametrize("B,H,W", [(1, 64, 64), (2, 48, 80)])
 def test_fp32_forward_chain(cuda_device, B, H, W):
     """The calibrated network's fp32 forward run as the forward runs it (split input, 18 convs, 4 transposed convs into
-    [up | enc] plane buffers, HEAD), one dc_conv_tc launch at a time: every layer equals the model's replay of its own
-    GPU input bit for bit, and m(x) / predict_u8 give exactly the chain's probabilities and mask.  The model forward is
-    then the GPU forward, so the model accounts for all of its error; the printed line compares it with float64."""
+    [up | enc] plane buffers, HEAD), one dc_conv_tc launch at a time (tc_chain.forward_chain): every layer equals the
+    model's replay of its own GPU input bit for bit, and m(x) / predict_u8 give exactly the chain's probabilities and
+    mask.  The model forward is then the GPU forward, so the model accounts for all of its error; the printed line
+    compares it with float64."""
     import oracle
     import test_gpu_fp32 as t32
-    L = _L()
     sd = t32._calibrated()
     m = t32._model(__import__("unet_dc_segmentation_b200").UNetDC, sd)
-    pk = m.packed()
-    wts = [pk.blobs[2 * i] for i in range(22)]
-    bss = [pk.blobs[2 * i + 1] for i in range(22)]
-    hw, hb = pk.blobs[44], float(pk.blobs[45][0])
-    dil = m.dilations
     u8 = t32._frames(B, max(H, W), 60)[:, :H, :W].contiguous()
     x32 = torch.from_numpy(u8.numpy().astype("float32") / __import__("numpy").float32(255))[:, None]
     x32 = x32.expand(B, 3, H, W).contiguous()
-
-    def buf(h, w, stride):
-        return torch.full((B, h, w, 3 * stride), float("nan"), dtype=torch.bfloat16, device="cuda")
-
-    xin = torch.zeros(B, H, W, 192, dtype=torch.bfloat16)
-    for p, pl in enumerate(sm.split64(x32.permute(0, 2, 3, 1).double())):
-        xin[..., 64 * p:64 * p + 3] = pl.bfloat16()
-    xin = xin.cuda()
-
-    def conv(i, epi, relu, h, w, cin, cout, d, src, ss, dst=None, ds=0, doff=0, pool=None, prob=None, mask=None):
-        up = epi == L.DC_EPI_UPSCATTER
-        kw = dict(kind=L.DC_KIND_UPCONV2 if up else L.DC_KIND_CONV3X3, epilogue=epi, relu=relu, B=B, H=h, W=w,
-                  Cin=cin, Cout=cout, dilation=d, in_=src.data_ptr(), in_stride=3 * ss, weight=wts[i].data_ptr(),
-                  bias=bss[i].data_ptr(), out_stride=3 * ds, out_offset=doff, planes=3, in_plane_stride=ss,
-                  out_plane_stride=ds)
-        if dst is not None:
-            kw["out"] = dst.data_ptr()
-        if pool is not None:
-            kw.update(pool_out=pool.data_ptr(), pool_stride=3 * cout, pool_plane_stride=cout)
-        if epi == L.DC_EPI_HEAD:
-            kw.update(head_w=hw.data_ptr(), head_b=hb, thresh=THRESH, prob_out=prob.data_ptr(), mask_out=mask.data_ptr())
-        en.conv_tc(**kw)
-        xs = _planes_of(src, ss, cin)
-        bias = bss[i].double()
-        case = f"chain {B}x{H}x{W} layer {i}"
-        if up:
-            ws = wts[i].double().reshape(4 * cout, 3, cin).permute(1, 0, 2)
-            tm.assert_normal_products(xs, ws)
-            y = tm.store_split(tm.run_steps(tm.upconv_steps(xs, ws, sm.TERMS)), bias.repeat(4), False)
-            want = y.reshape(B, h, w, 2, 2, cout).permute(0, 1, 3, 2, 4, 5).reshape(B, 2 * h, 2 * w, cout)
-            sm.assert_planes(dst, want, ds, doff, case, others=False)
-            return
-        ws = wts[i].double().reshape(cout, 9, 3, cin).permute(2, 0, 1, 3)
-        tm.assert_normal_products(xs, ws)
-        y = tm.store_split(tm.run_steps(tm.conv_steps(xs, ws, d, sm.TERMS)), bias, relu)
-        if epi == L.DC_EPI_HEAD:
-            logit = tm.head_logit(y, hw, hb).cpu()
-            en.assert_probs(prob, mask, logit, THRESH, case)
-            return logit
-        sm.assert_planes(dst, y, ds, doff, case, others=False)
-        if pool is not None:
-            sm.assert_planes(pool, sm.pool_split(y), cout, 0, f"{case}: pooled", others=False)
-
-    a = [buf(H >> l, W >> l, 64 << l) for l in range(5)]
-    cat = [buf(H >> l, W >> l, 128 << l) for l in range(4)]
-    pool = [buf(H >> (l + 1), W >> (l + 1), 64 << l) for l in range(4)]
-    conv(0, L.DC_EPI_STORE, 1, H, W, 64, 64, dil[0], xin, 64, a[0], 64)
-    conv(1, L.DC_EPI_STORE_POOL, 1, H, W, 64, 64, dil[0], a[0], 64, cat[0], 128, 64, pool[0])
-    for l in range(1, 4):
-        h, w, c = H >> l, W >> l, 64 << l
-        conv(2 * l, L.DC_EPI_STORE, 1, h, w, c // 2, c, dil[l], pool[l - 1], c // 2, a[l], c)
-        conv(2 * l + 1, L.DC_EPI_STORE_POOL, 1, h, w, c, c, dil[l], a[l], c, cat[l], 2 * c, c, pool[l])
-    bott = buf(H >> 4, W >> 4, 1024)
-    conv(8, L.DC_EPI_STORE, 1, H >> 4, W >> 4, 512, 1024, dil[4], pool[3], 512, a[4], 1024)
-    conv(9, L.DC_EPI_STORE, 1, H >> 4, W >> 4, 1024, 1024, dil[4], a[4], 1024, bott, 1024)
-    src = bott
-    prob = torch.full((B, H, W), float("nan"), device="cuda")
-    mask = torch.full((B, H, W), 7, dtype=torch.uint8, device="cuda")
-    for l in (3, 2, 1, 0):
-        h, w, c = H >> l, W >> l, 64 << l
-        base = 10 + 3 * (3 - l)
-        conv(base, L.DC_EPI_UPSCATTER, 0, h // 2, w // 2, 2 * c, c, 1, src, 2 * c, cat[l], 2 * c, 0)
-        ad = buf(h, w, c)
-        conv(base + 1, L.DC_EPI_STORE, 1, h, w, 2 * c, c, 1, cat[l], 2 * c, ad, c)
-        if l > 0:
-            src = buf(h, w, c)
-            conv(base + 2, L.DC_EPI_STORE, 1, h, w, c, c, 1, ad, c, src, c)
-        else:
-            conv(base + 2, L.DC_EPI_HEAD, 1, h, w, c, c, 1, ad, c, prob=prob, mask=mask)
+    prob, mask = tc.forward_chain(m, "fp32", "auto", u8.cuda(), x32.cuda(), tc.whole_map)
     mk, pr = m.predict_u8(u8.cuda(), THRESH, return_prob=True)
     assert torch.equal(pr[:, 0], prob) and torch.equal(mk, mask), "predict_u8 differs from the layer chain"
     assert torch.equal(m(x32.cuda())[:, 0], prob), "m(x) differs from the layer chain"
@@ -549,143 +472,30 @@ def test_bf16_pool_real(cuda_device, family, fam, i):
 
 # ----------------------------------------------------------------------------- the bf16 forward as a chain of layers
 
-def _bf16_blobs(m):
-    """The packed bf16 model's blobs by role (model._Packed: per layer [parity blob], weight, bias; the head; the fused
-    level-1 blob and bias9; per wide level x weights, skip weights, bias9)."""
-    from unet_dc_segmentation_b200.model import _LAYER_ORDER
-    it = iter(m.packed().blobs)
-    wts, bss, par = [], [], {}
-    for i, (name, idx) in enumerate(_LAYER_ORDER):
-        if m.parity_level1 and idx == 3 and name in m.parity_layers:
-            par[i] = next(it)
-        wts.append(next(it))
-        bss.append(next(it))
-    hw, hb = next(it), next(it)
-    fused = {1: (next(it), None, next(it))}
-    for lvl in (2, 3, 4):
-        fused[lvl] = (next(it), next(it), next(it))
-    assert next(it, None) is None and set(par) == {1, 21} and tuple(par[1].shape) == (2, 1152, 64)
-    return wts, bss, par, hw, float(hb[0]), fused
-
-
 @pytest.mark.parametrize("fam", ["auto", "generic"])
 @pytest.mark.parametrize("B,H,W", [(1, 64, 64), (2, 48, 80)])
 def test_bf16_forward_chain(cuda_device, family, fam, B, H, W):
     """The calibrated network's default bf16 forward run as dc_forward runs it (forward_impl, csrc/api.cu): the stem,
     enc1.3 STORE_POOL (conv_par2_kernel in auto), enc2-4 and the bottleneck, upconv + dec.0 fused for levels 4-2
     (conv_upfused_wide_kernel) and level 1 (conv_upfused2_kernel), each dec.3, dec1.3 HEAD (conv_par2_kernel in auto),
-    one launch at a time from the model's own blobs.  Every layer equals the model's replay of its own GPU input bit for
-    bit, and predict_u8 (u8 grey stem) and m(x) (fp32 stem) give exactly the chain's probabilities and mask.  Under
-    family generic conv_par2_kernel and the pair / halo kernels are off (launch_conv_tc), the fused kernels are not."""
-    import ctypes
+    one launch at a time from the model's own blobs (tc_chain.forward_chain).  Every layer equals the model's replay of
+    its own GPU input bit for bit, and predict_u8 (u8 grey stem) and m(x) (fp32 stem) give exactly the chain's
+    probabilities and mask.  Under family generic conv_par2_kernel and the pair / halo kernels are off
+    (launch_conv_tc), the fused kernels are not."""
     import numpy as np
     import test_gpu_fp32 as t32
     from unet_dc_segmentation_b200 import UNetDC
-    from unet_dc_segmentation_b200.model import fused_level_blobs, pack_upfused, pack_upfused_wide
-    L = _L()
     family(fam)
     sd = t32._calibrated()
     m = UNetDC()
     m.load_state_dict(sd)
     m = m.cuda().eval()
-    wts, bss, par, hw, hb, fused = _bf16_blobs(m)
-    sdd = {k: v.detach().cuda() for k, v in m.state_dict().items()}
-    dil = m.dilations
     u8 = t32._frames(B, max(H, W), 60)[:, :H, :W].contiguous()
     x32 = torch.from_numpy(u8.numpy().astype("float32") / np.float32(255))[:, None].expand(B, 3, H, W).contiguous()
-
-    def buf(h, w, c):
-        return torch.full((B, h, w, c), float("nan"), dtype=torch.bfloat16, device="cuda")
-
-    def conv(i, epi, relu, h, w, cin, cout, d, src, dst=None, pool=None, prob=None, mask=None):
-        wpar = par.get(i)
-        kw = dict(kind=L.DC_KIND_CONV3X3, epilogue=epi, relu=relu, B=B, H=h, W=w, Cin=cin, Cout=cout, dilation=d,
-                  in_=src.data_ptr(), in_stride=src.shape[-1], weight=wts[i].data_ptr(), bias=bss[i].data_ptr(),
-                  weight_par=wpar.data_ptr() if wpar is not None else None)
-        if dst is not None:
-            kw.update(out=dst.data_ptr(), out_stride=dst.shape[-1], out_offset=0)
-        if pool is not None:
-            kw.update(pool_out=pool.data_ptr(), pool_stride=cout)
-        if epi == L.DC_EPI_HEAD:
-            kw.update(head_w=hw.data_ptr(), head_b=hb, thresh=THRESH, prob_out=prob.data_ptr(), mask_out=mask.data_ptr())
-        en.conv_tc(**kw)
-        xs, bias = src[..., :cin].double(), bss[i].double()
-        w64 = wts[i].double().reshape(cout, 3, 3, cin)
-        if wpar is not None and fam == "auto" and d == 1:               # launch_conv_tc's test for conv_par2_kernel
-            acc = tm.class_acc(None, xs, None, w64.permute(1, 2, 0, 3), tm.upf_walks(tm.PAR_CHUNKS))
-        else:
-            acc = tm.run_steps(tm.conv_steps([xs], [w64.reshape(cout, 9, cin)], d, order=_bf16_order(fam, d)))
-        case = f"bf16 chain {B}x{H}x{W} {fam} layer {i}"
-        if epi == L.DC_EPI_HEAD:
-            logit = tm.head_logit(tm.store_split(acc, bias, True), hw, hb).cpu()
-            en.assert_probs(prob, mask, logit, THRESH, case)
-            return
-        y = tm.store_bf16(acc, bias, relu).cpu()
-        en.assert_exact(dst, y, case)
-        if pool is not None:
-            en.assert_exact(pool, tm.pool_bf16(y), f"{case}: pooled")
-
-    def upfused(lvl, h, w, c, src, skip, dst):
-        wx, wsk, b9 = fused[lvl]
-        comp, skipw, bias9 = fused_level_blobs(sdd, lvl, m._bn_eps(f"dec{lvl}", 1))
-        if lvl == 1:
-            assert torch.equal(pack_upfused(comp, skipw), wx)
-        else:
-            assert all(torch.equal(p, q) for p, q in zip(pack_upfused_wide(comp, skipw), (wx, wsk)))
-        assert torch.equal(bias9, b9)
-        a = L.UpfuseArgs()
-        a.B, a.H, a.W, a.channels = B, h // 2, w // 2, c
-        a.x, a.x_stride, a.skip, a.skip_stride = src.data_ptr(), 2 * c, skip.data_ptr(), c
-        a.weight, a.bias9, a.relu = wx.data_ptr(), b9.data_ptr(), 1
-        if wsk is not None:
-            a.weight_skip = wsk.data_ptr()
-        a.out, a.out_stride, a.out_offset = dst.data_ptr(), c, 0
-        L.check(L.load().dc_conv_upfused(ctypes.byref(a), L.stream_ptr()))
-        torch.cuda.synchronize()
-        xs, ss = src.double(), skip.double()
-        tm.assert_normal_products([xs, ss], [comp.double(), skipw.double()])
-        walks = tm.upf_walks(tm.UPF_CHUNKS) if lvl == 1 else tm.wide_walks(c)
-        acc = tm.class_acc(xs, ss, comp.double(), skipw.double(), walks)
-        en.assert_exact(dst, tm.store_border_bf16(acc, bias9.double(), True).cpu(), f"bf16 chain {B}x{H}x{W} {fam} fused level {lvl}")
-
-    def chain(in_kind):
-        a = [buf(H >> l, W >> l, 64 << l) for l in range(5)]
-        cat = [buf(H >> l, W >> l, 64 << l) for l in range(4)]          # fused levels: the skip half alone
-        pool = [buf(H >> (l + 1), W >> (l + 1), 64 << l) for l in range(4)]
-        dev = u8.cuda() if in_kind == 1 else x32.cuda()
-        s = L.StemArgs(in_kind, B, H, W, 64, dil[0], dev.data_ptr(), wts[0].data_ptr(), bss[0].data_ptr(), a[0].data_ptr(),
-                       64, 0)
-        L.check(L.load().dc_stem(ctypes.byref(s), L.stream_ptr()))
-        torch.cuda.synchronize()
-        x64 = u8.double()[:, None] if in_kind == 1 else x32.bfloat16().double()
-        acc = tm.run_steps(tm.stem_steps(tm.stem_cols(x64, dil[0]).cuda(), tm.stem_weights(wts[0].double(), in_kind)))
-        en.assert_exact(a[0], tm.store_bf16(acc, bss[0].double(), True).cpu(), f"bf16 chain {B}x{H}x{W} stem {in_kind}")
-        conv(1, L.DC_EPI_STORE_POOL, 1, H, W, 64, 64, dil[0], a[0], cat[0], pool[0])
-        for l in range(1, 4):
-            h, w, c = H >> l, W >> l, 64 << l
-            conv(2 * l, L.DC_EPI_STORE, 1, h, w, c // 2, c, dil[l], pool[l - 1], a[l])
-            conv(2 * l + 1, L.DC_EPI_STORE_POOL, 1, h, w, c, c, dil[l], a[l], cat[l], pool[l])
-        bott = buf(H >> 4, W >> 4, 1024)
-        conv(8, L.DC_EPI_STORE, 1, H >> 4, W >> 4, 512, 1024, dil[4], pool[3], a[4])
-        conv(9, L.DC_EPI_STORE, 1, H >> 4, W >> 4, 1024, 1024, dil[4], a[4], bott)
-        src = bott
-        prob = torch.full((B, H, W), float("nan"), device="cuda")
-        mask = torch.full((B, H, W), 7, dtype=torch.uint8, device="cuda")
-        for l in (3, 2, 1, 0):
-            h, w, c = H >> l, W >> l, 64 << l
-            ad = buf(h, w, c)
-            upfused(l + 1, h, w, c, src, cat[l], ad)
-            if l > 0:
-                src = buf(h, w, c)
-                conv(12 + 3 * (3 - l), L.DC_EPI_STORE, 1, h, w, c, c, 1, ad, src)
-            else:
-                conv(21, L.DC_EPI_HEAD, 1, h, w, c, c, 1, ad, prob=prob, mask=mask)
-        return prob, mask
-
-    prob, mask = chain(1)
+    prob, mask = tc.forward_chain(m, "bf16", fam, u8.cuda(), x32.cuda(), tc.whole_map, in_kind=1)
     mk, pr = m.predict_u8(u8.cuda(), THRESH, return_prob=True)
     assert torch.equal(pr[:, 0], prob) and torch.equal(mk, mask), "predict_u8 differs from the layer chain"
-    prob0, _ = chain(0)
+    prob0, _ = tc.forward_chain(m, "bf16", fam, u8.cuda(), x32.cuda(), tc.whole_map, in_kind=0)
     assert torch.equal(m(x32.cuda())[:, 0], prob0), "m(x) differs from the layer chain"
     p64 = sm.network(sd, x32)
     err = {k: float((v.double().cpu() - p64).abs().max()) for k, v in (("u8 grey entry", prob), ("fp32 entry", prob0))}

@@ -276,3 +276,130 @@ def test_walk_predictions_pinned():
            "upfused 64": _fingerprint(_fused_layer(64, 1, 40, 24, 1102, "kernel")),
            "upfused wide 128": _fingerprint(_fused_layer(128, 1, 16, 8, 1200, "kernel"))}
     assert got == PINNED
+
+
+# ----------------------------------------------------------------------------- replay at sites
+# The full-size chain (test_gpu_tc_accum_fullsize.py) replays chosen output sites of each layer instead of whole maps.
+# A site replay must give exactly the whole-map replay's bits at those sites, for every walk and epilogue.
+
+def _some_sites(B, h, w, d=1, tile=(4, 8)):
+    """Sites of every frame through select_sites' sampled path (the ring, edge-crossing rows, every tile, a few random
+    ones), however small the map."""
+    return tm.select_sites((B, h, w), d, tile, range(B), 1, seed=B + h + w, budget=0, small=0)
+
+
+def _at(t, s):
+    return t[s[0], s[1], s[2]]
+
+
+@pytest.mark.parametrize("walk", ["tap", "chunk", "split"])
+def test_site_replay_conv(walk):
+    """3x3 walks (tap / chunk order on bf16 maps, the split kernel's terms on planes) with the STORE, STORE_POOL and
+    HEAD epilogues.  The site replay gathers from the bf16 map itself."""
+    from unet_dc_segmentation_b200.model import pack_conv3x3, pack_conv3x3_split
+    B, H, W, cin, cout, d = 2, 10, 14, 64, 32, 3
+    x, w, b = tm.real_operands(B, H, W, cin, cout, seed=50)
+    if walk == "split":
+        xs = list(sm.split64(x).bfloat16())
+        ws = pack_conv3x3_split(w).double().reshape(cout, 9, 3, cin).permute(2, 0, 1, 3)
+        steps = lambda s: tm.conv_steps(xs, ws, d, sm.TERMS, sites=s)                       # noqa: E731
+    else:
+        xs = [x.bfloat16()]
+        ws = [pack_conv3x3(w).double().reshape(cout, 9, cin)]
+        steps = lambda s: tm.conv_steps(xs, ws, d, order=walk, sites=s)                     # noqa: E731
+    whole = tm.run_steps(steps(None))
+    s = _some_sites(B, H, W, d)
+    assert 0 < s[0].numel() < B * H * W
+    assert torch.equal(tm.run_steps(steps(s)), _at(whole, s))
+    y = tm.store_bf16(whole, b, True)
+    assert torch.equal(tm.store_bf16(tm.run_steps(steps(s)), b, True), _at(y, s))
+    pooled = tm.select_sites((B, H // 2, W // 2), 1, (2, 2), range(B), 1, budget=0, small=0)
+    blocks = tm.run_steps(steps(tm.class_sites(pooled)))
+    assert torch.equal(tm.pool_bf16(tm.store_bf16(blocks, b, True), blocks=True), _at(tm.pool_bf16(y), pooled))
+    hw = torch.linspace(-0.5, 0.5, cout, dtype=torch.float64).float().double()
+    logit = tm.head_logit(tm.store_split(whole, b, True), hw, 0.25)
+    assert torch.equal(tm.head_logit(tm.store_split(tm.run_steps(steps(s)), b, True), hw, 0.25), _at(logit, s))
+
+
+def test_site_replay_upconv():
+    from unet_dc_segmentation_b200.model import pack_upconv_split
+    B, H, W, cin, cout = 2, 5, 7, 128, 32
+    x, w, b = tm.real_operands(B, H, W, cin, cout, seed=51, upconv=True)
+    ws = pack_upconv_split(w).double().reshape(4 * cout, 3, cin).permute(1, 0, 2)
+    xs = list(sm.split64(x).bfloat16())
+    whole = tm.run_steps(tm.upconv_steps(xs, ws, sm.TERMS))
+    s = _some_sites(B, H, W)
+    assert torch.equal(tm.run_steps(tm.upconv_steps(xs, ws, sm.TERMS, sites=s)), _at(whole, s))
+
+
+@pytest.mark.parametrize("in_kind", [0, 1])
+def test_site_replay_stem(in_kind):
+    g = torch.Generator().manual_seed(52 + in_kind)
+    B, H, W, d = 2, 11, 18, 1
+    x = (torch.randint(0, 256, (B, 1, H, W), generator=g, dtype=torch.uint8) if in_kind else
+         torch.rand(B, 3, H, W, generator=g).bfloat16())
+    wk = tm.stem_weights(torch.randn(64, 27, generator=g).float().double() * 0.3, in_kind)
+    whole = tm.run_steps(tm.stem_steps(tm.stem_cols(x, d), wk))
+    s = _some_sites(B, H, W, d)
+    assert torch.equal(tm.run_steps(tm.stem_steps(tm.stem_cols(x, d, s), wk)), _at(whole, s))
+
+
+@pytest.mark.parametrize("walk", ["upf", "upf reversed", "upf skip first", "wide", "wide reversed", "par2"])
+def test_site_replay_class_walks(walk):
+    """Parity-class walks at half-resolution sites give the four class pixels of each; the fused epilogue at those
+    pixels (the border rows and columns included: the map is small enough for all of them) and the pool of each 2 x 2
+    block match the whole map."""
+    C = 128 if walk.startswith("wide") else 64
+    B, Hh, Wh = 2, 4, 6
+    x, skip, comp, skipw, bias9 = tm.upfused_real_operands(C, B, Hh, Wh, seed=53)
+    x, skip = x.bfloat16(), skip.bfloat16()
+    walks = {"upf": lambda: tm.upf_walks(tm.UPF_CHUNKS), "upf reversed": lambda: tm.upf_walks(tm.UPF_CHUNKS, True),
+             "upf skip first": lambda: tm.skip_first(tm.upf_walks(tm.UPF_CHUNKS)), "wide": lambda: tm.wide_walks(C),
+             "wide reversed": lambda: tm.wide_walks(C, True), "par2": lambda: tm.upf_walks(tm.PAR_CHUNKS)}[walk]()
+    if walk == "par2":
+        x, comp = None, None
+    whole = tm.class_acc(x, skip, comp, skipw, walks)
+    for s in (_some_sites(B, Hh, Wh, tile=(2, 2)), tm.select_sites((B, Hh, Wh), 1, (2, 4), range(B), 1)):
+        acc = tm.class_acc(x, skip, comp, skipw, walks, sites=s)
+        full = tm.class_sites(s)
+        assert torch.equal(acc, _at(whole, full))
+        y = tm.store_border_bf16(whole, bias9, True)
+        got = tm.store_border_bf16(acc, bias9, True, full, (2 * Hh, 2 * Wh))
+        assert torch.equal(got, _at(y, full))
+        assert torch.equal(tm.pool_bf16(got, blocks=True), _at(tm.pool_bf16(y), s))
+    rows, cols = tm.class_sites(s)[1], tm.class_sites(s)[2]
+    assert {0, 2 * Hh - 1} <= set(rows.tolist()) and {0, 2 * Wh - 1} <= set(cols.tolist())
+
+
+def test_select_sites():
+    """Every tile of the grid in every checked frame, every in-tile position, the ring and the rows and columns where a
+    dilated tap crosses the edge; the same sites for the same seed; the random part within the product budget."""
+    shape, d, tile, frames = (5, 100, 203), 8, (8, 16), (0, 4)
+    th, tw = tile
+    kw = dict(cost=1000, seed=3, budget=10 ** 7)
+    b, y, x = tm.select_sites(shape, d, tile, frames, **kw)
+    assert set(b.tolist()) == set(frames)
+    key = (b * 1000 + y) * 1000 + x
+    assert torch.equal(key, torch.unique(key)), "sites repeat or are not sorted"
+    assert bool(((y >= 0) & (y < 100) & (x >= 0) & (x < 203)).all())
+    for f in frames:
+        yf, xf = y[b == f], x[b == f]
+        assert len(set(zip((yf // th).tolist(), (xf // tw).tolist()))) == 13 * 13, "a tile without a site"
+        assert len(set(zip((yf % th).tolist(), (xf % tw).tolist()))) == th * tw, "an in-tile position missing"
+        for r in (0, 99, d - 1, d, 100 - d - 1, 100 - d):
+            assert int((yf == r).sum()) >= 203, f"row {r}"
+        for c in (0, 202, d - 1, d, 203 - d - 1, 203 - d):
+            assert int((xf == c).sum()) >= 100, f"column {c}"
+    again = tm.select_sites(shape, d, tile, frames, **kw)
+    assert all(torch.equal(p, q) for p, q in zip((b, y, x), again))
+    other = tm.select_sites(shape, d, tile, frames, **{**kw, "seed": 4})
+    assert not all(torch.equal(p, q) for p, q in zip((b, y, x), other))
+    assert b.numel() * kw["cost"] <= kw["budget"]
+    fixed = tm.select_sites(shape, d, tile, frames, cost=10 ** 9, budget=10 ** 7)
+    assert fixed[0].numel() < b.numel() and fixed[0].numel() * 10 ** 9 > 10 ** 7    # past the budget: no random sites
+    assert set(zip(*(t.tolist() for t in fixed))) <= set(zip(*(t.tolist() for t in (b, y, x))))
+    # a map with fewer tiles than in-tile positions still shows every position; a small map: every pixel
+    b, y, x = tm.select_sites((1, 40, 40), 16, (16, 8), (0,), cost=10 ** 9, small=0)
+    assert len(set(zip((y % 16).tolist(), (x % 8).tolist()))) == 128
+    b, y, x = tm.select_sites((3, 20, 30), 1, (8, 16), (1, 2), cost=10 ** 9)
+    assert b.numel() == 2 * 20 * 30 and set(b.tolist()) == {1, 2}
