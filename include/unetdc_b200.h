@@ -17,6 +17,7 @@
  *   dc_resize_linear_u8          the two cv2.resize calls     quantify_droplets_batch.py:44, :57
  *   dc_label_stats               quantify                     quantify_droplets_batch.py:81-95
  *   dc_table_csv                 df.to_csv of the per-image tables  quantify_droplets_batch.py:62-63
+ *   dc_png_encode                cv2.imwrite of the mask and overlay PNGs  quantify_droplets_batch.py:58, :78
  *   dc_overlay_stencil           cv2.findContours + cv2.drawContours of the overlays
  *                                                           quantify_droplets_batch.py:74-79
  *   dc_roi_mask / dc_radial_density / dc_spatial_density
@@ -51,7 +52,7 @@ extern "C" {
 /* Bumped whenever a struct or signature in this header changes, or an entry point's return code for some arguments
  * does; dc_version() returns the value the library was built with and the Python binding refuses to load a library
  * that disagrees. */
-#define DC_ABI_VERSION 210
+#define DC_ABI_VERSION 211
 
 const char* dc_last_error(void);
 int dc_version(void);
@@ -403,6 +404,37 @@ int dc_table_csv(const dc_table_csv_args_t* args, void* stream);
 int dc_debug_format_values(const void* values, int is_double, int64_t n, char* out, int64_t cap, int64_t* offsets);
 /* dc_table_csv on a table in HOST memory (every pointer of args a host pointer; the workspace is not used). */
 int dc_debug_table_csv_host(const dc_table_csv_args_t* args);
+
+/* ------------------------------------------------------------------ frames -> PNG files
+ * cv2.imwrite(path, img) with OpenCV's default PNG parameters, as the reference writes its masks (qdb:58, of mask * 255)
+ * and its overlays (qdb:78): every frame's complete file, byte for byte what OpenCV (libpng 1.6, zlib 1.3) writes --
+ * signature, IHDR (8-bit grey for C = 1, 8-bit RGB for C = 3), 8192-byte IDAT chunks, IEND; rows filtered with SUB (None
+ * when W = 1); deflate level 1, Z_RLE, memLevel 8, with libpng's zlib-header window rewrite for small images.
+ * images: u8 [B,H,W] (C = 1) or BGR [B,H,W,3] (C = 3), C-contiguous, exactly what cv2.imwrite takes (stored as RGB).
+ * Output: frame b's file is out[offsets[b] .. offsets[b+1]) (frames back to back).  Byte and bit offsets are 64-bit.
+ * No synchronisation and no allocation (the call fits in a CUDA graph), and nothing is written past out[out_bytes). */
+typedef struct dc_png_args {
+    const uint8_t* images;
+    int B, H, W, C;
+    uint8_t* out;
+    int64_t out_bytes;           /* >= dc_png_bounds(...) (DC_EINVAL otherwise) */
+    int64_t* offsets;            /* [B+1] */
+    void* workspace;             /* 256-byte aligned */
+    size_t workspace_bytes;
+} dc_png_args_t;
+
+/* out_bytes: the largest files a batch of this shape can need (zlib's deflateBound reasoning: no deflate block costs
+ * more than its stored form, plus the chunk overhead); workspace_bytes: what dc_png_encode needs.  Both static, so the
+ * encode can be captured in a CUDA graph.  Shape limits (DC_EINVAL otherwise): 1 <= B <= 65535, H, W >= 1, C 1 or 3,
+ * H * (1 + W * C) <= 2^31 - 2^20 filtered bytes per frame. */
+int dc_png_bounds(int B, int H, int W, int C, int64_t* out_bytes, size_t* workspace_bytes);
+int dc_png_encode(const dc_png_args_t* args, void* stream);
+/* TEST AID (host only, no GPU needed): the same code compiled for the host, one HOST image [H,W] / [H,W,C] -> its PNG in
+ * out (out_bytes >= dc_png_bounds(1, H, W, C)), *png_bytes its length.  block_stats (may be NULL): for deflate block
+ * k < stats_cap, its type (0 stored, 1 fixed, 2 dynamic) | 4 when the literal/length or distance code lengths were
+ * limited to 15 bits | 8 when the bit-length code lengths were limited to 7; *nblocks (may be NULL) the block count. */
+int dc_debug_png_host(const uint8_t* img, int H, int W, int C, uint8_t* out, int64_t out_bytes, int64_t* png_bytes,
+                      int32_t* block_stats, int64_t stats_cap, int64_t* nblocks);
 
 /* ---- overlay stencil --------------------------------------------------------------------------
  * stencil[b,y,x] = 1 exactly where

@@ -1,9 +1,10 @@
 """Files in -> files out through the drop-in CLI (cli.main), timed on the wall clock for both loops:
     python tools/cli_bench.py [--n 8] [--size 256] [--batch 8] [--img_size 512] [--reps 3] [--excel] [--fast_only]
-                              [--repo PATH]
+                              [--overlays] [--repo PATH]
 BASELINE config 1 = 8 frames of 256x256, batch 8, --img_size 512 (the reference's IMG_SIZE).  --excel drops
 --skip_excel (without xlsxwriter the CLI then writes all_droplets_noexcel.csv); --repo times the package of another
-checkout (A/B of two versions in one process-free comparison: run the script once per tree)."""
+checkout (A/B of two versions in one process-free comparison: run the script once per tree); --overlays adds
+--save_overlays (an overlay PNG per frame)."""
 import argparse
 import json
 import shutil
@@ -23,6 +24,7 @@ def main():
     ap.add_argument("--repo", default=str(REPO))
     ap.add_argument("--excel", action="store_true")
     ap.add_argument("--fast_only", action="store_true")
+    ap.add_argument("--overlays", action="store_true")
     ap.add_argument("--frames_dir", help="keep the generated frames and checkpoint here and reuse them on later runs")
     ap.add_argument("--n", type=int, default=8)
     ap.add_argument("--size", type=int, default=256)
@@ -41,9 +43,9 @@ def main():
             Image.fromarray(synthetic_image(a.size, i)).save(src / "in" / f"frame{i:04d}.png")
         torch.save(calibrated_state_dict(seed=0), src / "ckpt.pth")
     common = ["--img_dir", str(src / "in"), "--ckpt_path", str(src / "ckpt.pth"), "--batch", str(a.batch), "--img_size",
-              str(a.img_size), "--skip_histogram", "--px_per_micron", "3.45"] + ([] if a.excel else ["--skip_excel"])
+              str(a.img_size), "--skip_histogram", "--px_per_micron", "3.45"] + ([] if a.excel else ["--skip_excel"]) + (["--save_overlays"] if a.overlays else [])
     out = {"repo": str(a.repo), "frames": a.n, "size": a.size, "batch": a.batch, "img_size": a.img_size,
-           "excel": a.excel}
+           "excel": a.excel, "overlays": a.overlays}
     loops = (("fast", []),) if a.fast_only else (("fast", []), ("reference_loop", ["--reference_loop"]))
     for tag, extra in loops:
         times = []

@@ -3,7 +3,7 @@
 # usage (from the repo root, under gpurun): bash tools/gpu_check.sh [files...]
 mkdir -p gpurun_out
 nvidia-smi --query-gpu=name,driver_version,memory.total --format=csv > gpurun_out/smi.txt 2>&1
-FILES=${@:-"tests/test_gpu_fp32.py tests/test_gpu_tc_accum.py tests/test_gpu_tc_accum_fullsize.py tests/test_gpu_quantify.py tests/test_gpu_rolling_ball.py tests/test_gpu_resize.py tests/test_gpu_overlay.py tests/test_gpu_density.py tests/test_gpu_properties.py tests/test_gpu_conv.py tests/test_gpu_exact.py tests/test_gpu_forward.py tests/test_gpu_fullsize.py tests/test_gpu_envelope.py tests/test_gpu_rolling_ball_banded.py tests/test_gpu_cli.py tests/test_gpu_csv.py tests/test_gpu_stress.py"}
+FILES=${@:-"tests/test_gpu_fp32.py tests/test_gpu_tc_accum.py tests/test_gpu_tc_accum_fullsize.py tests/test_gpu_quantify.py tests/test_gpu_rolling_ball.py tests/test_gpu_resize.py tests/test_gpu_overlay.py tests/test_gpu_density.py tests/test_gpu_properties.py tests/test_gpu_conv.py tests/test_gpu_exact.py tests/test_gpu_forward.py tests/test_gpu_fullsize.py tests/test_gpu_envelope.py tests/test_gpu_rolling_ball_banded.py tests/test_gpu_cli.py tests/test_gpu_csv.py tests/test_gpu_png.py tests/test_gpu_stress.py"}
 rc=0
 for f in $FILES; do
   n=$(basename $f .py)

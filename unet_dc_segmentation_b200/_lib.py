@@ -17,7 +17,7 @@ DC_EPI_STORE, DC_EPI_STORE_POOL, DC_EPI_HEAD, DC_EPI_UPSCATTER = 0, 1, 2, 3
 DC_NUM_LAYERS = 23
 DC_CONV_FAMILY_AUTO, DC_CONV_FAMILY_GENERIC = 0, 2
 DC_PRECISION_BF16, DC_PRECISION_FP32 = 0, 1
-ABI_VERSION = 210          # DC_ABI_VERSION of include/unetdc_b200.h these ctypes structures mirror
+ABI_VERSION = 211          # DC_ABI_VERSION of include/unetdc_b200.h these ctypes structures mirror
 
 EXPORTS = [
     "dc_last_error", "dc_version", "dc_device_check", "dc_conv_tc", "dc_conv_upfused", "dc_debug_upfuse_schedule", "dc_debug_set_conv_family", "dc_stem", "dc_model_create",
@@ -28,6 +28,7 @@ EXPORTS = [
     "dc_roi_workspace_bytes", "dc_roi_mask", "dc_radial_workspace_bytes", "dc_radial_density",
     "dc_spatial_workspace_bytes", "dc_spatial_density",
     "dc_table_csv_bounds", "dc_table_csv", "dc_debug_format_values", "dc_debug_table_csv_host",
+    "dc_png_bounds", "dc_png_encode", "dc_debug_png_host",
 ]
 
 
@@ -120,6 +121,14 @@ class TableCsvArgs(Structure):
     ]
 
 
+class PngArgs(Structure):
+    _fields_ = [
+        ("images", c_void_p), ("B", c_int), ("H", c_int), ("W", c_int), ("C", c_int),
+        ("out", c_void_p), ("out_bytes", c_int64), ("offsets", c_void_p),
+        ("workspace", c_void_p), ("workspace_bytes", c_size_t),
+    ]
+
+
 class OverlayArgs(Structure):
     _fields_ = [
         ("mask", c_void_p), ("B", c_int), ("H", c_int), ("W", c_int), ("stencil", c_void_p),
@@ -205,6 +214,10 @@ def load(build_if_missing: bool = True) -> C.CDLL:
     lib.dc_table_csv.argtypes = [POINTER(TableCsvArgs), c_void_p]
     lib.dc_debug_format_values.argtypes = [c_void_p, c_int, c_int64, c_void_p, c_int64, c_void_p]
     lib.dc_debug_table_csv_host.argtypes = [POINTER(TableCsvArgs)]
+    lib.dc_png_bounds.argtypes = [c_int, c_int, c_int, c_int, POINTER(c_int64), POINTER(c_size_t)]
+    lib.dc_png_encode.argtypes = [POINTER(PngArgs), c_void_p]
+    lib.dc_debug_png_host.argtypes = [c_void_p, c_int, c_int, c_int, c_void_p, c_int64, POINTER(c_int64), c_void_p,
+                                      c_int64, POINTER(c_int64)]
     lib.dc_resize_linear_u8.argtypes = [POINTER(ResizeArgs), c_void_p]
     lib.dc_overlay_workspace_bytes.argtypes = [c_int, c_int, c_int, POINTER(c_size_t)]
     lib.dc_overlay_stencil.argtypes = [POINTER(OverlayArgs), c_void_p]

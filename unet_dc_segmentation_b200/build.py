@@ -15,7 +15,7 @@ PKG = Path(__file__).resolve().parent
 CSRC = PKG / "csrc"
 LIB_DIR = PKG / "lib"
 LIB_PATH = LIB_DIR / "libunetdc_b200.so"
-SOURCES = ["api.cu", "conv_tc.cu", "morph.cu", "ccl.cu", "resize.cu", "density.cu", "generic.cu", "csv.cu"]
+SOURCES = ["api.cu", "conv_tc.cu", "morph.cu", "ccl.cu", "resize.cu", "density.cu", "generic.cu", "csv.cu", "png.cu"]
 HEADERS = [CSRC / "common.cuh", CSRC / "upf_schedule.inc", CSRC / "csv_tables.inc", PKG.parent / "include" / "unetdc_b200.h"]
 
 NVCC_FLAGS = [

@@ -10,15 +10,16 @@ Function-for-function (reference file:line):
 On the device: rolling ball, both resizes (cv2.resize at qdb:44 and qdb:57 is bilinear -- the reference passes the
 interpolation flag in the `dst` slot, SURVEY.md 0.2 -- reproduced bit for bit by dc_resize_linear_u8; the identity
 when the frame is already IMG_SIZE), the network, the threshold, labelling, the table and the overlay contours (qdb:76-77,
-bit-exact against OpenCV's findContours + drawContours).  On the host, exactly as in the reference: PIL / cv2 decode,
-PNG / CSV / XLSX writing.  Added flags: `--img_size` (default 512 = the reference's
+bit-exact against OpenCV's findContours + drawContours), and in ``main`` the mask and overlay PNG files (dc_png_encode,
+byte for byte what cv2.imwrite writes, whenever the installed OpenCV is found to write those bytes).  On the host, exactly
+as in the reference: PIL / cv2 decode, the XLSX and the reports.  Added flags: `--img_size` (default 512 = the reference's
 IMG_SIZE constant) and `--density_maps` (the per-image maps of the reference's second front end, quantify_pipline.py:131-141).  Under torchrun (one rank per GPU) frames are sharded i -> rank i mod N, every
 rank writes the per-image files of its own frames, and the tables are gathered on rank 0, which writes the reports.
 
 ``main`` runs the FAST path (``run_fast``): frames are decoded by a thread pool, batched, and streamed through
-``DropletPipeline.run_host_pipelined`` -- u8 frames up, u8 masks (+ overlay stencils) and the per-image CSV files as
-text (formatted on the device by dc_table_csv) down, nothing else crosses PCIe -- while another pool writes the PNG /
-CSV files.  ``write_reports`` builds the reports of both loops from the per-image CSV texts.  ``preprocess`` / ``run_batch`` keep the
+``DropletPipeline.run_host_pipelined`` -- u8 frames (+ the overlay bases cv2.imread returned) up; u8 masks, overlay
+stencils, the per-image CSV files as text (dc_table_csv) and the mask and overlay PNG files (dc_png_encode) down --
+while another pool writes the files as bytes.  ``write_reports`` builds the reports of both loops from the per-image CSV texts.  ``preprocess`` / ``run_batch`` keep the
 reference's function-by-function shape (per-image round trips) for callers that use them as a library;
 ``--reference_loop`` makes ``main`` use them.
 """
@@ -241,6 +242,12 @@ def write_reports(out_dir: Path, per_image_rows, texts, sizes, skip_excel: bool,
             plt.close()
 
 
+def _decode_with_base(path):
+    """_decode, plus the overlay base of qdb:75 (cv2.imread; None when OpenCV cannot read the file)."""
+    import cv2
+    return _decode(path), cv2.imread(str(path))
+
+
 def _decode(path):
     """qdb:41: decode to RGB.  A frame whose three channels are identical (every grayscale file) is returned as one
     [H,W] plane: the rolling ball then corrects it once and the network folds the three identical input channels."""
@@ -266,6 +273,10 @@ def run_fast(images, mine, model, args, out_dir, mask_dir, overlay_dir):
     pipe = DropletPipeline(model, args.background_radius, args.prob_thresh, args.min_area, args.px_per_micron,
                            img_size=args.img_size)
     nthreads = max(2, min(16, (os.cpu_count() or 4)))
+    from .png import device_matches_opencv
+    png = device_matches_opencv(dev.index)           # else an OpenCV on another zlib: keep writing through cv2
+    want_ov = overlay_dir is not None
+    bases_in = png and want_ov
     metas = collections.deque()                      # one entry per batch handed to the pipeline, in order
     idx, per_image_rows, texts, sizes = [], [], [], []
 
@@ -279,40 +290,56 @@ def run_fast(images, mine, model, args, out_dir, mask_dir, overlay_dir):
                     i = next(it, None)
                     if i is None:
                         return
-                    pending.append((i, decoders.submit(_decode, images[i])))
+                    pending.append((i, decoders.submit(_decode_with_base if bases_in else _decode, images[i])))
             refill()
-            cur, cur_meta = [], []
+            cur, cur_meta, cur_base = [], [], []
+
+            def item():
+                metas.append(cur_meta)
+                names = [images[j].name for j in cur_meta]
+                if not bases_in:
+                    return np.stack(cur), names
+                # a base of another shape than the frame (an EXIF-rotated JPEG) keeps the host path: no device overlay
+                ok = [b is not None and b.shape == cur[0].shape[:2] + (3,) for b in cur_base]
+                bases = np.stack([b if o else np.zeros(cur[0].shape[:2] + (3,), np.uint8) for b, o in zip(cur_base, ok)])
+                return np.stack(cur), names, bases, np.array(ok)
             while pending:
                 i, fut = pending.popleft()
                 refill()
-                fr = fut.result()
+                fr, base = fut.result() if bases_in else (fut.result(), None)
                 if cur and (fr.shape != cur[0].shape or len(cur) == args.batch):
-                    metas.append(cur_meta)
-                    yield np.stack(cur), [images[j].name for j in cur_meta]
-                    cur, cur_meta = [], []
+                    yield item()
+                    cur, cur_meta, cur_base = [], [], []
                 cur.append(fr)
                 cur_meta.append(i)
+                cur_base.append(base)
             if cur:
-                metas.append(cur_meta)
-                yield np.stack(cur), [images[j].name for j in cur_meta]
+                yield item()
 
-        def write_image(i, mask, stencil, text):
+        def write_image(i, mask, stencil, text, mask_png, overlay_png):
             name = images[i].stem
-            cv2.imwrite(str(Path(mask_dir) / f"{name}_pred.png"), mask * 255)                 # qdb:58
+            if mask_png is not None:                                                          # qdb:58, encoded on the GPU
+                (Path(mask_dir) / f"{name}_pred.png").write_bytes(mask_png)
+            else:
+                cv2.imwrite(str(Path(mask_dir) / f"{name}_pred.png"), mask * 255)             # qdb:58
             (Path(mask_dir).parent / f"{name}_droplets.csv").write_bytes(text)                # qdb:62-63
-            if overlay_dir is not None:
+            if overlay_png is not None:                                                       # qdb:75-78 on the GPU
+                (Path(overlay_dir) / f"{name}_overlay.png").write_bytes(overlay_png)
+            elif overlay_dir is not None:
                 img = cv2.imread(str(images[i]))                                              # qdb:75
                 if img is not None:
                     draw_overlay(img, stencil)                                                # qdb:76-77, from the GPU
                     cv2.imwrite(str(Path(overlay_dir) / f"{name}_overlay.png"), img)          # qdb:78
 
         jobs = []
-        want_ov = overlay_dir is not None
-        for res in pipe.run_host_pipelined(batches(), dev, copy=True, want_overlay=want_ov, csv=True):
+        for res in pipe.run_host_pipelined(batches(), dev, copy=True, want_overlay=want_ov, csv=True, png=png):
             masks, tables = res[0], res[1]
             stencils = res[2] if want_ov else None
+            files = res[-1] if png else None
             for b, i in enumerate(metas.popleft()):
-                jobs.append(writers.submit(write_image, i, masks[b], stencils[b] if want_ov else None, tables.texts[b]))
+                jobs.append(writers.submit(write_image, i, masks[b], stencils[b] if want_ov else None, tables.texts[b],
+                                           files.masks[b] if png else None,
+                                           files.overlays[b] if bases_in else None))
                 idx.append(i)
                 texts.append(tables.texts[b])
                 sizes.append(tables.sizes[b])

@@ -253,6 +253,17 @@ int dc_debug_format_values(const void* values, int is_double, int64_t n, char* o
 
 int dc_debug_table_csv_host(const dc_table_csv_args_t* args) { return table_csv_host(args); }
 
+int dc_png_encode(const dc_png_args_t* args, void* stream) {
+    int rc = check_current_device(nullptr);
+    if (rc != DC_OK) return rc;
+    return launch_png_encode(args, (cudaStream_t)stream);
+}
+
+int dc_debug_png_host(const uint8_t* img, int H, int W, int C, uint8_t* out, int64_t out_bytes, int64_t* png_bytes,
+                      int32_t* block_stats, int64_t stats_cap, int64_t* nblocks) {
+    return png_encode_host(img, H, W, C, out, out_bytes, png_bytes, block_stats, stats_cap, nblocks);
+}
+
 int dc_overlay_workspace_bytes(int B, int H, int W, size_t* bytes) {
     DC_REQUIRE(bytes && B > 0 && H > 0 && W > 0, DC_EINVAL, "dc_overlay_workspace_bytes: bad argument");
     *bytes = overlay_workspace_bytes(B, H, W);

@@ -38,6 +38,9 @@ int upfuse_schedule(int* out, int cap);
 int launch_label_stats(const dc_label_args_t* a, cudaStream_t stream);
 int launch_table_csv(const dc_table_csv_args_t* a, cudaStream_t stream);
 int table_csv_host(const dc_table_csv_args_t* a);
+int launch_png_encode(const dc_png_args_t* a, cudaStream_t stream);
+int png_encode_host(const uint8_t* img, int H, int W, int C, uint8_t* out, int64_t out_bytes, int64_t* png_bytes,
+                    int32_t* block_stats, int64_t stats_cap, int64_t* nblocks);
 int format_values_host(const void* values, int is_double, int64_t n, char* out, int64_t cap, int64_t* offsets);
 int launch_rolling_ball(const dc_rolling_ball_args_t* a, cudaStream_t stream, bool tiled_only);
 int launch_rolling_ball_banded(const dc_rolling_ball_args_t* a, cudaStream_t stream, const char* who);

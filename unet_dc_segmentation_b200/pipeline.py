@@ -12,6 +12,7 @@ Stages, all on the current CUDA stream (no host synchronisation until the tables
                      epilogue does out_conv + sigmoid + `> prob_thresh` and writes the u8 mask
   dc_label_stats    labelling, min_area filter, compaction, area / centroid / diameter (+ micron columns)
   dc_table_csv      (run_host_pipelined(csv=True)) the per-image CSV files as text, formatted on the device
+  dc_png_encode     (run_host_pipelined(png=True)) the mask PNGs (x 255) and the painted overlays as PNG files
 """
 from __future__ import annotations
 
@@ -24,7 +25,8 @@ import torch
 from . import _lib
 from .model import UNetDC
 from .morphology import resize_linear_u8_device, rolling_ball_device, rolling_ball_workspace_bytes
-from .overlay import overlay_stencil_device, overlay_workspace_bytes
+from .overlay import OVERLAY_BGR, overlay_stencil_device, overlay_workspace_bytes
+from .png import encode_png_device, png_bounds
 from .quantify import (DEFAULT_CAPACITY, CsvTables, DropletTables, alloc_tables, csv_field, csv_text_device,
                        label_stats_device, label_workspace_bytes, pack_fields, table_csv_bounds, table_csv_device)
 
@@ -37,6 +39,12 @@ def _nvtx(name: str):
         yield
     finally:
         torch.cuda.nvtx.range_pop()
+
+
+@dataclass
+class PngFiles:
+    masks: list                    # bytes of every frame's {name}_pred.png (cv2.imwrite of mask * 255, qdb:58)
+    overlays: list | None          # bytes of every frame's overlay PNG (qdb:78); None where the frame had no base
 
 
 @dataclass
@@ -138,7 +146,8 @@ class DropletPipeline:
 
     # ------------------------------------------------------------------ pipelined host entry
     def run_host_pipelined(self, batches, device: torch.device | str = "cuda", copy: bool = True,
-                           want_overlay: bool = False, tables_archive: DropletTables | None = None, csv: bool = False):
+                           want_overlay: bool = False, tables_archive: DropletTables | None = None, csv: bool = False,
+                           png: bool = False):
         """Generator over host batches (each u8 [B,H,W] or [B,H,W,3], ideally pinned; all the same shape):
         yields (masks u8 numpy [B,H,W], list of per-image column dicts) per batch, in order.
 
@@ -158,7 +167,13 @@ class DropletPipeline:
         ``csv``: every item of ``batches`` is (images, filenames), and the tables come back as a ``CsvTables`` -- the
         per-image CSV files (qdb:62-63) formatted on the device by dc_table_csv inside the batch's own stream (and CUDA
         graph), their counts and area sums, and the one size column the reports need -- in place of the column dicts;
-        only those cross PCIe."""
+        only those cross PCIe.
+
+        ``png``: one more element is yielded, a ``PngFiles`` with every frame's mask PNG (the x 255 of qdb:58 and
+        dc_png_encode in the batch's stream and CUDA graph), byte for byte what cv2.imwrite writes.  With ``want_overlay``
+        every item also ends with the overlay bases cv2.imread returned (qdb:75) -- u8 BGR [B,H,W,3] and a per-frame
+        present flag -- and the overlays are painted (0, 255, 0) and encoded on the device too (frames without a base get
+        None).  The masks and stencils are still yielded."""
         dev = torch.device(device)
         if dev.index is None:
             dev = torch.device("cuda", torch.cuda.current_device())
@@ -176,7 +191,7 @@ class DropletPipeline:
             raise ValueError("csv=True reads the tables back as text; it cannot keep them in a tables_archive")
 
         def make_slot(shape, names_cap=0):
-            B = shape[0]
+            B, H, W = shape[:3]
             d = {"dev_in": torch.empty(shape, dtype=torch.uint8, device=dev),
                  "masks": torch.empty(tuple(shape[:3]), dtype=torch.uint8, device=dev),
                  "stencil": torch.empty(tuple(shape[:3]), dtype=torch.uint8, device=dev) if want_overlay else None,
@@ -198,13 +213,35 @@ class DropletPipeline:
                           "csv_ws": torch.empty(wsb, dtype=torch.uint8, device=dev),
                           "h_frame_off": torch.empty(B + 1, dtype=torch.int64).pin_memory(),
                           "h_area_sum": torch.empty(B, dtype=torch.int64).pin_memory()})
+            if png:
+                nbytes, wsb = png_bounds(B, H, W, 1)
+                d.update({"m255": torch.empty((B, H, W), dtype=torch.uint8, device=dev),
+                          "png_out": torch.empty(nbytes, dtype=torch.uint8, device=dev),
+                          "png_ws": torch.empty(wsb, dtype=torch.uint8, device=dev),
+                          "png_off": torch.empty(B + 1, dtype=torch.int64, device=dev),
+                          "h_png_off": torch.empty(B + 1, dtype=torch.int64).pin_memory()})
+                if want_overlay:
+                    nbytes, wsb = png_bounds(B, H, W, 3)
+                    d.update({"d_base": torch.empty((B, H, W, 3), dtype=torch.uint8, device=dev),
+                              "painted": torch.empty((B, H, W, 3), dtype=torch.uint8, device=dev),
+                              "green": torch.tensor(OVERLAY_BGR, dtype=torch.uint8, device=dev),
+                              "ov_out": torch.empty(nbytes, dtype=torch.uint8, device=dev),
+                              "ov_ws": torch.empty(wsb, dtype=torch.uint8, device=dev),
+                              "ov_off": torch.empty(B + 1, dtype=torch.int64, device=dev),
+                              "h_ov_off": torch.empty(B + 1, dtype=torch.int64).pin_memory()})
             d["ev_free"].record(s_run)
             return d
 
         h_text = [torch.empty(0, dtype=torch.uint8)]     # pinned text read-back buffer, grown on demand
+        h_png = [torch.empty(0, dtype=torch.uint8), torch.empty(0, dtype=torch.uint8)]   # mask / overlay PNG read-back
+        bases_in = png and want_overlay
 
         def stage(k, item):
-            host, names = item if csv else (item, None)
+            parts = tuple(item) if (csv or bases_in) else (item,)
+            host, names = parts[0], (parts[1] if csv else None)
+            if bases_in:
+                bases, present = parts[-2], np.asarray(parts[-1], dtype=bool)
+                bases = torch.from_numpy(np.ascontiguousarray(bases)) if isinstance(bases, np.ndarray) else bases
             host = torch.from_numpy(np.ascontiguousarray(host)) if isinstance(host, np.ndarray) else host
             if csv:
                 if len(names) != host.shape[0]:
@@ -213,7 +250,8 @@ class DropletPipeline:
             sl = slots[k % 2]
             if (sl is None or sl["dev_in"].shape != host.shape or sl["tables"].capacity != self.capacity
                     or (sl["tables"].area_um2 is not None) != micron or (sl["stencil"] is not None) != want_overlay
-                    or ("d_text" in sl) != csv or (csv and name_off[-1] > sl["names_cap"])):
+                    or ("d_text" in sl) != csv or (csv and name_off[-1] > sl["names_cap"])
+                    or ("png_out" in sl) != png or ("d_base" in sl) != bases_in):
                 names_cap = 2 * int(name_off[-1]) + 256 if csv else 0
                 sl = slots[k % 2] = make_slot(tuple(host.shape), names_cap)
             with torch.cuda.stream(s_in):
@@ -222,6 +260,11 @@ class DropletPipeline:
                 if csv:
                     sl["d_names"][:name_buf.size].copy_(torch.from_numpy(name_buf.copy()), non_blocking=True)
                     sl["d_name_off"].copy_(torch.from_numpy(name_off), non_blocking=True)
+                if bases_in:
+                    if tuple(bases.shape) != tuple(host.shape[:3]) + (3,) or bases.dtype != torch.uint8:
+                        raise ValueError(f"overlay bases must be uint8 {tuple(host.shape[:3]) + (3,)}")
+                    sl["d_base"].copy_(bases, non_blocking=True)
+                    sl["present"] = present.copy()
                 sl["ev_in"].record(s_in)
 
         archive_pos = [0]
@@ -242,6 +285,12 @@ class DropletPipeline:
                 if csv:
                     table_csv_device(tables_out, sl["d_names"], sl["d_name_off"], sl["names_cap"], sl["d_text"],
                                      sl["d_frame_off"], sl["d_area_sum"], sl["csv_ws"])
+                if png:
+                    torch.mul(sl["masks"], 255, out=sl["m255"])                                   # qdb:58
+                    encode_png_device(sl["m255"], sl["png_out"], sl["png_ws"], sl["png_off"])
+                    if want_overlay:                                                             # qdb:77-78
+                        torch.where(sl["stencil"].bool()[..., None], sl["green"], sl["d_base"], out=sl["painted"])
+                        encode_png_device(sl["painted"], sl["ov_out"], sl["ov_ws"], sl["ov_off"])
             if self.use_graphs and tables_archive is None and sl["graph"] is None and sl["uses"] >= 1:
                 # second use of the slot: every buffer the batch touches exists and is static -> capture once
                 g = torch.cuda.CUDAGraph()
@@ -262,12 +311,38 @@ class DropletPipeline:
                 if csv:
                     sl["h_frame_off"].copy_(sl["d_frame_off"], non_blocking=True)
                     sl["h_area_sum"].copy_(sl["d_area_sum"], non_blocking=True)
+                if png:
+                    sl["h_png_off"].copy_(sl["png_off"], non_blocking=True)
+                    if want_overlay:
+                        sl["h_ov_off"].copy_(sl["ov_off"], non_blocking=True)
                 sl["ev_counts"].record(s_out)
                 sl["h_masks"].copy_(sl["masks"], non_blocking=True)
                 if want_overlay:
                     sl["h_stencil"].copy_(sl["stencil"], non_blocking=True)
 
         def finish(k):
+            if not png:
+                return finish_tables(k)
+            sl = slots[k % 2]
+            sl["ev_counts"].synchronize()
+            offs = [sl["h_png_off"].numpy().copy()]
+            bufs = [sl["png_out"]]
+            if want_overlay:
+                offs.append(sl["h_ov_off"].numpy().copy())
+                bufs.append(sl["ov_out"])
+            with torch.cuda.stream(s_outs[k % 2]):       # queued before finish_tables releases the slot
+                for j, (o, buf) in enumerate(zip(offs, bufs)):
+                    total = int(o[-1])
+                    if h_png[j].numel() < total:
+                        h_png[j] = torch.empty(total + total // 2, dtype=torch.uint8).pin_memory()
+                    h_png[j][:total].copy_(buf[:total], non_blocking=True)
+            present = sl.get("present")
+            res = finish_tables(k)                        # synchronises the read-back stream
+            files = [[h_png[j].numpy()[o[b]:o[b + 1]].tobytes() for b in range(o.size - 1)] for j, o in enumerate(offs)]
+            ov = [f if p else None for f, p in zip(files[1], present)] if want_overlay else None
+            return tuple(res) + (PngFiles(files[0], ov),)
+
+        def finish_tables(k):
             sl = slots[k % 2]
             s_out = s_outs[k % 2]
             t = sl["tables"]
